@@ -2,7 +2,7 @@
 """Benchmark of the GNN keypoint head (BASELINE.json metric: RoIs/sec, 4096-keypoint head).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dtype bf16|fp32]
-                  [--config full4096|init64|ycbv1024|lm_sweep]
+                  [--config full4096|init64|ycbv1024|lm_sweep] [--dump-outputs DIR]
 
 One "step" = one pass of the post-backbone head over a batch of synthetic RoIs.  Default workload (the headline):
 BASELINE.json configs[2], "full progressive 512->4096 keypoint GNN head, batch 256 RoIs, bf16" -- 256 RoIs PER GPU
@@ -23,6 +23,10 @@ the library convolutions of the image branch; ``parity`` = agreement of the deco
 on a small sample, computed outside every timed region; ``cpu_baseline`` = the CPU restatement of the reference head on
 this box's host cores over a bounded sample.  ``--impl reference`` times only the CPU arm (the unmodified reference
 modules when /root/reference is present, else the oracle port; the line says which).
+
+``--dump-outputs DIR`` writes, after the timed steps, what the last timed step returned to its caller as float32 .npy files
+(a fixed seeded sample of the RoIs when the batch is larger than 60 MiB).  Inputs and weights come from fixed seeds, so two
+builds run with the same arguments can be compared output for output.
 """
 import argparse
 import json
@@ -48,6 +52,7 @@ DOMINANT_KERNEL_DRAM_SOURCE = "profiles/r02_h_edgeconv.txt (ncu --set full of be
 K3_KERNEL_DRAM_BYTES = 0.567e9 + 1.022e9
 K3_KERNEL_DRAM_SOURCE = "profiles/r02_h_taps_chain_query_tail.txt (ncu --set full, launch 0: dram read 0.567 GB + write 1.022 GB)"
 LM_OBJECT_IDS = (1, 2, 4, 5, 6, 8, 9, 10, 11, 12, 13, 14, 15)     # the 13 LM objects of test_lm.py:109
+DUMP_BUDGET_BYTES = 60 << 20      # --dump-outputs writes at most this much (plus the .npy headers): under 64 MB
 
 
 def load_peaks():
@@ -177,8 +182,9 @@ def make_inputs(case, dev, dtype, seed_rank):
     return feats, bbox
 
 
-def make_step(wl, case, bbox, gather):
-    """-> step(feats) -> (records or logits, done_event).  The records leave in the packed 2-byte form."""
+def make_step(wl, case, bbox, gather, last=None):
+    """-> step(feats) -> (records or logits, done_event).  The records leave in the packed 2-byte form.  With a dict
+    ``last``, every step leaves there the tensors its caller receives (for --dump-outputs)."""
     net, obj_ids = case["net"], case["obj_ids"]
     pexp = case["p3d"][obj_ids - 1] if wl["lm"] else case["p3d"].expand(case["B"], -1, -1)
     if wl["init_only"]:
@@ -187,18 +193,46 @@ def make_step(wl, case, bbox, gather):
         def step(f):
             bits = net(f, obj_ids) if wl["lm"] else net(f)
             # decode of the low-level bits (pipeline.py:363-369): roi mask + 3+3-bit cell ids
-            P.from_mask_prob_to_mask(bits[:, 0:1].contiguous())
-            P.from_code_prob_to_id(bits[:, 1:4].contiguous())
+            mask = P.from_mask_prob_to_mask(bits[:, 0:1].contiguous())
+            x_id = P.from_code_prob_to_id(bits[:, 1:4].contiguous())
             ids = P.from_code_prob_to_id(bits[:, 4:7].contiguous())
+            if last is not None:
+                last.update(init_bits=bits, roi_mask=mask, x_id=x_id, y_id=ids)
             ev = torch.cuda.Event()
             ev.record()
             return ids, ev
         return step
 
     def step(f):
-        _, corr = net.forward_with_correspondences(f, pexp, bbox, obj_ids=obj_ids, packed=True)
+        out, corr = net.forward_with_correspondences(f, pexp, bbox, obj_ids=obj_ids, packed=True)
+        if last is not None:
+            last.update(zip(("roi_bit", "x_bits", "y_bits", "seg", "x_id", "y_id"), out), records=corr)
         return gather.submit(corr)
     return step
+
+
+def dump_outputs(out_dir, last):
+    """--dump-outputs: write the tensors of ``last`` as ``out_dir/<name>.npy`` in float32.  The packed correspondence records
+    are unpacked into what their consumer reads (records_uv, records_flags).  If the whole batch exceeds DUMP_BUDGET_BYTES,
+    a fixed seeded sample of RoIs is written instead: the same rows of every array, listed in roi_rows.npy."""
+    import numpy as np
+    from checkerpose_b200 import ops
+    host = {}
+    for name, t in last.items():
+        if name == "records":
+            uv, flags, _, _, _ = ops.unpack_correspondences_host(t)
+            host["records_uv"], host["records_flags"] = uv, flags.astype(np.float32)
+        else:
+            host[name] = t.float().cpu().numpy()
+    B = len(host["x_id"])
+    per_roi = sum(a[0].nbytes for a in host.values()) + 8          # + its entry in roi_rows.npy
+    rows = np.arange(B)
+    if B * per_roi > DUMP_BUDGET_BYTES:
+        rows = np.sort(torch.randperm(B, generator=torch.Generator().manual_seed(0))[:DUMP_BUDGET_BYTES // per_roi].numpy())
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in host.items():
+        np.save(os.path.join(out_dir, name + ".npy"), np.ascontiguousarray(a[rows]))
+    np.save(os.path.join(out_dir, "roi_rows.npy"), rows.astype(np.float64))
 
 
 # ------------------------------------------------------------------------------------------------------
@@ -409,7 +443,8 @@ def run_ours(args):
     B, N = case["B"], case["N"]
     feats, bbox = make_inputs(case, dev, dtype, rank)
     gather = cpdist.OverlappedGather(dev)
-    step = make_step(wl, case, bbox, gather)
+    last = {} if args.dump_outputs else None
+    step = make_step(wl, case, bbox, gather, last)
 
     nwarm = args.warmup if args.profile else max(args.warmup, 3)
     for _ in range(nwarm):
@@ -430,6 +465,8 @@ def run_ours(args):
     value = B * world / (ms_step * 1e-3)
     roof, roof_k3 = kernel_rooflines(log, ms_total, args.steps, B, N, dtype, world)
     roof_conv = conv_roofline(log, ms_total, args.steps, world)
+    if last is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)      # the last timed step's outputs, before the legs below run the step again
 
     if args.profile:   # under ncu: no e2e / CPU legs, numbers printed here are NOT bench values
         if rank == 0:
@@ -554,6 +591,7 @@ def run_sweep(args, wl, dev, rank, world, dtype, barrier):
     Ns = [int(x) for x in args.sweep_n.split(",")]
     Ks = [int(x) for x in args.sweep_k.split(",")]
     table = []
+    last = {} if args.dump_outputs else None
     for N in Ns:
         for K in Ks:
             if K > N:
@@ -561,7 +599,7 @@ def run_sweep(args, wl, dev, rank, world, dtype, barrier):
             case = build_case(wl, dev, rank, N=N, K=K)
             feats, bbox = make_inputs(case, dev, dtype, rank)
             gather = cpdist.OverlappedGather(dev)
-            step = make_step(wl, case, bbox, gather)
+            step = make_step(wl, case, bbox, gather, last)
             for _ in range(max(args.warmup, 3)):
                 step(feats)
             ms = timed_loop(step, feats, args.steps, barrier, world, dev) / args.steps
@@ -570,6 +608,8 @@ def run_sweep(args, wl, dev, rank, world, dtype, barrier):
                           "staged_kernel": bool(plan.staged), "max_distinct_rows_per_tile": int(plan.max_unique)})
             del case, feats, step
             torch.cuda.empty_cache()
+    if last is not None and rank == 0:
+        dump_outputs(args.dump_outputs, last)      # the last timed step of the last (N, K) entry
     if rank == 0:
         head_entry = next((t for t in table if t["npoint"] == 4096 and t["graph_k"] == 20), table[-1])
         print(json.dumps({"metric": "RoIs/sec (lm_sweep)", "value": head_entry["rois_per_s"], "unit": UNIT, "n_gpus": world, "steps": args.steps,
@@ -598,6 +638,8 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-parity", action="store_true")
     ap.add_argument("--profile", action="store_true", help="short run for ncu: timed loop only, warm-up exactly --warmup")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last timed step returned as DIR/<name>.npy (float32, under 64 MB)")
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference(args)

@@ -209,6 +209,37 @@ def test_bench_reference_arm_contract():
     assert bench.LM_OBJECT_IDS == (1, 2, 4, 5, 6, 8, 9, 10, 11, 12, 13, 14, 15)
 
 
+def test_bench_dump_outputs_float32_and_seeded_sample(tmp_path, monkeypatch):
+    """--dump-outputs: one float32 .npy per tensor the step returned (packed records unpacked); above the byte budget,
+    the same fixed seeded sample of RoIs from every array, listed in roi_rows.npy."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench", os.path.join(REPO, "bench.py"))
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    B, N = 16, 64
+    g = torch.Generator().manual_seed(0)
+    last = dict(roi_bit=torch.randn(B, 1, N, generator=g), x_bits=torch.randn(B, 6, N, generator=g),
+                y_bits=torch.randn(B, 6, N, generator=g), seg=torch.randn(B, 2, 64, 64, generator=g),
+                x_id=torch.randint(0, 64, (B, N), generator=g), y_id=torch.randint(0, 64, (B, N), generator=g),
+                records=torch.zeros(B, 16 + 2 * N, dtype=torch.uint8))
+
+    def dump(name):
+        bench.dump_outputs(str(tmp_path / name), last)
+        return {f[:-4]: np.load(tmp_path / name / f) for f in os.listdir(tmp_path / name)}
+    full = dump("full")
+    assert sorted(full) == ["records_flags", "records_uv", "roi_bit", "roi_rows", "seg", "x_bits", "x_id", "y_bits", "y_id"]
+    assert all(a.dtype == np.float32 and len(a) == B for k, a in full.items() if k != "roi_rows")
+    assert np.array_equal(full["roi_rows"], np.arange(B)) and full["records_uv"].shape == (B, N, 2)
+    assert np.array_equal(full["x_bits"], last["x_bits"].numpy()) and np.array_equal(full["y_id"], last["y_id"].numpy())
+    per_roi = sum(a[0].nbytes for a in full.values())
+    monkeypatch.setattr(bench, "DUMP_BUDGET_BYTES", 5 * per_roi)
+    a, b = dump("a"), dump("b")
+    rows = a["roi_rows"].astype(np.int64)
+    assert len(rows) == 5 and np.array_equal(np.unique(rows), rows) and sum(x.nbytes for x in a.values()) <= 5 * per_roi
+    for k in full:
+        assert np.array_equal(a[k], b[k]) and (k == "roi_rows" or np.array_equal(a[k], full[k][rows])), k
+
+
 # ------------------------------------------------------------------------------------------------ graph plan (host code)
 @pytest.mark.parametrize("ds,objs,N,K", [("lmo", (1,), 4096, 20), ("ycbv", (21,), 512, 20), ("lm", (2, 9), 300, 8), ("lmo", (5,), 1024, 40),
                                          ("lmo", (8,), 200, 13)])
