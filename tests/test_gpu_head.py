@@ -6,7 +6,8 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import HEAD_CASES, check_head_checksums, head_case_inputs, rel_err, syn
+from helpers import (BF16_MAX, BF16_RMS, BF16_STAGE_MAX, BF16_STAGE_RMS, HEAD_CASES, check_head_checksums, head_case_inputs,
+                     rel_err, syn)
 
 pytestmark = pytest.mark.gpu
 torch.set_grad_enabled(False)
@@ -116,11 +117,8 @@ def test_head_fp32_vs_reference_golden(golden, name):
     assert gf.shape == (B, 64, N) and rel_err(gf.cpu(), g["init_graph_feat"]) < 1e-3
 
 
-# bf16 tolerances.  north_star's bar is 1e-2 relative per bf16 op; the per-module tests in test_gpu_kernels.py hold
-# it outright.  The init head chains four bf16 layers (conv1x1, 2 EdgeConv, Linear) and every tensor between them
-# is re-quantised to bf16, so its logits are held to 1e-2 in the rms sense with 2e-2 for the worst element
-# (measured: rms 0.3-1.1e-2, max 0.6-1.0e-2; scripts/precision_sim.py reproduces this budget on the CPU).
-BF16_RMS, BF16_MAX = 1.5e-2, 2e-2
+# bf16 tolerances: BF16_RMS / BF16_MAX (init-stage logits) and BF16_STAGE_RMS / BF16_STAGE_MAX (one refine stage at
+# N = 4096) live in helpers.py with the measurements behind them.
 
 
 @pytest.mark.parametrize("name", list(HEAD_CASES))
@@ -268,12 +266,6 @@ def test_full_size_properties(dtype):
 
 
 _FULL_ORACLE = {}
-# N = 4096: a refine stage is a chain of 9 bf16 layers (4-tap gather, 2 Linear, 3 EdgeConv = 3 x [P|Q] GEMM + max, 3 query
-# Linear) whose tensors are each re-quantised to bf16.  Measured on B200, teacher-forced: new bits rms 0.96-1.65e-2 / max
-# 1.7-2.25e-2 of scale, graph feature rms 0.8e-2 / max 1.1-1.4e-2 (north_star's 1e-2 holds per module, see
-# test_gpu_kernels.py; it cannot hold for the logits at the end of a 9-layer bf16 chain).  Sign bits flip for 0.06-0.3 % of
-# the keypoints per stage, all of them inside the relative margin below.
-BF16_STAGE_RMS, BF16_STAGE_MAX = 2e-2, 2.5e-2
 
 
 def _full_size_case(ds, obj):

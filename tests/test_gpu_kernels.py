@@ -114,7 +114,12 @@ def test_static_graph_module_fp32(cp, golden, tag):
 
 
 @pytest.mark.parametrize("ds,objs,N,K,Co,B", [("lmo", (1,), 4096, 20, 256, 3), ("lm", (3, 7), 300, 20, 64, 4), ("ycbv", (5,), 1000, 8, 96, 2),
-                                               ("lmo", (5,), 512, 40, 32, 2)])
+                                               ("lmo", (5,), 512, 40, 32, 2),
+                                               # KP = 16 / 32, and padded lists (K < KP) at every other size
+                                               ("lm", (2,), 1024, 16, 128, 2), ("ycbv", (3, 4, 5), 1024, 32, 64, 3),
+                                               ("lm", (6,), 700, 13, 96, 2), ("lmo", (1,), 300, 27, 256, 2),
+                                               ("ycbv", (7,), 1000, 37, 32, 2), ("ycbv", (9, 10), 129, 5, 64, 3),
+                                               ("lm", (11,), 512, 17, 128, 2)])
 def test_edge_aggregate_staged_f32_bit_exact(cp, ds, objs, N, K, Co, B):
     """float32 aggregation on the graph plan (rows staged per tile, node pairs) == the unstaged gather kernel, bit for bit
     (max and one add per element: no rounding freedom), incl. ragged last tiles and per-RoI graphs."""
