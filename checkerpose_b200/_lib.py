@@ -90,9 +90,6 @@ class ConvSlabParams(C.Structure):
         ("num_phases", c_i32), ("phase", SlabPhase * SLAB_MAX_PHASES),
         ("vy0", c_i32), ("vy1", c_i32), ("vx0", c_i32), ("vx1", c_i32),
         ("compact", c_i32), ("out_sb", c_i64), ("out_sy", c_i32), ("out_sx", c_i32),
-        ("up_a", c_vp), ("up_a_sb", c_i64), ("up_a_sh", c_i64), ("up_a_sw", c_i64), ("up_Ca", c_i32),
-        ("up_b", c_vp), ("up_b_sb", c_i64), ("up_b_sh", c_i64), ("up_b_sw", c_i64), ("up_Cb", c_i32),
-        ("up_H", c_i32), ("up_W", c_i32),
         ("seg_w", c_vp), ("seg_b", c_vp), ("seg_out", c_vp), ("seg_n", c_i32),
     ]
 

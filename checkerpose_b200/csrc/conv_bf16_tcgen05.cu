@@ -221,7 +221,7 @@ __device__ void weight_producer(const CvParams& kp, uint8_t* sm, Bars* bars) {
     const int rows0 = min(128, cols), rows1 = cols - rows0;
     for (int kc = 0; kc < kp.KC; ++kc, ++it) {
       const uint32_t s = it % STAGES;
-      if (it >= STAGES) mbar_wait_idle(&bars->empty[s], ((it / STAGES) - 1) & 1);
+      if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       if (MC) {
         // both CTAs of the cluster consume the same weight tile (nblk == 1): each fetches HALF of its rows from L2 and
         // multicasts them into both CTAs' stage s; every CTA's barrier expects the whole tile

@@ -13,7 +13,7 @@
 // after the matrix zero-filled), and tap t is the same shared memory read through a descriptor whose start address is moved
 // by shift_t rows.  Measured on B200: tcgen05.mma applies the 128-byte swizzle on ABSOLUTE shared-memory address bits (the
 // pattern TMA wrote), so a start address that is not a multiple of 8 rows needs nothing else -- putting the row phase into
-// the descriptor's base-offset field (bits 49-51) gives wrong results (CP_SLAB_BASEOFF=1 reproduces that).  No loader warps.
+// the descriptor's base-offset field (bits 49-51) gives wrong results.  No loader warps.
 //
 // CTA pairs (cluster of 2, tcgen05.mma.cta_group::2, M = 256): each CTA holds the slab of its own 128 positions and HALF of
 // every weight tile; the leader's MMA reads both halves.  Weight traffic into each SM's shared memory halves again.
@@ -38,8 +38,6 @@ namespace {
 
 constexpr int TILE_M = 128;
 constexpr int NTHREADS = 256;            // TMA-fed kernel: 8 warps
-constexpr int NTHREADS_UP = 512;         // fused upsampling: + 8 interpolating loader warps
-constexpr int UP_WARP0 = 8, UP_WARPS = 8;
 constexpr int EPI_WARP0 = 4;
 constexpr int MAX_AB = 6;
 constexpr int MAX_WS = 8;
@@ -63,9 +61,6 @@ struct SlabParams {
   int lo;             // smallest tap shift: the slab of tile rt starts at row rt * 128 + lo
   int RB;             // rows per TMA box (two boxes per slab)
   int a_buf_bytes, w_slot_bytes, AB, WS, off_w, off_epi, off_bar;   // AB slab buffers, WS weight stages
-  int base_off;       // 1: descriptors carry the row phase in their base-offset field
-  int span;           // largest - smallest tap shift: the taps of a tile read slab rows [0, 128 + span)
-  float up_scale_h, up_scale_w;
   int64_t G;
 };
 
@@ -114,23 +109,6 @@ __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
         "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
       : "r"(taddr));
 }
-// Wait of the leader's MMA thread on a barrier the peer CTA arrives on as well.  The data behind it is only read by the MMA
-// unit (async proxy), never by this thread: the default CTA-scope wait is enough, as in CUTLASS' 2-SM pipelines.
-// CP_SLAB_ACQ_CLUSTER (build option) restores the cluster-scope acquire for A/B measurements.
-template <bool PAIR>
-__device__ __forceinline__ void wait_full(uint64_t* bar, uint32_t parity) {
-#ifdef CP_SLAB_ACQ_CLUSTER
-  if (PAIR) {
-    const uint32_t a = smem_u32(bar);
-    uint32_t spins = 0;
-    while (!mbar_try_wait_cluster(a, parity))
-      if (++spins > (1u << 27)) __trap();
-    return;
-  }
-#endif
-  mbar_wait(bar, parity);
-}
-
 // ------------------------------------------------------------------------------------------------------
 template <bool PAIR>
 __device__ void slab_producer(const SlabParams& kp, const CUtensorMap* x_map, uint8_t* sm, Bars* bars) {
@@ -143,7 +121,7 @@ __device__ void slab_producer(const SlabParams& kp, const CUtensorMap* x_map, ui
     units.at(i, ph, rt);
     const int row_start = rt * TILE_M + kp.lo;
     for (int cc = 0; cc < kp.c_chunks; ++cc) {
-      if (around > 0) mbar_wait_idle(&bars->a_empty[ab], (around - 1) & 1);
+      if (around > 0) mbar_wait(&bars->a_empty[ab], (around - 1) & 1);
       if (elect_one()) {
         const uint32_t dst = sm_base + ab * (uint32_t)kp.a_buf_bytes;
         mbar_arrive_expect_tx(&bars->a_full[ab], 2 * box_bytes);
@@ -151,93 +129,6 @@ __device__ void slab_producer(const SlabParams& kp, const CUtensorMap* x_map, ui
         tma_load_2d(dst + box_bytes, x_map, cc * 64, row_start + kp.RB, &bars->a_full[ab]);
       }
       __syncwarp();
-      if (++ab == (uint32_t)kp.AB) { ab = 0; ++around; }
-    }
-  }
-}
-
-// Fused x2 bilinear upsampling (align_corners=True) of cat([up_a, up_b]): the loader warps write the slab the TMA unit would
-// have fetched from the stored map -- same values (the arithmetic of upsample2x_cat_nhwc_kernel, image_ops.cu: four combined
-// weights, fmaf chain, round to bf16), same SWIZZLE_128B placement, zeros on the border and outside the batch.  8 lanes own
-// one slab row (16 bytes = 8 channels each), a warp 4 rows, a pass of the 8 warps 32 rows; the four source vectors of
-// three passes are in flight together.  The source rows are L2-resident (a quarter of the map's size) and mostly L1 hits.
-template <bool PAIR>
-__device__ void up_loader(const SlabParams& kp, uint8_t* sm, Bars* bars, int tl) {
-  const cp_conv_slab_params& p = kp.p;
-  const Units<PAIR> units(kp);
-  const uint32_t sm_base = smem_u32(sm);
-  const int chunk = tl & 7, r0 = tl >> 3;
-  const int rows = TILE_M + kp.span;
-  const int H = p.up_H, W = p.up_W;
-  const bf16* pa = reinterpret_cast<const bf16*>(p.up_a);
-  const bf16* pb = reinterpret_cast<const bf16*>(p.up_b);
-  uint32_t ab = 0, around = 0;
-  constexpr int GROUP = 3;
-  for (int i = 0; i < units.count; ++i) {
-    int ph, rt;
-    units.at(i, ph, rt);
-    const int64_t row_start = (int64_t)rt * TILE_M + kp.lo;
-    for (int cc = 0; cc < kp.c_chunks; ++cc) {
-      const int c0 = cc * 64 + chunk * 8;
-      const bool from_a = c0 < p.up_Ca;
-      const bf16* src = from_a ? pa + c0 : pb + (c0 - p.up_Ca);
-      const int64_t s_sb = from_a ? p.up_a_sb : p.up_b_sb;
-      const int s_sh = (int)(from_a ? p.up_a_sh : p.up_b_sh), s_sw = (int)(from_a ? p.up_a_sw : p.up_b_sw);
-      if (around > 0) mbar_wait(&bars->a_empty[ab], (around - 1) & 1);
-      const uint32_t dst0 = sm_base + ab * (uint32_t)kp.a_buf_bytes;
-      for (int r = r0; r < rows; r += 32 * GROUP) {
-        uint4 v[GROUP][4];
-        float wgt[GROUP][4];
-        bool live[GROUP];
-#pragma unroll
-        for (int u = 0; u < GROUP; ++u) {
-          const int rr = r + 32 * u;
-          const int64_t g = row_start + rr;
-          live[u] = false;
-          if (rr < rows && g >= 0 && g < kp.G) {
-            const uint32_t gi = (uint32_t)g;
-            const uint32_t b = gi / (uint32_t)kp.img, rem = gi - b * (uint32_t)kp.img;
-            const uint32_t py = rem / (uint32_t)p.Wp, px = rem - py * (uint32_t)p.Wp;
-            if ((int)py < p.Hp - 1 && (int)px < p.Wp - 1) {
-              live[u] = true;
-              const float hr = kp.up_scale_h * (float)py, wr = kp.up_scale_w * (float)px;
-              const int h1 = (int)hr, w1 = (int)wr;
-              const int dh = (h1 < H - 1) ? s_sh : 0, dw = (w1 < W - 1) ? s_sw : 0;
-              const float h1l = hr - (float)h1, h0l = 1.f - h1l;
-              const float w1l = wr - (float)w1, w0l = 1.f - w1l;
-              wgt[u][0] = h0l * w0l; wgt[u][1] = h0l * w1l; wgt[u][2] = h1l * w0l; wgt[u][3] = h1l * w1l;
-              const bf16* s00 = src + (int64_t)b * s_sb + h1 * s_sh + w1 * s_sw;
-              v[u][0] = __ldg(reinterpret_cast<const uint4*>(s00));
-              v[u][1] = __ldg(reinterpret_cast<const uint4*>(s00 + dw));
-              v[u][2] = __ldg(reinterpret_cast<const uint4*>(s00 + dh));
-              v[u][3] = __ldg(reinterpret_cast<const uint4*>(s00 + dh + dw));
-            }
-          }
-        }
-#pragma unroll
-        for (int u = 0; u < GROUP; ++u) {
-          const int rr = r + 32 * u;
-          if (rr >= rows) continue;
-          uint4 o = make_uint4(0, 0, 0, 0);
-          if (live[u]) {
-            uint32_t ow[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) {
-              const uint32_t w00 = (&v[u][0].x)[e], w01 = (&v[u][1].x)[e], w10 = (&v[u][2].x)[e], w11 = (&v[u][3].x)[e];
-              float lo = wgt[u][0] * __uint_as_float(w00 << 16), hi = wgt[u][0] * __uint_as_float(w00 & 0xffff0000u);
-              lo = fmaf(wgt[u][1], __uint_as_float(w01 << 16), lo); hi = fmaf(wgt[u][1], __uint_as_float(w01 & 0xffff0000u), hi);
-              lo = fmaf(wgt[u][2], __uint_as_float(w10 << 16), lo); hi = fmaf(wgt[u][2], __uint_as_float(w10 & 0xffff0000u), hi);
-              lo = fmaf(wgt[u][3], __uint_as_float(w11 << 16), lo); hi = fmaf(wgt[u][3], __uint_as_float(w11 & 0xffff0000u), hi);
-              ow[e] = f2_to_bf2(lo, hi);
-            }
-            o = make_uint4(ow[0], ow[1], ow[2], ow[3]);
-          }
-          sts128(dst0 + rr * 128 + ((chunk ^ (rr & 7)) << 4), o);
-        }
-      }
-      fence_proxy_async_smem();      // generic-proxy writes of the slab -> visible to the tensor core's async proxy
-      __syncwarp();
-      if ((tl & 31) == 0) mbar_arrive(&bars->a_full[ab]);
       if (++ab == (uint32_t)kp.AB) { ab = 0; ++around; }
     }
   }
@@ -257,7 +148,7 @@ __device__ void weight_producer(const SlabParams& kp, uint8_t* sm, Bars* bars) {
     const cp_slab_phase& P = p.phase[ph];
     for (int cc = 0; cc < kp.c_chunks; ++cc) {
       for (int t = 0; t < P.ntaps; ++t) {
-        if (round > 0) mbar_wait_idle(&bars->w_empty[s], (round - 1) & 1);
+        if (round > 0) mbar_wait(&bars->w_empty[s], (round - 1) & 1);
         if (elect_one()) {
           const size_t kc = (size_t)P.wtap[t] * kp.c_chunks + cc;
           uint8_t* w_s = sm + kp.off_w + s * kp.w_slot_bytes;
@@ -294,25 +185,26 @@ __device__ void mma_issuer(const SlabParams& kp, uint8_t* sm, Bars* bars, uint32
     units.at(i, ph, rt);
     const cp_slab_phase& P = p.phase[ph];
     const uint32_t slot = tcount & 1;
-    if (tcount >= 2) wait_full<PAIR>(&bars->acc_empty[slot], ((tcount >> 1) - 1) & 1);
+    // CTA pairs: the peer arrives on these barriers as well.  The data behind them is only read by the MMA unit (async
+    // proxy), never by this thread, so the default CTA-scope wait is enough, as in CUTLASS' 2-SM pipelines.
+    if (tcount >= 2) mbar_wait(&bars->acc_empty[slot], ((tcount >> 1) - 1) & 1);
     const uint32_t d = tmem_base + slot * 256;
     for (int cc = 0; cc < kp.c_chunks; ++cc) {
-      wait_full<PAIR>(&bars->a_full[ab], around & 1);
+      mbar_wait(&bars->a_full[ab], around & 1);
       const uint32_t a_lo0 = smem_desc_lo(sm_base + ab * (uint32_t)kp.a_buf_bytes);
       for (int t = 0; t < P.ntaps; ++t) {
-        wait_full<PAIR>(&bars->w_full[s], wround & 1);
+        mbar_wait(&bars->w_full[s], wround & 1);
         tc_fence_after_sync();
         const uint32_t rel = (uint32_t)(P.shift[t] - kp.lo);            // rows from the start of the slab
         const uint32_t a_lo = a_lo0 + rel * 8;                          // 128 bytes per row, in units of 16
-        const uint32_t a_hi = kp.base_off ? desc_hi_base_offset(rel) : DESC_HI_SW128;
         const uint32_t w_lo = smem_desc_lo(sm_base + kp.off_w + s * kp.w_slot_bytes);
         const bool last_t = t == P.ntaps - 1;
         if (elect_one()) {
 #pragma unroll
           for (uint32_t k = 0; k < 4; ++k) {
             const uint32_t acc = (uint32_t)((cc | t | (int)k) != 0);
-            if (PAIR) mma2_bf16_ss_lohi(d, a_lo + 2 * k, a_hi, w_lo + 2 * k, idesc, acc);
-            else mma_bf16_ss_lohi(d, a_lo + 2 * k, a_hi, w_lo + 2 * k, idesc, acc);
+            if (PAIR) mma2_bf16_ss_lo(d, a_lo + 2 * k, w_lo + 2 * k, idesc, acc);
+            else mma_bf16_ss_lo(d, a_lo + 2 * k, w_lo + 2 * k, idesc, acc);
           }
           if (PAIR) {
             mma2_commit_both(smem_u32(&bars->w_empty[s]));
@@ -475,8 +367,8 @@ __device__ void epilogue(const SlabParams& kp, const CUtensorMap* out_map, uint8
   if (kp.tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
 }
 
-template <bool PAIR, bool UP>
-__global__ void __launch_bounds__(UP ? NTHREADS_UP : NTHREADS, 1) conv_slab_kernel(const __grid_constant__ SlabParams kp, const __grid_constant__ CUtensorMap x_map,
+template <bool PAIR>
+__global__ void __launch_bounds__(NTHREADS, 1) conv_slab_kernel(const __grid_constant__ SlabParams kp, const __grid_constant__ CUtensorMap x_map,
                                                                  const __grid_constant__ CUtensorMap out_map) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -486,7 +378,7 @@ __global__ void __launch_bounds__(UP ? NTHREADS_UP : NTHREADS, 1) conv_slab_kern
   if (threadIdx.x == 0) {
     // pairs: the leader's "full" barriers also collect the peer's relay, its acc_empty both CTAs' epilogue warps
     for (int a = 0; a < MAX_AB; ++a) {
-      mbar_init(&bars->a_full[a], (UP ? UP_WARPS : 1) + (PAIR && leader ? 1 : 0));
+      mbar_init(&bars->a_full[a], PAIR && leader ? 2 : 1);
       mbar_init(&bars->a_empty[a], 1);
     }
     for (int s = 0; s < MAX_WS; ++s) {
@@ -516,10 +408,9 @@ __global__ void __launch_bounds__(UP ? NTHREADS_UP : NTHREADS, 1) conv_slab_kern
   tc_fence_after_sync();
   const uint32_t tmem_base = bars->tmem_slot;
 
-  if (UP && warp >= UP_WARP0) up_loader<PAIR>(kp, sm, bars, (int)threadIdx.x - UP_WARP0 * 32);
-  else if (warp >= EPI_WARP0) epilogue<PAIR>(kp, &out_map, sm, bars, tmem_base, warp - EPI_WARP0, lane);
+  if (warp >= EPI_WARP0) epilogue<PAIR>(kp, &out_map, sm, bars, tmem_base, warp - EPI_WARP0, lane);
   else if (warp == 0) weight_producer<PAIR>(kp, sm, bars);
-  else if (warp == 3 && !UP) slab_producer<PAIR>(kp, &x_map, sm, bars);
+  else if (warp == 3) slab_producer<PAIR>(kp, &x_map, sm, bars);
   else if (warp == 1) {
     if (leader) mma_issuer<PAIR>(kp, sm, bars, tmem_base);
     else relay_peer(kp, bars);
@@ -534,14 +425,14 @@ __global__ void __launch_bounds__(UP ? NTHREADS_UP : NTHREADS, 1) conv_slab_kern
   }
 }
 
-template <bool PAIR, bool UP>
+template <bool PAIR>
 cudaError_t launch(const SlabParams& kp, const CUtensorMap& x_map, const CUtensorMap& out_map, int grid, int smem, cudaStream_t s) {
-  cudaError_t e = cudaFuncSetAttribute(conv_slab_kernel<PAIR, UP>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
+  cudaError_t e = cudaFuncSetAttribute(conv_slab_kernel<PAIR>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
   if (e != cudaSuccess) return e;
   cudaLaunchConfig_t cfg;
   memset(&cfg, 0, sizeof(cfg));
   cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(UP ? NTHREADS_UP : NTHREADS);
+  cfg.blockDim = dim3(NTHREADS);
   cfg.dynamicSmemBytes = (size_t)smem;
   cfg.stream = s;
   cudaLaunchAttribute attr[1];
@@ -551,7 +442,7 @@ cudaError_t launch(const SlabParams& kp, const CUtensorMap& x_map, const CUtenso
   attr[0].val.clusterDim.z = 1;
   cfg.attrs = attr;
   cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, conv_slab_kernel<PAIR, UP>, kp, x_map, out_map);
+  return cudaLaunchKernelEx(&cfg, conv_slab_kernel<PAIR>, kp, x_map, out_map);
 }
 
 }  // namespace
@@ -559,20 +450,10 @@ cudaError_t launch(const SlabParams& kp, const CUtensorMap& x_map, const CUtenso
 extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   CP_REQUIRE(pp, CP_E_INVALID, "cp_conv_slab: null params");
   const cp_conv_slab_params& p = *pp;
-  const bool up = p.up_a != nullptr;
-  CP_REQUIRE((p.x || up) && p.w_packed && p.out && p.B > 0 && p.Hp > 0 && p.Wp > 0 && p.Nout > 0, CP_E_INVALID, "cp_conv_slab: bad arguments");
+  CP_REQUIRE(p.x && p.w_packed && p.out && p.B > 0 && p.Hp > 0 && p.Wp > 0 && p.Nout > 0, CP_E_INVALID, "cp_conv_slab: bad arguments");
   CP_REQUIRE(p.C > 0 && p.C % 64 == 0 && (reinterpret_cast<uintptr_t>(p.w_packed) & 15) == 0 &&
-             (up || (p.ldx >= p.C && (p.ldx & 7) == 0 && (reinterpret_cast<uintptr_t>(p.x) & 15) == 0)), CP_E_UNSUPPORTED,
+             p.ldx >= p.C && (p.ldx & 7) == 0 && (reinterpret_cast<uintptr_t>(p.x) & 15) == 0, CP_E_UNSUPPORTED,
              "cp_conv_slab: C=%d must be a multiple of 64, pixel rows and weights 16-byte aligned", p.C);
-  if (up) {
-    CP_REQUIRE(p.up_H > 0 && p.up_W > 0 && p.Hp == 2 * p.up_H + 1 && p.Wp == 2 * p.up_W + 1 && p.up_Ca > 0 && p.up_Ca % 64 == 0 && p.up_Cb >= 0 &&
-               p.up_Ca + p.up_Cb == p.C && (p.up_Cb == 0 || p.up_b), CP_E_INVALID,
-               "cp_conv_slab: fused upsampling needs Hp = 2H+1, Wp = 2W+1, C = Ca+Cb, Ca %% 64 == 0 (H=%d W=%d Ca=%d Cb=%d)", p.up_H, p.up_W, p.up_Ca, p.up_Cb);
-    CP_REQUIRE(((p.up_a_sb | p.up_a_sh | p.up_a_sw | p.up_b_sb | p.up_b_sh | p.up_b_sw) & 7) == 0 && (reinterpret_cast<uintptr_t>(p.up_a) & 15) == 0 &&
-               (reinterpret_cast<uintptr_t>(p.up_b) & 15) == 0 && (int64_t)(p.up_H - 1) * p.up_a_sh + (int64_t)(p.up_W - 1) * p.up_a_sw < (1ll << 31) &&
-               (int64_t)(p.up_H - 1) * p.up_b_sh + (int64_t)(p.up_W - 1) * p.up_b_sw < (1ll << 31), CP_E_UNSUPPORTED,
-               "cp_conv_slab: fused upsampling sources must be 16-byte aligned NHWC views, one map below 2^31 elements");
-  }
   CP_REQUIRE(p.Nout <= 256 && p.ld_out >= p.Nout, CP_E_UNSUPPORTED, "cp_conv_slab: Nout=%d must be <= 256 and <= ld_out", p.Nout);
   CP_REQUIRE(p.num_phases >= 1 && p.num_phases <= CP_SLAB_MAX_PHASES && (p.num_phases == 1 || p.compact), CP_E_INVALID,
              "cp_conv_slab: %d phases (several phases need a compact destination)", p.num_phases);
@@ -597,10 +478,6 @@ extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   }
   CP_REQUIRE((int64_t)(wt_max + 1) * p.C <= p.K && p.K % 64 == 0, CP_E_INVALID, "cp_conv_slab: weight tap %d beyond K=%d", wt_max, p.K);
   kp.lo = lo;
-  kp.span = hi - lo;
-  // align_corners=True: scale = (in - 1) / (out - 1), as cp_upsample2x_cat_nhwc computes it
-  kp.up_scale_h = up && 2 * p.up_H > 1 ? (float)(p.up_H - 1) / (float)(2 * p.up_H - 1) : 0.f;
-  kp.up_scale_w = up && 2 * p.up_W > 1 ? (float)(p.up_W - 1) / (float)(2 * p.up_W - 1) : 0.f;
   const int R = TILE_M + hi - lo;
   kp.RB = ((R + 1) / 2 + 7) / 8 * 8;
   CP_REQUIRE(kp.RB <= 256, CP_E_UNSUPPORTED, "cp_conv_slab: tap span %d rows too wide for one slab (map width %d)", hi - lo, p.Wp);
@@ -611,8 +488,6 @@ extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   kp.npad = (p.Nout + 15) / 16 * 16;
   const char* pair_env = getenv("CP_SLAB_PAIR");
   const bool pair = !(pair_env && pair_env[0] == '0') && (kp.npad == 256 || kp.npad <= 128) && kp.row_tiles >= 2;
-  const char* bo_env = getenv("CP_SLAB_BASEOFF");
-  kp.base_off = bo_env && bo_env[0] == '1';   // measured: tcgen05 swizzles on absolute address bits -- the field stays 0
   kp.a_buf_bytes = 2 * kp.RB * 128;
   const int w_rows = pair ? kp.npad / 2 : kp.npad;
   kp.w_slot_bytes = (w_rows * 128 + 1023) / 1024 * 1024;
@@ -621,11 +496,9 @@ extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   const int avail = SMEM_LIMIT - (1024 + 4 * 2 * EPI_TILE_BYTES + BAR_BYTES + SEG_BYTES);
   kp.AB = (avail - 4 * kp.w_slot_bytes) / kp.a_buf_bytes;
   kp.AB = kp.AB > MAX_AB ? MAX_AB : kp.AB;
-  if (const char* ab_env = getenv("CP_SLAB_AB")) kp.AB = atoi(ab_env) < kp.AB && atoi(ab_env) >= 2 ? atoi(ab_env) : kp.AB;   // A/B measurements
   CP_REQUIRE(kp.AB >= 2, CP_E_UNSUPPORTED, "cp_conv_slab: no room for two activation slabs");
   kp.WS = (avail - kp.AB * kp.a_buf_bytes) / kp.w_slot_bytes;
   kp.WS = kp.WS > MAX_WS ? MAX_WS : kp.WS;
-  if (const char* ws_env = getenv("CP_SLAB_WS")) kp.WS = atoi(ws_env) < kp.WS && atoi(ws_env) >= 2 ? atoi(ws_env) : kp.WS;
   CP_REQUIRE(kp.WS >= 2, CP_E_UNSUPPORTED, "cp_conv_slab: no room for the weight ring");
   kp.off_w = kp.AB * kp.a_buf_bytes;
   kp.off_epi = kp.off_w + kp.WS * kp.w_slot_bytes;
@@ -636,7 +509,7 @@ extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   CUtensorMap x_map, out_map;
   memset(&x_map, 0, sizeof(x_map));
   memset(&out_map, 0, sizeof(out_map));
-  int rc = up ? CP_OK : cp::make_bf16_operand_map(&x_map, p.x, p.C, kp.G, p.ldx, "cp_conv_slab", kp.RB);
+  int rc = cp::make_bf16_operand_map(&x_map, p.x, p.C, kp.G, p.ldx, "cp_conv_slab", kp.RB);
   if (rc != CP_OK) return rc;
   kp.tma_out = (!p.compact && (p.ld_out & 7) == 0 && p.Nout % 32 == 0 && (reinterpret_cast<uintptr_t>(p.out) & 15) == 0) ? 1 : 0;
   if (kp.tma_out) {
@@ -648,12 +521,11 @@ extern "C" int cp_conv_slab(const cp_conv_slab_params* pp, cp_stream_t s) {
   if (pair) {
     const int units = (kp.row_tiles + 1) / 2 * p.num_phases;
     const int clusters = units < num_sms / 2 ? units : num_sms / 2;
-    e = up ? launch<true, true>(kp, x_map, out_map, 2 * clusters, smem, (cudaStream_t)s)
-           : launch<true, false>(kp, x_map, out_map, 2 * clusters, smem, (cudaStream_t)s);
+    e = launch<true>(kp, x_map, out_map, 2 * clusters, smem, (cudaStream_t)s);
   } else {
     const int units = kp.row_tiles * p.num_phases;
     const int grid = units < num_sms ? units : num_sms;
-    e = up ? launch<false, true>(kp, x_map, out_map, grid, smem, (cudaStream_t)s) : launch<false, false>(kp, x_map, out_map, grid, smem, (cudaStream_t)s);
+    e = launch<false>(kp, x_map, out_map, grid, smem, (cudaStream_t)s);
   }
   CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "cp_conv_slab: launch failed: %s", cudaGetErrorString(e));
   CP_CHECK_LAUNCH("cp_conv_slab");

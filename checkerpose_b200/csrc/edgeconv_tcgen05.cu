@@ -27,16 +27,8 @@
 // The aggregation of tile i+1 overlaps the MMAs and the epilogue of tile i; every hand-off is an mbarrier.
 // What bounds the kernel: DESIGN.md section 5.
 //
-// CTA-pair variant (template parameter PAIR; cluster of 2 CTAs = 2 SMs, cta_group::2): each CTA stages, aggregates and
-// drains its OWN tile exactly as above, but the two tiles share every MMA: the leader's MMA warp issues
-// tcgen05.mma.cta_group::2 (M = 256 = the two tiles, N = 256) once both CTAs' A slices are complete; each CTA streams and
-// holds only HALF of every weight tile (N/2 rows) and reads its A slice twice instead of four times -- 384 KB less per
-// tile through the shared-memory port that binds this kernel.  Hand-offs across the pair: the peer's aggregators /
-// epilogue warps arrive on the LEADER's a_full / acc_empty barriers (mapa + mbarrier.arrive.shared::cluster), the peer's
-// otherwise idle MMA warp relays "my weight half has landed" to the leader's b_full, and the leader's
-// tcgen05.commit.multicast::cluster releases A slices, weight stages and accumulator blocks in both CTAs.
+// A CTA-pair variant (cta_group::2, two tiles sharing every MMA) was measured no faster and removed: DESIGN.md section 8.
 #include <cuda.h>
-#include <stdlib.h>
 #include <string.h>
 
 #include "common.cuh"
@@ -60,34 +52,17 @@ constexpr int STG_WARP0 = MMA_WARP + 3;         // two idle warps complete the c
 constexpr int NUM_STG_WARPS = 4;
 constexpr int STG_THREADS = NUM_STG_WARPS * 32;
 constexpr int NUM_WARPS = STG_WARP0 + NUM_STG_WARPS;
-#ifndef CP_REGS_AGG
 // measured (ms per launch, 256->512 / 256->256 + a_out): 72/64/56/40 0.623 / 0.600; 80/56/56/24 0.655 / 0.601;
 // 80/56/48/32 0.632 / 0.601; 80/48/56/40 0.668 / 0.607; 80/56/40/40 0.663 / 0.688 (the stagers need 56, the MMA warp
 // spills below 40, the epilogue slows below 64)
-#define CP_REGS_AGG 72
-#define CP_REGS_EPI 64
-#define CP_REGS_STG 56
-#define CP_REGS_CTRL 40
-#endif
-constexpr int REGS_AGG = CP_REGS_AGG, REGS_EPI = CP_REGS_EPI, REGS_CTRL = CP_REGS_CTRL, REGS_STG = CP_REGS_STG;   // the kernel is launched at 64
+constexpr int REGS_AGG = 72, REGS_EPI = 64, REGS_CTRL = 40, REGS_STG = 56;   // the kernel is launched at 64
 static_assert(NUM_WARPS == 32 && NUM_AGG_WARPS * REGS_AGG + NUM_EPI_WARPS * REGS_EPI + 4 * REGS_CTRL + NUM_STG_WARPS * REGS_STG <= NUM_WARPS * 64,
               "register budget");
 constexpr int NTHREADS = NUM_WARPS * 32;
 constexpr int A_BUF_BYTES = TILE_M * 128;    // one K slice of the A operand: 128 rows x 64 bf16
-#ifndef CP_A_BUFS
-#define CP_A_BUFS 3
-#endif
-#ifndef CP_B_STAGES
-#define CP_B_STAGES 3
-#endif
-constexpr int A_BUFS = CP_A_BUFS;
-#ifndef CP_MMA_N
-#define CP_MMA_N 128                         // columns per tcgen05.mma.  256 (32 KB stages, half the A re-reads) was measured no
-                                             // faster with the earlier issue loop (DESIGN.md section 8); the current mma_issuer is N = 128 only
-#endif
-constexpr int MMA_N = CP_MMA_N;
-constexpr int B_STAGE_BYTES = MMA_N * 128;   // one K slice of MMA_N weight rows
-constexpr int B_STAGES = CP_B_STAGES;
+constexpr int A_BUFS = 3;
+constexpr int B_STAGE_BYTES = 128 * 128;     // one K slice of a packed 128-row weight tile (the N of one tcgen05.mma)
+constexpr int B_STAGES = 3;
 constexpr int NBAR = 4;                      // staging rounds that may be unreleased at any time
 constexpr int UI = CP_PLAN_UMAX / NUM_QW;    // list entries per quarter-warp
 constexpr int TBUF_BYTES = 32 * 64;          // per epilogue warp: a tile of 32 rows x 32 bf16 (SWIZZLE_64B) for the TMA stores
@@ -100,11 +75,7 @@ static_assert(UI == 8 && NUM_QW == CP_PLAN_LIST_LANES, "the issue path loads a q
 constexpr int OFF_A = 0;
 constexpr int OFF_B = OFF_A + A_BUFS * A_BUF_BYTES;
 constexpr int OFF_TBUF = OFF_B + B_STAGES * B_STAGE_BYTES;
-#ifndef CP_TBUFS
-#define CP_TBUFS 1                           // store tiles per epilogue warp (2: the next block is written while the TMA engine reads this one)
-#endif
-constexpr int TBUFS = CP_TBUFS;
-constexpr int OFF_BIAS = OFF_TBUF + NUM_EPI_WARPS * TBUFS * TBUF_BYTES;
+constexpr int OFF_BIAS = OFF_TBUF + NUM_EPI_WARPS * TBUF_BYTES;
 constexpr int OFF_BAR = OFF_BIAS + BIAS_BYTES;
 constexpr int OFF_WQ = OFF_BAR + 256;                          // per stager warp: virtual ring position of the last NBAR rounds
 constexpr int OFF_PROG = OFF_WQ + NUM_STG_WARPS * 16 + 64;
@@ -128,27 +99,17 @@ struct EcParams {
   int tiles_per_roi;
   int tpr_shift;     // log2(tiles_per_roi) when it is a power of two (every shipped N), else -1
   int tma_out;       // bf16 output with nout % 32 == 0: the epilogue stores through the tensor map
-  int n_last;        // columns of the last accumulator block (multiple of 16)
-  WTile wt[MAX_WTILES];  // order: slice-major, then column block (CTA pairs: then cluster rank -- each CTA's half of the block)
+  WTile wt[MAX_WTILES];  // order: slice-major, then column block
 };
 
-// Tiles of this CTA.  Single CTAs walk the tiles with stride gridDim.x; a CTA pair (cluster rank r) takes tile 2p + r of
-// pair p.  With an odd tile count the last pair's second CTA repeats the last tile (identical values stored twice).
-template <bool PAIR>
+// Tiles of this CTA: blockIdx.x, then every gridDim.x-th tile.
 struct TileIt {
   int first, step, count, last;
   __device__ __forceinline__ explicit TileIt(const EcParams& kp) {
     last = kp.num_tiles - 1;
-    if (PAIR) {
-      const int cid = (int)blockIdx.x >> 1, ncl = (int)gridDim.x >> 1, npairs = (kp.num_tiles + 1) >> 1;
-      first = 2 * cid + (int)(blockIdx.x & 1);
-      step = 2 * ncl;
-      count = cid < npairs ? (npairs - cid + ncl - 1) / ncl : 0;
-    } else {
-      first = (int)blockIdx.x;
-      step = (int)gridDim.x;
-      count = first < kp.num_tiles ? (kp.num_tiles - first + step - 1) / step : 0;
-    }
+    first = (int)blockIdx.x;
+    step = (int)gridDim.x;
+    count = first < kp.num_tiles ? (kp.num_tiles - first + step - 1) / step : 0;
   }
   __device__ __forceinline__ int tile(int i) const {
     const int t = first + i * step;
@@ -239,45 +200,23 @@ __device__ __forceinline__ void tile_coords(const EcParams& kp, int tile, int& b
   g = kp.p.graph_sel ? __ldg(kp.p.graph_sel + b) : 0;
 }
 
-#ifdef CP_TRACE
-// debug builds only: clock64 timestamps of CTA 0's hand-offs (role r writes cp_trace[r * 1024 + k])
-__device__ long long cp_trace[8 * 1024];
-#define TR(role, k) do { if (blockIdx.x == 0 && (k) < 1024 && ((role) != 0 || (threadIdx.x & 31) == 0)) cp_trace[(role) * 1024 + (k)] = clock64(); } while (0)
-#else
-#define TR(role, k)
-#endif
-#ifdef CP_PROFILE_PHASES
-__device__ unsigned long long cp_dbg_phase[16];
-#define PH_T(v) const long long v = clock64()
-#define PH_ADD(i, a, b) ph[i] += (b) - (a)
-#else
-#define PH_T(v)
-#define PH_ADD(i, a, b)
-#endif
-
 // ------------------------------------------------------------------------------------------------------
 // weight producer / MMA issuer
 // ------------------------------------------------------------------------------------------------------
-template <bool PAIR>
 __device__ void weight_producer(const EcParams& kp, uint8_t* sm, Bars* bars) {
-  constexpr int SUB = MMA_N / 128;     // packed 128-row tiles per stage
-  const int NBM = (kp.NB + SUB - 1) / SUB;
-  const int rank = PAIR ? (int)(blockIdx.x & 1) : 0;
-  const TileIt<PAIR> tiles(kp);
+  const int NB = kp.NB;
+  const TileIt tiles(kp);
   uint32_t cnt = 0;
   for (int ti = 0; ti < tiles.count; ++ti) {
     for (int c = 0; c < kp.KC; ++c)
-      for (int nbm = 0; nbm < NBM; ++nbm, ++cnt) {
+      for (int nb = 0; nb < NB; ++nb, ++cnt) {
         const int s = cnt % B_STAGES;
         const uint32_t use = cnt / B_STAGES;
-        if (use > 0) mbar_wait_idle(&bars->b_empty[s], (use - 1) & 1);
-        const WTile& w0 = PAIR ? kp.wt[(c * kp.NB + nbm) * 2 + rank] : kp.wt[c * kp.NB + nbm * SUB];
-        const bool two = !PAIR && SUB == 2 && nbm * SUB + 1 < kp.NB;
-        const uint32_t bytes1 = two ? kp.wt[c * kp.NB + nbm * SUB + 1].bytes : 0u;
+        if (use > 0) mbar_wait(&bars->b_empty[s], (use - 1) & 1);
+        const WTile& w = kp.wt[c * NB + nb];
         if (elect_one()) {
-          mbar_arrive_expect_tx(&bars->b_full[s], w0.bytes + bytes1);
-          bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, w0.ptr, w0.bytes, &bars->b_full[s]);
-          if (two) bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES + 128 * 128, kp.wt[c * kp.NB + nbm * SUB + 1].ptr, bytes1, &bars->b_full[s]);
+          mbar_arrive_expect_tx(&bars->b_full[s], w.bytes);
+          bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, w.ptr, w.bytes, &bars->b_full[s]);
         }
         __syncwarp();
       }
@@ -288,7 +227,6 @@ __device__ void weight_producer(const EcParams& kp, uint8_t* sm, Bars* bars) {
 // tile time, so the loop keeps running ring positions / parities / descriptor words in registers (no modulo, no
 // constant-bank table look-ups, no 64-bit descriptor rebuild per MMA) and issues under elect.sync.
 __device__ void mma_issuer(const EcParams& kp, uint8_t* sm, Bars* bars, uint32_t tmem_base) {
-  static_assert(MMA_N == 128, "one 128-row weight tile per stage");
   const uint32_t a_lo0 = smem_desc_lo(smem_u32(sm + OFF_A)), b_lo0 = smem_desc_lo(smem_u32(sm + OFF_B));
   const uint32_t a_full0 = smem_u32(&bars->a_full[0]), a_empty0 = smem_u32(&bars->a_empty[0]);
   const uint32_t b_full0 = smem_u32(&bars->b_full[0]), b_empty0 = smem_u32(&bars->b_empty[0]);
@@ -311,7 +249,7 @@ __device__ void mma_issuer(const EcParams& kp, uint8_t* sm, Bars* bars, uint32_t
   auto commit_s = [](uint32_t bar_s) {
     asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar_s) : "memory");
   };
-  const TileIt<false> tiles(kp);
+  const TileIt tiles(kp);
   for (int ti = 0; ti < tiles.count; ++ti) {
     for (int c = 0; c < KC; ++c) {
       wait_s(a_full0 + ab * 8, a_par);
@@ -325,12 +263,10 @@ __device__ void mma_issuer(const EcParams& kp, uint8_t* sm, Bars* bars, uint32_t
         const uint32_t idesc = nb == NB - 1 ? idesc_last : idesc_full;
         const uint32_t d = tmem_base + (uint32_t)(nb * 128);
         if (elect_one()) {
-#ifndef CP_KO_MMA
           mma_bf16_ss_lo(d, a_lo, b_lo, idesc, (uint32_t)(c != 0));
           mma_bf16_ss_lo(d, a_lo + 2, b_lo + 2, idesc, 1u);
           mma_bf16_ss_lo(d, a_lo + 4, b_lo + 4, idesc, 1u);
           mma_bf16_ss_lo(d, a_lo + 6, b_lo + 6, idesc, 1u);
-#endif
           commit_s(b_empty0 + bs * 8);
           if (last_slice) commit_s(acc_full0 + nb * 8);
           if (nb == NB - 1) commit_s(a_empty0 + ab * 8);
@@ -345,71 +281,6 @@ __device__ void mma_issuer(const EcParams& kp, uint8_t* sm, Bars* bars, uint32_t
   }
 }
 
-// CTA pairs: the leader's MMA warp.  One tcgen05.mma.cta_group::2 covers both CTAs' tiles (M = 256) and 256 output columns;
-// a_full / b_full / acc_empty collect arrivals from both CTAs (waited with cluster-scope acquire), the commits release
-// the buffers in both.
-__device__ void mma_issuer_pair(const EcParams& kp, uint8_t* sm, Bars* bars, uint32_t tmem_base) {
-  const uint32_t a_lo0 = smem_desc_lo(smem_u32(sm + OFF_A)), b_lo0 = smem_desc_lo(smem_u32(sm + OFF_B));
-  const uint32_t a_full0 = smem_u32(&bars->a_full[0]), a_empty0 = smem_u32(&bars->a_empty[0]);
-  const uint32_t b_full0 = smem_u32(&bars->b_full[0]), b_empty0 = smem_u32(&bars->b_empty[0]);
-  const uint32_t acc_full0 = smem_u32(&bars->acc_full[0]), acc_empty0 = smem_u32(&bars->acc_empty[0]);
-  const int KC = kp.KC, NB = kp.NB;
-  const uint32_t idesc_full = make_idesc_bf16(256, 256);
-  const uint32_t idesc_last = make_idesc_bf16(256, (uint32_t)kp.n_last);
-  uint32_t ab = 0, a_par = 0, bs = 0, b_par = 0, acc_par = 0;
-  bool first_tile = true;
-  auto wait_c = [](uint32_t bar_s, uint32_t parity) {
-    uint32_t spins = 0;
-    while (!mbar_try_wait_cluster(bar_s, parity))
-      if (++spins > (1u << 27)) __trap();
-  };
-  const TileIt<true> tiles(kp);
-  for (int ti = 0; ti < tiles.count; ++ti) {
-    for (int c = 0; c < KC; ++c) {
-      wait_c(a_full0 + ab * 8, a_par);                      // both CTAs' aggregators finished this slice
-      const uint32_t a_lo = a_lo0 + ab * (A_BUF_BYTES >> 4);
-      const bool last_slice = c == KC - 1;
-      for (int nb = 0; nb < NB; ++nb) {
-        wait_c(b_full0 + bs * 8, b_par);                    // both halves of the weight block have landed
-        if (c == 0 && !first_tile) wait_c(acc_empty0 + nb * 8, acc_par);
-        tc_fence_after_sync();
-        const uint32_t b_lo = b_lo0 + bs * (B_STAGE_BYTES >> 4);
-        const uint32_t idesc = nb == NB - 1 ? idesc_last : idesc_full;
-        const uint32_t d = tmem_base + (uint32_t)(nb * 256);
-        if (elect_one()) {
-          mma2_bf16_ss_lo(d, a_lo, b_lo, idesc, (uint32_t)(c != 0));
-          mma2_bf16_ss_lo(d, a_lo + 2, b_lo + 2, idesc, 1u);
-          mma2_bf16_ss_lo(d, a_lo + 4, b_lo + 4, idesc, 1u);
-          mma2_bf16_ss_lo(d, a_lo + 6, b_lo + 6, idesc, 1u);
-          mma2_commit_both(b_empty0 + bs * 8);
-          if (last_slice) mma2_commit_both(acc_full0 + nb * 8);
-          if (nb == NB - 1) mma2_commit_both(a_empty0 + ab * 8);
-        }
-        __syncwarp();
-        if (++bs == B_STAGES) { bs = 0; b_par ^= 1; }
-      }
-      if (++ab == A_BUFS) { ab = 0; a_par ^= 1; }
-    }
-    if (!first_tile) acc_par ^= 1;
-    first_tile = false;
-  }
-}
-
-// CTA pairs: the peer's MMA warp has nothing to issue; it tells the leader when the peer's half of a weight stage has landed.
-__device__ void weight_relay_peer(const EcParams& kp, Bars* bars) {
-  const uint32_t leader_b_full0 = mapa_rank(smem_u32(&bars->b_full[0]), 0);
-  uint32_t bs = 0, b_par = 0;
-  const TileIt<true> tiles(kp);
-  for (int ti = 0; ti < tiles.count; ++ti)
-    for (int c = 0; c < kp.KC; ++c)
-      for (int nb = 0; nb < kp.NB; ++nb) {
-        mbar_wait(&bars->b_full[bs], b_par);
-        if (elect_one()) mbar_arrive_remote(leader_b_full0 + bs * 8);
-        __syncwarp();
-        if (++bs == B_STAGES) { bs = 0; b_par ^= 1; }
-      }
-}
-
 // Ring position of the next round (U rows, contiguous): a pure function of the list lengths of the tiles this CTA
 // processes, so the stagers and every aggregator warp compute it on their own and never exchange positions.
 __device__ __forceinline__ uint32_t ring_place(uint32_t& ph, uint32_t U, uint32_t R) {
@@ -422,7 +293,7 @@ __device__ __forceinline__ uint32_t ring_place(uint32_t& ph, uint32_t U, uint32_
 // ------------------------------------------------------------------------------------------------------
 // stagers: one warpgroup copies every round's distinct neighbour row slices into the ring
 // ------------------------------------------------------------------------------------------------------
-template <int KCH, bool PAIR>
+template <int KCH>
 __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int lane) {
   constexpr int PROG_BYTES = prog_bytes(KCH), OFF_RING = off_ring(KCH);
   constexpr uint32_t R = ring_rows(KCH);
@@ -434,7 +305,7 @@ __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int 
   const uint32_t vs = sm_base + OFF_WQ + pw * 16;        // per-warp copy of vstart[NBAR] (same-value stores by all lanes)
   const uint32_t row_bytes = (uint32_t)p.ld_z * 2;
   const uint32_t KC = (uint32_t)kp.KC;
-  const TileIt<PAIR> tiles(kp);
+  const TileIt tiles(kp);
   const int my_tiles = tiles.count;
   uint32_t vh = 0, ph = 0;      // ring head: virtual (monotonic) and physical row
   uint32_t rel = 0;             // rounds < rel are known to be released by all aggregator warps
@@ -476,10 +347,9 @@ __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int 
       while (rel < r) {
         const uint32_t oldest_v = lds32(vs + (rel % NBAR) * 4);
         if (nvh + U - oldest_v <= R && (int)rel > need_rel) break;
-        mbar_wait_idle(&bars->stg_empty[rel % NBAR], (rel / NBAR) & 1);
+        mbar_wait(&bars->stg_empty[rel % NBAR], (rel / NBAR) & 1);
         ++rel;
       }
-      if (tid == 0) TR(5, r * 2 + 0);
       sts32(vs + (r % NBAR) * 4, nvh);
       __syncwarp();      // every lane stores the same value and reads it back later: order the lanes explicitly (racecheck)
       vh = nvh + U;
@@ -489,9 +359,7 @@ __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int 
 #pragma unroll 4
       for (uint32_t j = (uint32_t)q; j < U; j += 16) {
         const uint32_t row = __ldg(lst + (j & (NUM_QW - 1)) * UI + (j >> 6));
-#ifndef CP_KO_COPY   // timing experiment only (wrong results)
         cp_async16(dst + (j - (uint32_t)q) * 128u, src + (size_t)row * row_bytes);
-#endif
       }
       if (c == 0) {  // the tile's pair programs ride along with its first round
         const uint32_t pd = sm_base + OFF_PROG + (ti & 1) * PROG_BYTES;
@@ -500,7 +368,6 @@ __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int 
       }
       // asynchronous arrival: fires when all of this thread's copies so far have landed; nobody waits here
       asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(&bars->stg_full[r % NBAR])) : "memory");
-      if (tid == 0) TR(5, r * 2 + 1);
     }
   }
 }
@@ -527,7 +394,7 @@ __device__ __forceinline__ uint4 finish_node(uint4 m, uint4 q, float slope, bool
   return make_uint4(ow[0], ow[1], ow[2], ow[3]);
 }
 
-template <int KCH, bool PAIR>
+template <int KCH>
 __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, int lane) {
   constexpr int KP = 4 * KCH, PW = prog_width(KCH), PROG_BYTES = prog_bytes(KCH), OFF_RING = off_ring(KCH);
   constexpr uint32_t R = ring_rows(KCH);
@@ -541,17 +408,12 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
   const uint32_t KC = (uint32_t)kp.KC;
   uint32_t it = 0;      // round being reduced
   uint32_t ph = 0;      // ring head (replica of the stagers')
-#ifdef CP_PROFILE_PHASES
-  long long ph_[8] = {0, 0, 0, 0, 0, 0, 0, 0};
-#endif
   auto tile_U = [&](int tile) -> uint32_t {
     int b, t, g;
     tile_coords(kp, tile, b, t, g);
     return (uint32_t)__ldg(pl.ucount + (size_t)g * pl.T + t);
   };
-  const TileIt<PAIR> tiles(kp);
-  // CTA pairs: "this A slice is complete" goes to the LEADER's barrier, which collects both CTAs' aggregator warps
-  const uint32_t a_full_leader0 = PAIR ? mapa_rank(smem_u32(&bars->a_full[0]), 0) : 0u;
+  const TileIt tiles(kp);
   uint32_t U_next = tiles.count > 0 ? tile_U(tiles.tile(0)) : 0u;
   for (uint32_t ti = 0; ti < (uint32_t)tiles.count; ++ti) {
     const int tile = tiles.tile((int)ti);
@@ -562,12 +424,8 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
     const uint32_t U = U_next;
     if ((int)ti + 1 < tiles.count) U_next = tile_U(tiles.tile((int)ti + 1));
     for (uint32_t c = 0; c < KC; ++c, ++it) {
-      PH_T(t0);
       const uint32_t stg = sm_base + OFF_RING + ring_place(ph, U, R) * 128u + sub * 16;
-      if (lane == 0 && (aw == 0 || aw == 15)) TR(1 + (aw == 15), it * 4 + 0);
       mbar_wait(&bars->stg_full[it % NBAR], (it / NBAR) & 1);
-      if (lane == 0 && (aw == 0 || aw == 15)) TR(1 + (aw == 15), it * 4 + 1);
-      PH_T(t3);
 
       // ---- this quarter-warp's pair; the overlap-sorted pair groups rotate over the warps from slice to slice so that
       //      every warp sees the same mix of cheap (large C) and expensive pairs over a tile ----
@@ -575,20 +433,12 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
       const uint32_t pe = prog_s + pair * (PW * 2);
       const uint32_t info = lds32(pe + 2 * KP * 2);
       const int na = info & 255, nb = (info >> 8) & 255;
-#ifdef CP_KO_READS   // timing experiment only (wrong results): no row reads
-      const uint32_t nc4 = 0, nr4 = 0;
-#else
       const uint32_t nc4 = info >> 18;              // chunks (of 4 rows) the pair shares        } warp-uniform
       const uint32_t nr4 = (uint32_t)KCH - nc4;     // chunks of each node's own rows            }
-#endif
       // own Q slices: issued first, their (L2) latency hides behind the row reads
       const bf16* zq = reinterpret_cast<const bf16*>(p.z) + p.Co + c * 64 + sub * 8;
-#ifdef CP_KO_Q
-      const uint4 qa = make_uint4(0, 0, 0, 0), qb = qa;
-#else
       const uint4 qa = na != 255 ? ldg_nc_v4(zq + (size_t)(row0 + na) * p.ld_z) : make_uint4(0, 0, 0, 0);
       const uint4 qb = nb != 255 ? ldg_nc_v4(zq + (size_t)(row0 + nb) * p.ld_z) : make_uint4(0, 0, 0, 0);
-#endif
 
       uint4 acc = make_uint4(NEG_INF2, NEG_INF2, NEG_INF2, NEG_INF2);
       uint32_t pa = pe;
@@ -604,13 +454,8 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
         accb = max_quad(accb, stg, ob.x, ob.y);
       }
 
-      PH_T(t4);
       const uint32_t ab = it % A_BUFS;
-      if (lane == 0 && (aw == 0 || aw == 15)) TR(1 + (aw == 15), it * 4 + 2);
       if (it >= A_BUFS) mbar_wait(&bars->a_empty[ab], ((it / A_BUFS) - 1) & 1);   // MMAs that read this buffer are done
-      if (lane == 0 && (aw == 0 || aw == 15)) TR(1 + (aw == 15), it * 4 + 3);
-      PH_T(t5);
-#ifndef CP_KO_FINISH
       if (na != 255) {
         const uint4 o = finish_node(acc, qa, slope, fast_lrelu);
         sts128(sm_base + a_offset(ab, na, sub), o);
@@ -622,22 +467,13 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
         if (p.a_out) *reinterpret_cast<uint4*>(reinterpret_cast<bf16*>(p.a_out) + (size_t)(row0 + nb) * p.ld_a_out + c * 64 + sub * 8) = o;
       }
       fence_proxy_async_smem();  // generic-proxy writes of A -> visible to the tensor core's async proxy
-#endif
       __syncwarp();
       if (lane == 0) {
-        if (PAIR) mbar_arrive_remote(a_full_leader0 + ab * 8);
-        else mbar_arrive(&bars->a_full[ab]);
+        mbar_arrive(&bars->a_full[ab]);
         mbar_arrive(&bars->stg_empty[it % NBAR]);
       }
-#ifdef CP_PROFILE_PHASES
-      { PH_T(t6); ph_[2] += t3 - t0; ph_[3] += t4 - t3; ph_[4] += t5 - t4; ph_[5] += t6 - t5; }
-#endif
     }
   }
-#ifdef CP_PROFILE_PHASES
-  if (lane == 0)
-    for (int i = 0; i < 6; ++i) atomicAdd(&cp_dbg_phase[i], (unsigned long long)ph_[i]);
-#endif
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -648,29 +484,24 @@ __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t sm
                ::"l"(map), "r"(smem_src), "r"(c0), "r"(c1), "r"(c2) : "memory");
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-template <int N> __device__ __forceinline__ void bulk_wait_read() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
+__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
 
-template <bool ACT, bool TMA_OUT, bool PAIR>
+template <bool ACT, bool TMA_OUT>
 __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, uint8_t* sm, Bars* bars, uint32_t tmem_base, int ew, int lane) {
-  constexpr int ACC_BLK = PAIR ? 256 : 128;      // columns per accumulator block (= per MMA)
-  constexpr int ACC_SH = PAIR ? 8 : 7;
-  const uint32_t acc_empty_leader0 = PAIR ? mapa_rank(smem_u32(&bars->acc_empty[0]), 0) : 0u;
-  const TileIt<PAIR> tiles(kp);
+  constexpr int ACC_BLK = 128;      // columns per accumulator block (= per MMA)
+  constexpr int ACC_SH = 7;
+  const TileIt tiles(kp);
   const cp_edgeconv_params& p = kp.p;
   const cp_chain_layer& L = p.layer;
   const int q = ew & 3, h = ew >> 2;
   const int row = q * 32 + lane;
   const uint32_t tbase = tmem_base + ((uint32_t)(q * 32) << 16);
   const uint32_t sm_base = smem_u32(sm);
-  const uint32_t tbuf = sm_base + OFF_TBUF + ew * (TBUFS * TBUF_BYTES);
-  uint32_t nstore = 0;   // TMA stores issued by this warp
+  const uint32_t tbuf = sm_base + OFF_TBUF + ew * TBUF_BYTES;
   const uint32_t bias_s = sm_base + OFF_BIAS;
   const float slope = L.slope;
   const uint32_t bias_blocks = bars->bias_blocks;
   const int sw = (lane >> 1) & 3;   // SWIZZLE_64B: 16-byte chunk index ^= bits 1-2 of the row
-#ifdef CP_PROFILE_PHASES
-  long long ph[8] = {0};
-#endif
   for (int ti = 0; ti < tiles.count; ++ti) {
     const int tile = tiles.tile(ti);
     const int b = tile_roi(kp, tile), t = tile - b * kp.tiles_per_roi;
@@ -678,25 +509,17 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
     const int rows_valid = min(TILE_M, p.N - n0);
     const bool row_ok = row < rows_valid;
     const size_t grow0 = (size_t)b * p.N + n0;
-    PH_T(e0);
     for (int c0 = h * 32; c0 < kp.NB * ACC_BLK; c0 += 32 * (NUM_EPI_WARPS / 4)) {
       if ((c0 & (ACC_BLK - 1)) == h * 32) {   // this warp's first block of an accumulator block
-        PH_T(w0);
-        mbar_wait_idle(&bars->acc_full[c0 >> ACC_SH], ti & 1);
-        PH_T(w1);
-        PH_ADD(6, w0, w1);
+        mbar_wait(&bars->acc_full[c0 >> ACC_SH], ti & 1);
         tc_fence_after_sync();
       }
-      if (lane == 0 && (ew == 0 || ew == 7)) TR(3 + (ew == 7), ti * 8 + (c0 >> 6));
       const bool last_of_block = (c0 & (ACC_BLK - 1)) == h * 32 + ACC_BLK - 32 * (NUM_EPI_WARPS / 4);
       if (c0 >= kp.npad) {          // nothing to drain in a ragged block's tail; still release the block
         if (last_of_block) {
           tc_fence_before_sync();
           __syncwarp();
-          if (lane == 0) {
-            if (PAIR) mbar_arrive_remote(acc_empty_leader0 + (c0 >> ACC_SH) * 8);
-            else mbar_arrive(&bars->acc_empty[c0 >> ACC_SH]);
-          }
+          if (lane == 0) mbar_arrive(&bars->acc_empty[c0 >> ACC_SH]);
         }
         continue;
       }
@@ -731,24 +554,20 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
       if (TMA_OUT) {
         // 32 rows x 64 B tile in the SWIZZLE_64B layout of the tensor map; the TMA engine writes it to
         // out[b, n0 + 32 q .. +32, c0 .. c0+32) and clips rows beyond N
-        const uint32_t tb = tbuf + (nstore % TBUFS) * TBUF_BYTES;
-        ++nstore;
-        if (lane == 0) bulk_wait_read<TBUFS - 1>();   // the store that last used this buffer is done reading it
+        if (lane == 0) bulk_wait_read0();   // the warp's previous store is done reading the tile
         __syncwarp();
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
           const uint4 w = make_uint4(f2_to_bf2(v[e * 8], v[e * 8 + 1]), f2_to_bf2(v[e * 8 + 2], v[e * 8 + 3]),
                                      f2_to_bf2(v[e * 8 + 4], v[e * 8 + 5]), f2_to_bf2(v[e * 8 + 6], v[e * 8 + 7]));
-          sts128(tb + lane * 64 + ((e ^ sw) << 4), w);
+          sts128(tbuf + lane * 64 + ((e ^ sw) << 4), w);
         }
         fence_proxy_async_smem();
         __syncwarp();
-#ifndef CP_KO_EPI_STORE
         if (lane == 0 && q * 32 < rows_valid) {
-          tma_store_3d(out_map, tb, c0, n0 + q * 32, b);
+          tma_store_3d(out_map, tbuf, c0, n0 + q * 32, b);
           bulk_commit();
         }
-#endif
       } else if (row_ok) {
         if (p.out_mode == CP_OUT_BF16) {
           bf16* o = reinterpret_cast<bf16*>(p.out) + (grow0 + row) * p.ld_out + c0;
@@ -767,24 +586,14 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
       if (last_of_block) {   // this warp is done with the accumulator block: the next tile's MMAs may overwrite it
         tc_fence_before_sync();
         __syncwarp();
-        if (lane == 0) {
-          if (PAIR) mbar_arrive_remote(acc_empty_leader0 + (c0 >> ACC_SH) * 8);
-          else mbar_arrive(&bars->acc_empty[c0 >> ACC_SH]);
-        }
+        if (lane == 0) mbar_arrive(&bars->acc_empty[c0 >> ACC_SH]);
       }
     }
-#ifdef CP_PROFILE_PHASES
-    { PH_T(e2); PH_ADD(7, e0, e2); }   // [6] = waiting for accumulator blocks, [7] = the whole tile (waits included)
-#endif
   }
-#ifdef CP_PROFILE_PHASES
-  if (lane == 0)
-    for (int i = 6; i < 8; ++i) atomicAdd(&cp_dbg_phase[i], (unsigned long long)ph[i]);
-#endif
-  if (TMA_OUT && lane == 0) bulk_wait_read<0>();   // shared memory must outlive the last stores' reads
+  if (TMA_OUT && lane == 0) bulk_wait_read0();   // shared memory must outlive the last stores' reads
 }
 
-template <int KCH, bool PAIR>
+template <int KCH>
 __global__ void __launch_bounds__(NTHREADS, 1) edgeconv_kernel(const __grid_constant__ EcParams kp, const __grid_constant__ CUtensorMap out_map) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -796,26 +605,21 @@ __global__ void __launch_bounds__(NTHREADS, 1) edgeconv_kernel(const __grid_cons
       mbar_init(&bars->stg_full[s], STG_THREADS);     // every stager thread, asynchronously, once its copies of the round landed
       mbar_init(&bars->stg_empty[s], NUM_AGG_WARPS);
     }
-    // CTA pairs: the leader's a_full / acc_empty collect both CTAs' warps, its b_full the peer's relay as well
-    const bool leader = PAIR && (blockIdx.x & 1) == 0;
     for (int c = 0; c < A_BUFS; ++c) {
-      mbar_init(&bars->a_full[c], PAIR ? 2 * NUM_AGG_WARPS : NUM_AGG_WARPS);
+      mbar_init(&bars->a_full[c], NUM_AGG_WARPS);
       mbar_init(&bars->a_empty[c], 1);
     }
     for (int s = 0; s < B_STAGES; ++s) {
-      mbar_init(&bars->b_full[s], leader ? 2 : 1);
+      mbar_init(&bars->b_full[s], 1);
       mbar_init(&bars->b_empty[s], 1);
     }
     for (int nb = 0; nb < 4; ++nb) {
       mbar_init(&bars->acc_full[nb], 1);
-      mbar_init(&bars->acc_empty[nb], PAIR ? 2 * NUM_EPI_WARPS : NUM_EPI_WARPS);
+      mbar_init(&bars->acc_empty[nb], NUM_EPI_WARPS);
     }
     fence_mbar_init();
   }
-  if (warp == W_WARP) {
-    if (PAIR) tmem_alloc_pair(&bars->tmem_slot, TMEM_COLS);
-    else tmem_alloc(&bars->tmem_slot, TMEM_COLS);
-  }
+  if (warp == W_WARP) tmem_alloc(&bars->tmem_slot, TMEM_COLS);
   for (int i = threadIdx.x; i < BIAS_BYTES / 4; i += NTHREADS)   // bias row (zero-padded) for the epilogue's broadcast loads
     reinterpret_cast<float*>(sm + OFF_BIAS)[i] = (kp.p.layer.bias && i < kp.p.layer.nout) ? kp.p.layer.bias[i] : 0.f;
   if (warp == 0) {
@@ -826,92 +630,48 @@ __global__ void __launch_bounds__(NTHREADS, 1) edgeconv_kernel(const __grid_cons
     if (lane == 0) bars->bias_blocks = m;
   }
   tc_fence_before_sync();
-  if (PAIR) cluster_sync_all();      // both CTAs' barriers are initialised before anyone arrives remotely
-  else __syncthreads();
+  __syncthreads();
   tc_fence_after_sync();
   const uint32_t tmem_base = bars->tmem_slot;
 
   if (warp >= STG_WARP0) {
     if (REGS_STG < 64) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_STG));
-    stager<KCH, PAIR>(kp, sm, bars, warp - STG_WARP0, lane);
+    stager<KCH>(kp, sm, bars, warp - STG_WARP0, lane);
   } else if (warp >= W_WARP) {   // control warpgroup
     if (REGS_CTRL < 64) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_CTRL));
-    if (warp == MMA_WARP) {
-      if (!PAIR) mma_issuer(kp, sm, bars, tmem_base);
-      else if ((blockIdx.x & 1) == 0) mma_issuer_pair(kp, sm, bars, tmem_base);
-      else weight_relay_peer(kp, bars);
-    } else if (warp == W_WARP) {
-      weight_producer<PAIR>(kp, sm, bars);
-    }
+    if (warp == MMA_WARP) mma_issuer(kp, sm, bars, tmem_base);
+    else if (warp == W_WARP) weight_producer(kp, sm, bars);
     __syncwarp();
   } else if (warp >= EPI_WARP0) {
     if (REGS_EPI < 64) asm volatile("setmaxnreg.dec.sync.aligned.u32 %0;" ::"n"(REGS_EPI));
     const int q = warp - EPI_WARP0;
     const bool tma_out = kp.tma_out != 0;
     if (kp.p.layer.act) {
-      if (tma_out) epilogue_warps<true, true, PAIR>(kp, &out_map, sm, bars, tmem_base, q, lane);
-      else epilogue_warps<true, false, PAIR>(kp, &out_map, sm, bars, tmem_base, q, lane);
+      if (tma_out) epilogue_warps<true, true>(kp, &out_map, sm, bars, tmem_base, q, lane);
+      else epilogue_warps<true, false>(kp, &out_map, sm, bars, tmem_base, q, lane);
     } else {
-      if (tma_out) epilogue_warps<false, true, PAIR>(kp, &out_map, sm, bars, tmem_base, q, lane);
-      else epilogue_warps<false, false, PAIR>(kp, &out_map, sm, bars, tmem_base, q, lane);
+      if (tma_out) epilogue_warps<false, true>(kp, &out_map, sm, bars, tmem_base, q, lane);
+      else epilogue_warps<false, false>(kp, &out_map, sm, bars, tmem_base, q, lane);
     }
   } else {
     if (REGS_AGG > 64) asm volatile("setmaxnreg.inc.sync.aligned.u32 %0;" ::"n"(REGS_AGG));
-    aggregator<KCH, PAIR>(kp, sm, bars, warp, lane);
+    aggregator<KCH>(kp, sm, bars, warp, lane);
   }
 
   tc_fence_before_sync();
-  if (PAIR) cluster_sync_all();      // the peer may still arrive on / read from this CTA's shared memory until here
-  else __syncthreads();
-  if (warp == W_WARP) {
-    if (PAIR) tmem_dealloc_pair(tmem_base, TMEM_COLS);
-    else tmem_dealloc(tmem_base, TMEM_COLS);
-  }
+  __syncthreads();
+  if (warp == W_WARP) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
 template <int KCH>
-cudaError_t launch(const EcParams& kp, const CUtensorMap& map, int grid, bool pair, cudaStream_t s) {
-  if (!pair) {
-    cudaError_t e = cudaFuncSetAttribute(edgeconv_kernel<KCH, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-    if (e != cudaSuccess) return e;
-    edgeconv_kernel<KCH, false><<<grid, NTHREADS, SMEM_BYTES, s>>>(kp, map);
-    return cudaSuccess;
-  }
-  cudaError_t e = cudaFuncSetAttribute(edgeconv_kernel<KCH, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+cudaError_t launch(const EcParams& kp, const CUtensorMap& map, int grid, cudaStream_t s) {
+  cudaError_t e = cudaFuncSetAttribute(edgeconv_kernel<KCH>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
   if (e != cudaSuccess) return e;
-  cudaLaunchConfig_t cfg;
-  memset(&cfg, 0, sizeof(cfg));
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(NTHREADS);
-  cfg.dynamicSmemBytes = SMEM_BYTES;
-  cfg.stream = s;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2;
-  attr[0].val.clusterDim.y = 1;
-  attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, edgeconv_kernel<KCH, true>, kp, map);
+  edgeconv_kernel<KCH><<<grid, NTHREADS, SMEM_BYTES, s>>>(kp, map);
+  return cudaSuccess;
 }
 
 }  // namespace
-
-#ifdef CP_TRACE
-extern "C" int cp_debug_read_trace(long long* out, int n) {
-  cudaDeviceSynchronize();
-  return cudaMemcpyFromSymbol(out, cp_trace, sizeof(long long) * (size_t)(n < 8 * 1024 ? n : 8 * 1024)) == cudaSuccess ? 0 : -1;
-}
-#endif
-#ifdef CP_PROFILE_PHASES
-// debug builds only: cycles the aggregator warps spent per phase (summed over warps and SMs); resets the counters
-extern "C" int cp_debug_read_phases(unsigned long long* out16) {
-  unsigned long long z[16] = {0};
-  cudaDeviceSynchronize();
-  if (cudaMemcpyFromSymbol(out16, cp_dbg_phase, sizeof(z)) != cudaSuccess) return -1;
-  return cudaMemcpyToSymbol(cp_dbg_phase, z, sizeof(z)) == cudaSuccess ? 0 : -1;
-}
-#endif
 
 extern "C" int cp_edgeconv_ring_rows(int KP) {
   switch (KP) {
@@ -953,15 +713,7 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
   kp.KC = p.Co / 64;
   kp.npad = (L.nout + 15) & ~15;
   CP_REQUIRE(kp.npad <= TMEM_COLS, CP_E_UNSUPPORTED, "cp_edgeconv_fwd: nout=%d > 512", L.nout);
-  // CTA pairs (cta_group::2, N = 256 per MMA): opt-in with CP_EDGECONV_PAIR=1, possible when the output is whole
-  // 256-column blocks or one block of <= 128 columns (each CTA's half of a weight block is then one contiguous piece of
-  // a packed 128-row tile).  Measured on B200 (DESIGN.md section 8): bit-identical results, 0.69 vs 0.63 ms per launch --
-  // the pair moves 20 % fewer bytes through each SM's shared-memory port, but every MMA now waits for the slower of two
-  // CTAs' aggregators, and this kernel is bound by its hand-off chain, not by the port.  Hence off by default.
-  const char* pair_env = getenv("CP_EDGECONV_PAIR");
-  const bool pair = pair_env && pair_env[0] == '1' && (kp.npad % 256 == 0 || kp.npad <= 128);
-  kp.NB = pair ? (kp.npad + 255) / 256 : (kp.npad + 127) / 128;
-  kp.n_last = pair ? kp.npad - (kp.NB - 1) * 256 : kp.npad - (kp.NB - 1) * 128;
+  kp.NB = (kp.npad + 127) / 128;
   kp.tiles_per_roi = (p.N + TILE_M - 1) / TILE_M;
   kp.tpr_shift = -1;
   for (int sft = 0; sft < 30; ++sft)
@@ -975,30 +727,14 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
   const uint8_t* wbase = reinterpret_cast<const uint8_t*>(L.w_packed);
   for (int c = 0; c < kp.KC; ++c)
     for (int nb = 0; nb < kp.NB; ++nb) {
-      if (!pair) {
-        const int rows = (kp.npad - nb * 128 < 128) ? (kp.npad - nb * 128) : 128;
-        WTile& w = kp.wt[c * kp.NB + nb];
-        w.ptr = wbase + (size_t)nb * 128 * L.kin * 2 + (size_t)c * rows * 128;
-        w.bytes = (uint32_t)rows * 128;
-        w.pad = 0;
-        continue;
-      }
-      // the block's N2 columns = rows of the packed weight image; rank r holds rows [r N2/2, (r + 1) N2/2)
-      const int N2 = nb == kp.NB - 1 ? kp.n_last : 256;
-      for (int r = 0; r < 2; ++r) {
-        WTile& w = kp.wt[(c * kp.NB + nb) * 2 + r];
-        if (N2 == 256) w.ptr = wbase + (size_t)(2 * nb + r) * 128 * L.kin * 2 + (size_t)c * 128 * 128;
-        else w.ptr = wbase + (size_t)(2 * nb) * 128 * L.kin * 2 + (size_t)c * N2 * 128 + (size_t)r * (N2 / 2) * 128;
-        w.bytes = (uint32_t)(N2 / 2) * 128;
-        w.pad = 0;
-      }
+      const int rows = (kp.npad - nb * 128 < 128) ? (kp.npad - nb * 128) : 128;
+      WTile& w = kp.wt[c * kp.NB + nb];
+      w.ptr = wbase + (size_t)nb * 128 * L.kin * 2 + (size_t)c * rows * 128;
+      w.bytes = (uint32_t)rows * 128;
+      w.pad = 0;
     }
   const int num_sms = cp::num_sms();
-  int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;
-  if (pair) {
-    const int want = 2 * ((kp.num_tiles + 1) / 2);
-    grid = want < (num_sms & ~1) ? want : (num_sms & ~1);
-  }
+  const int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;
   // bf16 outputs whose width is a multiple of 32 columns leave through TMA tensor stores: a 3-D map (columns, nodes, RoIs)
   // with a 32 x 32 box, so that rows beyond N of a ragged last tile are clipped instead of landing in the next RoI
   CUtensorMap map;
@@ -1010,11 +746,11 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
   }
   cudaError_t e;
   switch (pl.KP) {
-    case 8: e = launch<2>(kp, map, grid, pair, (cudaStream_t)s); break;
-    case 16: e = launch<4>(kp, map, grid, pair, (cudaStream_t)s); break;
-    case 20: e = launch<5>(kp, map, grid, pair, (cudaStream_t)s); break;
-    case 32: e = launch<8>(kp, map, grid, pair, (cudaStream_t)s); break;
-    default: e = launch<10>(kp, map, grid, pair, (cudaStream_t)s); break;
+    case 8: e = launch<2>(kp, map, grid, (cudaStream_t)s); break;
+    case 16: e = launch<4>(kp, map, grid, (cudaStream_t)s); break;
+    case 20: e = launch<5>(kp, map, grid, (cudaStream_t)s); break;
+    case 32: e = launch<8>(kp, map, grid, (cudaStream_t)s); break;
+    default: e = launch<10>(kp, map, grid, (cudaStream_t)s); break;
   }
   CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "cp_edgeconv_fwd: launch failed: %s", cudaGetErrorString(e));
   CP_CHECK_LAUNCH("cp_edgeconv_fwd");

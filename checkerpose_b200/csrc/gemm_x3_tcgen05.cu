@@ -218,7 +218,7 @@ __device__ void weight_producer(const X3Params& kp, uint8_t* sm, Bars* bars) {
     const int rows0 = min(128, cols), rows1 = cols - rows0;    // the two packed 128-row blocks of this pass
     for (int kc = 0; kc < kp.KC; ++kc, ++it) {
       const uint32_t s = it % STAGES;
-      if (it >= STAGES) mbar_wait_idle(&bars->empty[s], ((it / STAGES) - 1) & 1);
+      if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       if (elect_one()) {
         uint8_t* w_hi = sm + s * STAGE_BYTES + 2 * A_BYTES;
         uint8_t* w_lo = w_hi + W_BYTES;

@@ -110,7 +110,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     uint32_t it = 0;
     for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x, ++it) {
       const uint32_t s = it % STAGES;
-      if (it >= STAGES) mbar_wait_idle(&bars->empty[s], ((it / STAGES) - 1) & 1);
+      if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       if (elect_one()) {
         mbar_arrive_expect_tx(&bars->full[s], (uint32_t)(KC * A_CHUNK_BYTES));
         for (int c = 0; c < KC; ++c) tma_load_2d(sm + s * A_STAGE_BYTES + c * A_CHUNK_BYTES, &src_map, c * 64, tile * TILE_M, &bars->full[s]);
@@ -148,7 +148,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     uint32_t it = 0;
     for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x, ++it) {
       const uint32_t slot = it & 1;
-      mbar_wait_idle(&bars->acc_full[slot], (it >> 1) & 1);
+      mbar_wait(&bars->acc_full[slot], (it >> 1) & 1);
       tc_fence_after_sync();
       const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + slot * NMID;
       float lx = cst[192], ly = cst[193];

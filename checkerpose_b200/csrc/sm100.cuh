@@ -39,21 +39,6 @@ __device__ __forceinline__ void mbar_wait(uint64_t* bar, uint32_t parity) {
   }
 }
 
-// Wait of a role that runs ahead of or behind the critical path (weight / staging producers, the epilogue between
-// tiles): back off with nanosleep, so that the spin takes neither issue slots nor power from the working warps (the
-// benchmark step runs under the board's power cap: profiles/).
-#ifndef CP_IDLE_SLEEP_NS
-#define CP_IDLE_SLEEP_NS 0
-#endif
-__device__ __forceinline__ void mbar_wait_idle(uint64_t* bar, uint32_t parity) {
-  if (mbar_try_wait(bar, parity)) return;
-  uint32_t spins = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if (CP_IDLE_SLEEP_NS) __nanosleep(CP_IDLE_SLEEP_NS);
-    if (++spins > (1u << 27)) __trap();
-  }
-}
-
 // One lane of a converged warp (elect.sync): the single-thread instructions (tcgen05.mma / commit, bulk copies) are
 // issued under this predicate while the surrounding control flow stays warp-uniform, so that ptxas keeps their
 // operands in uniform registers (under an `if (lane == 0)` region it wraps every one of them in a broadcast loop).
@@ -164,15 +149,6 @@ __device__ __forceinline__ void mbar_arrive_cluster(uint32_t cluster_addr) {   /
 __device__ __forceinline__ void mbar_arrive_remote(uint32_t cluster_addr) {
   asm volatile("mbarrier.arrive.shared::cluster.b64 _, [%0];" ::"r"(cluster_addr) : "memory");
 }
-__device__ __forceinline__ bool mbar_try_wait_cluster(uint32_t bar_s, uint32_t parity) {   // acquire at cluster scope
-  uint32_t ok;
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t"
-      "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 p, [%1], %2;\n\t"
-      "selp.u32 %0, 1, 0, p;\n\t}"
-      : "=r"(ok) : "r"(bar_s), "r"(parity) : "memory");
-  return ok != 0;
-}
 __device__ __forceinline__ void tmem_alloc_pair(uint32_t* slot_in_smem, uint32_t ncols) {  // one warp in EACH CTA, same warp id
   asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(slot_in_smem)), "r"(ncols) : "memory");
   asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
@@ -192,31 +168,6 @@ __device__ __forceinline__ void mma2_bf16_ss_lo(uint32_t d_tmem, uint32_t a_lo, 
       "mov.b64 db, {%2, %5};\n\t"
       "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %3, p;\n\t}"
       ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(0x40004040u)
-      : "memory");
-}
-// The same two MMAs with the A descriptor's HIGH word given as well: an operand that starts at a row r of a SWIZZLE_128B
-// tile which is not a multiple of 8 carries the row phase in the descriptor's base-offset field (bits 49-51:
-// (start address >> 7) & 7) -- the tap-shifted views of one activation slab in conv_slab_tcgen05.cu.
-constexpr uint32_t DESC_HI_SW128 = 0x40004040u;
-__device__ __forceinline__ uint32_t desc_hi_base_offset(uint32_t row_phase) { return DESC_HI_SW128 | ((row_phase & 7u) << 17); }
-__device__ __forceinline__ void mma_bf16_ss_lohi(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "mov.b64 da, {%1, %6};\n\t"
-      "mov.b64 db, {%2, %5};\n\t"
-      "tcgen05.mma.cta_group::1.kind::f16 [%0], da, db, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(DESC_HI_SW128), "r"(a_hi)
-      : "memory");
-}
-__device__ __forceinline__ void mma2_bf16_ss_lohi(uint32_t d_tmem, uint32_t a_lo, uint32_t a_hi, uint32_t b_lo, uint32_t idesc, uint32_t accumulate) {
-  asm volatile(
-      "{\n\t.reg .pred p;\n\t.reg .b64 da, db;\n\t"
-      "setp.ne.b32 p, %4, 0;\n\t"
-      "mov.b64 da, {%1, %6};\n\t"
-      "mov.b64 db, {%2, %5};\n\t"
-      "tcgen05.mma.cta_group::2.kind::f16 [%0], da, db, %3, p;\n\t}"
-      ::"r"(d_tmem), "r"(a_lo), "r"(b_lo), "r"(idesc), "r"(accumulate), "r"(DESC_HI_SW128), "r"(a_hi)
       : "memory");
 }
 // arrive (when all tcgen05 ops issued so far by this thread have completed) on the barrier at this offset in BOTH CTAs

@@ -32,37 +32,18 @@ using namespace sm100;
 namespace {
 
 constexpr int TILE_M = 128;
-#ifndef CP_K3_GWARPS
-#define CP_K3_GWARPS 4
-#endif
-#ifndef CP_K3_EWARPS
-#define CP_K3_EWARPS 8
-#endif
-constexpr int NUM_G_WARPS = CP_K3_GWARPS, G_THREADS = NUM_G_WARPS * 32;
-constexpr int NUM_E_WARPS = CP_K3_EWARPS;      // a multiple of 4: NUM_E_WARPS / 4 warps per TMEM lane quarter
-// warp layout: gather warps first; with two gather warps the weight producer and the MMA issuer take warps 2 and 3 and
-// TWELVE epilogue warps fill 4..15 (the epilogue is what this kernel waits for); otherwise they follow the epilogue warps
-constexpr bool COMPACT_ROLES = NUM_G_WARPS == 2;
+constexpr int NUM_G_WARPS = 4, G_THREADS = NUM_G_WARPS * 32;
+constexpr int NUM_E_WARPS = 8;              // a multiple of 4: NUM_E_WARPS / 4 warps per TMEM lane quarter
 constexpr int E_WARP0 = 4;
-constexpr int W_WARP = COMPACT_ROLES ? 2 : E_WARP0 + NUM_E_WARPS, MMA_WARP = W_WARP + 1;
-constexpr int NUM_WARPS = COMPACT_ROLES ? E_WARP0 + NUM_E_WARPS : (NUM_E_WARPS == 8 ? 16 : MMA_WARP + 1);   // 8 epilogue warps: two idle warps, 512 threads leave 128 registers per thread
+constexpr int W_WARP = E_WARP0 + NUM_E_WARPS, MMA_WARP = W_WARP + 1;
+constexpr int NUM_WARPS = 16;               // two idle warps: 512 threads leave 128 registers per thread
 static_assert(NUM_E_WARPS % 4 == 0 && E_WARP0 % 4 == 0 && NUM_G_WARPS <= E_WARP0 && TILE_M % (NUM_G_WARPS * 4) == 0, "epilogue warp w drains TMEM lane quarter w % 4");
 constexpr int NTHREADS = NUM_WARPS * 32;
 constexpr int CHUNK_BYTES = TILE_M * 128;   // 128 rows x 64 bf16
-#ifndef CP_K3_NX
-#define CP_K3_NX 4
-#endif
-#ifndef CP_K3_BSTAGES
-#define CP_K3_BSTAGES 4
-#endif
-constexpr int NX = CP_K3_NX;                // gather ring slots
+constexpr int NX = 4;                       // gather ring slots
 constexpr int NH = 4;                       // chunks of h0 / h1 (256 channels)
-constexpr int B_STAGES = CP_K3_BSTAGES, B_STAGE_BYTES = 128 * 128;
-constexpr int TBUF_BYTES = 32 * 64;          // per epilogue warp: tiles of 32 rows x 32 bf16 (SWIZZLE_64B) for the TMA stores
-#ifndef CP_K3_TBUFS
-#define CP_K3_TBUFS 1
-#endif
-constexpr int TBUFS = CP_K3_TBUFS;           // tiles per warp: with 2 a store only waits for the one before the previous
+constexpr int B_STAGES = 4, B_STAGE_BYTES = 128 * 128;
+constexpr int TBUF_BYTES = 32 * 64;          // per epilogue warp: a tile of 32 rows x 32 bf16 (SWIZZLE_64B) for the TMA stores
 constexpr int BIAS_FLOATS = 1024;           // 256 + 256 + 512
 constexpr int ACC_COLS = 256;
 constexpr int MAX_WT = 48;
@@ -71,7 +52,7 @@ constexpr int OFF_X = 0;
 constexpr int OFF_H = OFF_X + NX * CHUNK_BYTES;
 constexpr int OFF_B = OFF_H + NH * CHUNK_BYTES;
 constexpr int OFF_TBUF = OFF_B + B_STAGES * B_STAGE_BYTES;
-constexpr int OFF_BIAS = OFF_TBUF + NUM_E_WARPS * TBUFS * TBUF_BYTES;
+constexpr int OFF_BIAS = OFF_TBUF + NUM_E_WARPS * TBUF_BYTES;
 constexpr int OFF_BAR = OFF_BIAS + BIAS_FLOATS * 4;
 constexpr int SMEM_BYTES = OFF_BAR + 512;
 static_assert(SMEM_BYTES + 1024 <= 227 * 1024, "shared memory budget");
@@ -163,7 +144,7 @@ __device__ void gather_warps(const TcParams& kp, uint8_t* sm, Bars* bars, int gw
     const uint8_t* gf = reinterpret_cast<const uint8_t*>(p.graph_feat) + ((size_t)b * p.N + n0) * p.ld_gf * 2 + piece * 16;
     for (int c = 0; c < kp.KX; ++c, ++cnt) {
       const uint32_t slot = cnt % NX;
-      if (cnt >= NX) mbar_wait_idle(&bars->x_empty[slot], ((cnt / NX) - 1) & 1);
+      if (cnt >= NX) mbar_wait(&bars->x_empty[slot], ((cnt / NX) - 1) & 1);
       const uint32_t dst = sm_base + OFF_X + slot * CHUNK_BYTES;
       if (c < 4) {
         const int tap_off = (((c & 1) ? p.tap_step : 0) * p.Wp + ((c & 2) ? p.tap_step : 0)) * 128;
@@ -196,7 +177,7 @@ __device__ void weight_producer(const TcParams& kp, uint8_t* sm, Bars* bars) {
     for (int w = 0; w < kp.T; ++w, ++cnt) {
       const int s = cnt % B_STAGES;
       const uint32_t use = cnt / B_STAGES;
-      if (use > 0) mbar_wait_idle(&bars->b_empty[s], (use - 1) & 1);
+      if (use > 0) mbar_wait(&bars->b_empty[s], (use - 1) & 1);
       if (elect_one()) {
         mbar_arrive_expect_tx(&bars->b_full[s], kp.wt[w].bytes);
         bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, kp.wt[w].ptr, kp.wt[w].bytes, &bars->b_full[s]);
@@ -303,8 +284,6 @@ __device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t sm
 }
 __device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
 __device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-template <int N>
-__device__ __forceinline__ void bulk_wait_read_n() { asm volatile("cp.async.bulk.wait_group.read %0;" ::"n"(N) : "memory"); }
 
 __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, uint8_t* sm, Bars* bars, uint32_t tmem_base, int ew, int lane) {
   const cp_chain_params& p = kp.p;
@@ -312,8 +291,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
   const int row = q * 32 + lane;
   const uint32_t sm_base = smem_u32(sm);
   const uint32_t bias_s = sm_base + OFF_BIAS;
-  const uint32_t tbuf0 = sm_base + OFF_TBUF + ew * (TBUFS * TBUF_BYTES);
-  uint32_t nstore = 0;
+  const uint32_t tbuf = sm_base + OFF_TBUF + ew * TBUF_BYTES;
   const int sw = (lane >> 1) & 3;   // SWIZZLE_64B: 16-byte chunk index ^= bits 1-2 of the row
   uint32_t st = 0, hfree = 0;
   for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x) {
@@ -327,7 +305,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
       const int ncols = k < 2 ? ACC_COLS : kp.P2 * 128;                  // columns of this stage
       const int col0 = k < 2 ? 0 : (k - 2) * ACC_COLS;                   // first output column of the stage
       const uint32_t bias_l = bias_s + (uint32_t)(layer * 256 + col0) * 4;   // layers 0, 1: 256 floats each; layer 2 after them
-      mbar_wait_idle(&bars->acc_full[slot], (st >> 1) & 1);
+      mbar_wait(&bars->acc_full[slot], (st >> 1) & 1);
       tc_fence_after_sync();
       if (k < 2) {   // the H buffer must be free: h1 of the previous tile (k = 0) / h0 of this tile (k = 1) consumed
         if (hfree > 0) mbar_wait(&bars->h_free, (hfree - 1) & 1);
@@ -373,9 +351,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
           __syncwarp();
           if (lane == 0) mbar_arrive(&bars->h_full[c0 >> 6]);   // this warp's half of chunk c0 / 64 is in place
         } else {
-          const uint32_t tbuf = tbuf0 + (nstore % TBUFS) * TBUF_BYTES;
-          ++nstore;
-          if (lane == 0) bulk_wait_read_n<TBUFS - 1>();   // the store that last used this buffer is done reading it
+          if (lane == 0) bulk_wait_read0();   // the warp's previous store is done reading the tile
           __syncwarp();
 #pragma unroll
           for (int e = 0; e < 4; ++e) sts128(tbuf + lane * 64 + ((e ^ sw) << 4), w[e]);

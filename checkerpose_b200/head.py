@@ -17,7 +17,6 @@ on the implicit-GEMM form of ``cp_gemm_x3``.
 from __future__ import annotations
 
 import contextlib
-import os
 
 import torch
 import torch.nn as nn
@@ -532,18 +531,11 @@ class _OwnConvSeq:
         return y.permute(0, 3, 1, 2)
 
 
-# Fused upsampling + first convolution of an up_net block (cp_conv_slab with up_a: bit-identical, one launch and no
-# intermediate map).  Measured inside the step (DESIGN.md section 8): the 8 interpolating loader warps cannot feed the pair
-# MMA -- each slab row is interpolated twice (tile halo) and the tensor pipe consumes a slab in ~4600 clk -- so the two fused
-# convolutions lose 0.8 ms where the stand-alone upsampling kernels cost 0.55 ms.  Opt-in.
-_FUSE_UPSAMPLE = os.environ.get("CP_FUSE_UPSAMPLE", "0") == "1"
-
-
 class _SlabConvSeq(_OwnConvSeq):
     """The bf16 image branch on cp_conv_slab: every map of a block lives in a BORDERED NHWC buffer (B, H+1, W+1, C) -- a zero
     last row and last column per image, which over the flat pixel index are all four borders at once -- so that a kernel tap is
     a row shift of one TMA-loaded activation slab (csrc/conv_slab_tcgen05.cu).  The x2 upsampling of the concatenated skip
-    connection is fused into the block's first convolution (its loader warps interpolate the slab), 3x3 / 1x1 convolutions map buffer to buffer (their epilogue rewrites the border as zeros),
+    connection writes straight into a bordered buffer (cp_upsample2x_cat_nhwc_to), 3x3 / 1x1 convolutions map buffer to buffer (their epilogue rewrites the border as zeros),
     the transposed convolution of the first block runs as its four output parities, and patch_generator (2x2, padding 1)
     produces exactly the stored grid as a contiguous (B, H+1, W+1, E) map.  The NCHW view handed back to the caller is the interior of the
     buffer and remembers it (``_cp_padded``): the next block / patch_generator / seg_block pick the buffer up again
@@ -578,18 +570,8 @@ class _SlabConvSeq(_OwnConvSeq):
         buf = None          # zero-bordered (B,H+2,W+2,C) map, or None while y (plain NHWC) holds the current map
         y = None
         if kinds[0][0] == "up":
-            a, s = self._cl(x), None if skip is None else self._cl(skip)
-            nxt = kinds[1] if len(kinds) > 1 else None
-            ct = a.shape[1] + (0 if s is None else s.shape[1])
-            if (_FUSE_UPSAMPLE and nxt is not None and nxt[0] == "conv" and nxt[3][0] <= 256 and nxt[3][1] == nxt[3][2] and nxt[3][1] in (1, 3)
-                    and nxt[3][3] == nxt[3][1] // 2 and nxt[3][4] == ct and a.shape[1] % 64 == 0):
-                # the x2 upsampling happens inside the first convolution's loader warps: no intermediate map
-                _, ws, b, (cout, kh, kw, pad, cin_pad), relu = nxt
-                buf = ops.conv_slab_same_up(a, s, ws, cout, kh, kw, b, relu, 0.0)
-                start = 2
-            else:
-                buf = ops.upsample2x_cat_padded(a, s)
-                start = 1
+            buf = ops.upsample2x_cat_padded(self._cl(x), None if skip is None else self._cl(skip))
+            start = 1
         elif kinds[0][0] == "convT" and kinds[0][3][1:4] == (3, 3, 1) and kinds[0][3][0] <= 256:
             _, ws, b, (cout, kh, kw, pad, cin_pad), relu = kinds[0]
             if skip is not None:

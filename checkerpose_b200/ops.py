@@ -403,43 +403,6 @@ def conv_slab_same(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0, 
     return out if seg is None else (out, seg_out)
 
 
-def conv_slab_same_up(a, b, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0):
-    """conv_slab_same(upsample2x_cat_padded(a, b), ...) in ONE launch: the kernel's loader warps interpolate every activation
-    slab from the low-resolution sources (bit-identical to the stand-alone upsampling's bf16 values), so the (B, 2H+1, 2W+1,
-    Ca+Cb) map is never written to or read back from HBM.  a, b: channels_last (B,C,H,W) bf16 views; Ca % 64 == 0."""
-    _need_cuda(a, b, bias, w_packed)
-    B, Ca, H, W = a.shape
-    Cb = 0 if b is None else b.shape[1]
-    if a.dtype != torch.bfloat16 or (b is not None and (b.shape[0] != B or b.shape[2:] != a.shape[2:] or b.dtype != a.dtype)):
-        raise RuntimeError("conv_slab_same_up: sources disagree in shape or dtype")
-    assert KH % 2 == 1 and KW % 2 == 1 and KH <= 3 and KW <= 3
-    Hp, Wp, Cin = 2 * H + 1, 2 * W + 1, Ca + Cb
-    p = ConvSlabParams()
-    p.x, p.B, p.Hp, p.Wp, p.C, p.ldx = None, B, Hp, Wp, Cin, Cin
-    p.w_packed, p.K = _p(w_packed), KH * KW * Cin
-    p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
-    p.Nout = int(nout)
-    out = torch.empty((B, Hp, Wp, nout), dtype=torch.bfloat16, device=a.device)
-    p.out, p.ld_out = _p(out), int(nout)
-    p.num_phases = 1
-    ph = p.phase[0]
-    ph.ntaps = KH * KW
-    for ky in range(KH):
-        for kx in range(KW):
-            t = ky * KW + kx
-            ph.wtap[t] = t
-            ph.shift[t] = (ky - KH // 2) * Wp + (kx - KW // 2)
-    p.vy0, p.vy1, p.vx0, p.vx1 = 0, Hp - 1, 0, Wp - 1
-    p.compact = 0
-    sa = _nhwc_strides(a)
-    sb = (0, 0, 0) if b is None else _nhwc_strides(b)
-    p.up_a, p.up_a_sb, p.up_a_sh, p.up_a_sw, p.up_Ca = _p(a), sa[0], sa[1], sa[2], Ca
-    p.up_b, p.up_b_sb, p.up_b_sh, p.up_b_sw, p.up_Cb = _p(b), sb[0], sb[1], sb[2], Cb
-    p.up_H, p.up_W = H, W
-    _conv_slab(p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * (Hp - 1) * (Wp - 1) * KH * KW * Cin * int(nout)))
-    return out
-
-
 def conv_slab_full(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0):
     """Conv2d 2 x 2, stride 1, padding 1 (patch_generator, pipeline.py:144-145) over a bordered bf16 map xp (B, H+1, W+1, Cin)
     -> contiguous (B, H+1, W+1, nout): output (oy, ox) reads pixels (oy-1+ky, ox-1+kx), so the output grid IS the stored grid

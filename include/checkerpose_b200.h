@@ -169,14 +169,6 @@ typedef struct {
   int num_phases; cp_slab_phase phase[CP_SLAB_MAX_PHASES];
   int vy0, vy1, vx0, vx1;
   int compact; int64_t out_sb; int out_sy, out_sx;
-  /* Fused activation source (up_a != NULL; x is ignored): the map is the bordered (B, 2*up_H+1, 2*up_W+1, up_Ca+up_Cb) image
-   * of cp_upsample2x_cat_nhwc(up_a, up_b) -- nn.UpsamplingBilinear2d(2) of the concatenated skip connection, pipeline.py:201,372 --
-   * interpolated slab by slab inside the kernel (bit-identical to the stand-alone kernel's bf16 result) instead of being
-   * written to and read back from HBM.  Hp = 2*up_H+1, Wp = 2*up_W+1, C = up_Ca+up_Cb; up_Ca % 64 == 0; NHWC views with
-   * element strides (sb, sh, sw), channel stride 1. */
-  const void* up_a; int64_t up_a_sb, up_a_sh, up_a_sw; int up_Ca;
-  const void* up_b; int64_t up_b_sb, up_b_sh, up_b_sw; int up_Cb;
-  int up_H, up_W;
   /* Fused 1x1 head on the convolution's own output (seg_w != NULL; needs compact == 0): seg_block of pipeline.py:349,383.
    * seg_out[b, j, py - vy0, px - vx0] = seg_b[j] + sum_n bf16(out[g, n]) * seg_w[j, n]  (fp32, NCHW (B, seg_n, vy1-vy0, vx1-vx0)),
    * computed in the epilogue from the values being stored: the map is not read again.  seg_n <= 4. */

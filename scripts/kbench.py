@@ -48,37 +48,6 @@ def main():
         out = torch.empty((B, N, 2 * C), dtype=torch.bfloat16, device=dev)
         t = timed(lambda: ops.edgeconv_fwd(z=z, plan=plan, graph_sel=None, agg_slope=0.2, layer=layer, out=out, out_mode=ops.OUT_BF16))
         print(f"[{tag}] K2 256->[P|Q]512      {t:.4f} ms/launch  checksum {checksum(out)}")
-        from checkerpose_b200._lib import lib
-        if hasattr(lib, "cp_debug_read_phases"):      # CP_PROFILE_PHASES builds
-            import ctypes
-            buf = (ctypes.c_ulonglong * 16)()
-            lib.cp_debug_read_phases(buf)
-            ops.edgeconv_fwd(z=z, plan=plan, graph_sel=None, agg_slope=0.2, layer=layer, out=out, out_mode=ops.OUT_BF16)
-            lib.cp_debug_read_phases(buf)
-            tiles = B * (N // 128)
-            rounds = tiles * 4 * 16
-            names = ["-", "-", "stg_full wait", "Q+reduce", "a_empty wait", "finish+store+arrive"]
-            print("   aggregator, clk per warp-round: " + ", ".join(f"{n} {buf[i] / rounds:.0f}" for i, n in enumerate(names) if n != "-"))
-            print(f"   epilogue, clk per warp-tile: waiting for accumulator blocks {buf[6] / tiles / 8:.0f}, tile total {buf[7] / tiles / 8:.0f}")
-        if hasattr(lib, "cp_debug_read_trace"):       # CP_TRACE builds: timeline of CTA 0, tiles 8..11
-            import ctypes
-            buf = (ctypes.c_longlong * 8192)()
-            lib.cp_debug_read_trace(buf, 8192)
-            tr = [list(buf[r * 1024:(r + 1) * 1024]) for r in range(8)]
-            t0 = tr[1][8 * 4 * 4]
-            for ti in range(8, 12):
-                print(f"   tile {ti}")
-                for c in range(4):
-                    it = ti * 4 + c
-                    a0 = [tr[1][it * 4 + k] - t0 for k in range(4)]
-                    a15 = [tr[2][it * 4 + k] - t0 for k in range(4)]
-                    st = [tr[5][it * 2 + k] - t0 for k in range(2)]
-                    print(f"     round {it}: agg0 start {a0[0]:7d} stg_ok {a0[1]:7d} reduced {a0[2]:7d} a_empty_ok {a0[3]:7d} | agg15 {a15[0]:7d} {a15[1]:7d} {a15[2]:7d} {a15[3]:7d}"
-                          f" | stager space_ok {st[0]:7d} issued {st[1]:7d}")
-                e0 = [tr[3][ti * 8 + k] - t0 for k in range(8)]
-                e7 = [tr[4][ti * 8 + k] - t0 for k in range(8)]
-                print(f"     epilogue warp0 blocks (cols 0,64,..): {e0[0::1]}")
-                print(f"     epilogue warp7 blocks (cols 32,96,..): {e7[0::1]}")
         wq = torch.randn(C, C, generator=g) / C ** 0.5
         layer_q = ops.chain_layer(ops.pack_weight(wq.to(dev)), torch.randn(C, generator=g).to(dev), C, C, True, 0.01)
         a_out = torch.empty((B, N, C), dtype=torch.bfloat16, device=dev)

@@ -1,5 +1,5 @@
 """Slab convolution (cp_conv_slab) at the image-branch shapes of the benchmark configuration: error against float64 on a
-small case for every variant (single CTA / CTA pair, the descriptor's base-offset field on / off), then time next to the
+small case (single CTAs or CTA pairs, as CP_SLAB_PAIR selects), then time next to the
 gather kernel cp_conv_bf16 and cuDNN: python scripts/kbench_slab.py"""
 import os
 import sys
@@ -56,7 +56,7 @@ def check(dev, g):
 def main():
     dev = torch.device("cuda", 0)
     g = torch.Generator(device=dev).manual_seed(3)
-    print(f"variant pair={os.environ.get('CP_SLAB_PAIR', '1')} base_offset={os.environ.get('CP_SLAB_BASEOFF', '1')}")
+    print(f"variant pair={os.environ.get('CP_SLAB_PAIR', '1')}")
     check(dev, g)
     if os.environ.get("KB_CHECK_ONLY"):
         return

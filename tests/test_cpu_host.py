@@ -35,6 +35,43 @@ def test_library_exports_every_declared_symbol():
     assert set(names) <= exported
 
 
+# ctypes structure of checkerpose_b200/_lib.py -> its typedef in include/checkerpose_b200.h
+ABI_STRUCTS = {
+    "ChainLayer": "cp_chain_layer", "ChainParams": "cp_chain_params", "GraphPlanStruct": "cp_graph_plan",
+    "EdgeConvParams": "cp_edgeconv_params", "GemmX3Params": "cp_gemm_x3_params", "ConvBf16Params": "cp_conv_bf16_params",
+    "SlabPhase": "cp_slab_phase", "ConvSlabParams": "cp_conv_slab_params", "QueryDecodeParams": "cp_query_decode_params",
+}
+
+
+def test_ctypes_structures_match_the_header_layout(tmp_path):
+    """Every parameter struct passed by pointer has the same size and field offsets in ctypes as in the C header (compiled
+    with the host C compiler); a mismatch would otherwise only show on the GPU as garbage in the fields behind it."""
+    import ctypes
+    from checkerpose_b200 import _lib
+    structs = sorted(n for n, v in vars(_lib).items() if isinstance(v, type) and issubclass(v, ctypes.Structure) and v is not ctypes.Structure)
+    assert structs == sorted(ABI_STRUCTS)
+    lines, expect = [], []
+    for py_name, c_name in ABI_STRUCTS.items():
+        cls = getattr(_lib, py_name)
+        lines.append(f'printf("%zu\\n", sizeof({c_name}));')
+        expect.append((c_name, ctypes.sizeof(cls)))
+        for field, _ in cls._fields_:
+            lines.append(f'printf("%zu %zu\\n", offsetof({c_name}, {field}), sizeof((({c_name}*)0)->{field}));')
+            desc = getattr(cls, field)
+            expect.append((f"{c_name}.{field} (offset, size)", f"{desc.offset} {desc.size}"))
+    src = tmp_path / "layout.c"
+    src.write_text("#include <stddef.h>\n#include <stdio.h>\n#include \"checkerpose_b200.h\"\nint main(void) {\n  "
+                   + "\n  ".join(lines) + "\n  return 0;\n}\n")
+    exe = tmp_path / "layout"
+    cc = subprocess.run([os.environ.get("CC", "gcc"), "-std=c99", "-Wall", "-Werror", "-I", os.path.join(REPO, "include"),
+                         "-o", str(exe), str(src)], capture_output=True, text=True)
+    assert cc.returncode == 0, cc.stderr      # a ctypes field the header does not have fails here
+    got = subprocess.run([str(exe)], capture_output=True, text=True, check=True).stdout.splitlines()
+    assert len(got) == len(expect)
+    for (what, want), line in zip(expect, got):
+        assert line == str(want), f"{what}: header {line}, ctypes {want}"
+
+
 def test_library_is_sm100a_with_blackwell_instructions():
     from checkerpose_b200 import _lib
     r = subprocess.run(["cuobjdump", "-lelf", _lib.LIB_PATH], capture_output=True, text=True)

@@ -281,24 +281,6 @@ def test_plan_above_limit_is_refused_and_falls_back(ops):
         run_case(ops, plan, idx, [1, 0, 1], 3, Co, nout, seed=Co, tag=f"U=513 chain fallback Co={Co} nout={nout}", kernel="chain")
 
 
-# ------------------------------------------------------------------------------------------------ CTA pairs
-@gpu
-@pytest.mark.parametrize("KP", KPS)
-def test_edgeconv_cta_pair_every_kp(ops, monkeypatch, KP):
-    """CP_EDGECONV_PAIR=1 == the single-CTA kernel bit for bit at every KP: 15 tiles (odd: the last pair repeats a
-    tile), a ragged last tile, half of the tiles above R/2 (one round in flight)."""
-    R = int(ops.lib.cp_edgeconv_ring_rows(KP))
-    idx, plan = synthetic_graph(ops, 2, 600, KP, lambda g, t, nv: (KP * 3, R // 2 + 1)[(g + t) % 2], seed=KP)
-    assert plan.staged and plan.T * 3 % 2 == 1 and plan.max_unique > R // 2
-    sel = [1, 0, 1]
-    for Co, nout in ((128, 256), (64, 7), (256, 128)):
-        res = []
-        for pair in ("0", "1"):
-            monkeypatch.setenv("CP_EDGECONV_PAIR", pair)
-            res.append(run_case(ops, plan, idx, sel, 3, Co, nout, seed=KP + Co, tag=f"pair={pair} KP={KP} Co={Co} nout={nout}"))
-        assert torch.equal(res[0][0], res[1][0]) and torch.equal(res[0][1].nan_to_num(), res[1][1].nan_to_num()), (KP, Co, nout)
-
-
 # ------------------------------------------------------------------------------------------------ fallbacks
 @gpu
 @pytest.mark.parametrize("K", [40, 41, 64])

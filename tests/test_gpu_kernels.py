@@ -474,31 +474,6 @@ def test_conv_slab_matches_fp64(cp, monkeypatch, pair, kind, B, H, W, Cin, Cout)
 
 
 @pytest.mark.parametrize("pair", ["1", "0"])
-@pytest.mark.parametrize("B,H,W,Ca,Cb,Cout,k", [(3, 8, 8, 128, 64, 256, 3), (2, 16, 16, 256, 256, 256, 3), (5, 5, 7, 64, 0, 64, 3), (2, 32, 32, 64, 64, 32, 1)])
-def test_conv_slab_fused_upsample_is_bit_identical(cp, monkeypatch, pair, B, H, W, Ca, Cb, Cout, k):
-    """The convolution whose loader warps interpolate the x2-upsampled, concatenated map on the fly must equal, bit for bit,
-    the same convolution over the map written by the stand-alone upsampling kernel (same bf16 activations, same MMA order)."""
-    ops = cp.ops
-    monkeypatch.setenv("CP_SLAB_PAIR", pair)
-    g = torch.Generator().manual_seed(B + H + Ca + Cout)
-    a = torch.randn(B, H, W, Ca, generator=g).to(torch.bfloat16).cuda().permute(0, 3, 1, 2)
-    b = torch.randn(B, H, W, Cb, generator=g).to(torch.bfloat16).cuda().permute(0, 3, 1, 2) if Cb else None
-    if (Ca + Cb) % 64:
-        pytest.skip("channel count not a multiple of 64")
-    w = torch.randn(Cout, k * k * (Ca + Cb), generator=g) / (k * k * (Ca + Cb)) ** 0.5
-    bias = torch.randn(Cout, generator=g).cuda()
-    wp = ops.pack_weight(w.cuda())
-    two = ops.conv_slab_same(ops.upsample2x_cat_padded(a, b), wp, Cout, k, k, bias, True, 0.0)
-    one = ops.conv_slab_same_up(a, b, wp, Cout, k, k, bias, True, 0.0)
-    assert one.shape == two.shape == (B, 2 * H + 1, 2 * W + 1, Cout)
-    assert torch.equal(one, two)
-    # a strided source: the interior of a bordered map
-    buf = ops.to_bordered(a.permute(0, 2, 3, 1)).contiguous()
-    view = buf[:, :-1, :-1].permute(0, 3, 1, 2)
-    assert torch.equal(ops.conv_slab_same_up(view, b, wp, Cout, k, k, bias, True, 0.0), two)
-
-
-@pytest.mark.parametrize("pair", ["1", "0"])
 @pytest.mark.parametrize("B,H,W,Cin,Cout,nseg", [(3, 16, 16, 128, 256, 2), (2, 9, 11, 64, 64, 1), (2, 12, 12, 64, 256, 4)])
 def test_conv_slab_fused_seg_head(cp, monkeypatch, pair, B, H, W, Cin, Cout, nseg):
     """seg_block (1x1) computed in the last convolution's epilogue: equals the 1x1 convolution of the bf16 map the same launch
@@ -678,37 +653,6 @@ def _fixture_plan(cp, ds, objs, N, K):
     plan = cp.ops.GraphPlan(idx.to(torch.int32).cuda(), p3d)
     assert plan.staged
     return plan
-
-
-@pytest.mark.parametrize("N,B,nout", [(4096, 3, 512), (300, 5, 256), (512, 2, 16), (640, 1, 128)])
-def test_edgeconv_cta_pair_matches_single_cta(cp, monkeypatch, N, B, nout):
-    """The CTA-pair variant of the staged EdgeConv kernel (cluster of 2, tcgen05.mma.cta_group::2, M = 256: opt-in with
-    CP_EDGECONV_PAIR=1) equals the single-CTA kernel bit for bit, incl. odd tile counts (the last pair repeats a tile),
-    ragged last tiles, and outputs of 16 / 128 / 256 / 512 columns."""
-    ops = cp.ops
-    C = 256 if nout != 128 else 64
-    if nout == 16:
-        C = 64
-    p3d = syn.p3d_normed_tensor(syn.load_fps_xyz("lmo", 1, N)).cuda()
-    _, idx32 = ops.knn(p3d, 20, want_i32=True)
-    plan = ops.GraphPlan(idx32, p3d)
-    g = torch.Generator().manual_seed(N + nout)
-    z = torch.randn(B, N, 2 * C, generator=g).to(torch.bfloat16).cuda()
-    w = torch.randn(nout, C, generator=g) / C ** 0.5
-    bias = torch.randn(nout, generator=g).cuda()
-    layer = ops.chain_layer(ops.pack_weight(w.cuda()), bias, C, nout, nout != 16, 0.01)
-    outs = []
-    for pair in ("0", "1"):
-        monkeypatch.setenv("CP_EDGECONV_PAIR", pair)
-        if nout == 16:
-            out = torch.zeros((B, N, 16), dtype=torch.float32, device="cuda")
-            ops.edgeconv_fwd(z=z, plan=plan, graph_sel=None, agg_slope=0.2, layer=layer, out=out, out_mode=ops.OUT_F32, n_valid=7)
-        else:
-            out = torch.zeros((B, N, nout), dtype=torch.bfloat16, device="cuda")
-            ops.edgeconv_fwd(z=z, plan=plan, graph_sel=None, agg_slope=0.2, layer=layer, out=out, out_mode=ops.OUT_BF16)
-        outs.append(out.clone())
-    assert torch.isfinite(outs[0].float()).all() and float(outs[0].float().abs().sum()) > 0
-    assert torch.equal(outs[0], outs[1])
 
 
 @pytest.mark.parametrize("ds,objs,N,K,Co,Nout,B,out_f32", [

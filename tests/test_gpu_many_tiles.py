@@ -49,9 +49,9 @@ def cdiv(a, b):
 # ------------------------------------------------------------------------------------------------ launch geometry
 def grid_of(rule, work, S):
     """The launchers' grid rules.  ``work`` = tiles, or units / tile pairs for the cluster kernels.
-    sm:   min(tiles, S)        cp_gemm_x3, cp_conv_bf16 (single CTA), cp_conv_slab (single), K3, K4, cp_edgeconv_fwd (single)
+    sm:   min(tiles, S)        cp_gemm_x3, cp_conv_bf16 (single CTA), cp_conv_slab (single), K3, K4, cp_edgeconv_fwd
     2sm:  min(tiles, 2S)       cp_chain_fwd, cp_edge_aggregate_staged_f32 with <= 110 KB of shared memory
-    half: min(units, S/2)      clusters of cp_conv_slab (pair), of cp_conv_bf16 (multicast), of cp_edgeconv_fwd (pair)"""
+    half: min(units, S/2)      clusters of cp_conv_slab (pair), of cp_conv_bf16 (multicast)"""
     cap = {"sm": S, "2sm": 2 * S, "half": S // 2}[rule]
     return min(work, cap)
 
@@ -609,8 +609,7 @@ def test_edge_aggregate_staged_f32_many_tiles(ops, K):
     report(tag, work, grid, per, 0.0)
 
 
-@pytest.mark.parametrize("pair", ["0", "1"])
-def test_edgeconv_staged_many_tiles(ops, monkeypatch, pair):
+def test_edgeconv_staged_many_tiles(ops):
     """cp_edgeconv_fwd at the benchmark's refine shape: N = 4096, K = 20, Co = 256 -> 512 bf16 with a_out."""
     S = num_sms()
     N, K, B, Co, nout = 4096, 20, 24, 256, 512
@@ -620,14 +619,9 @@ def test_edgeconv_staged_many_tiles(ops, monkeypatch, pair):
     assert plan.staged
     tpr = plan.T
     tiles = B * tpr
-    monkeypatch.setenv("CP_EDGECONV_PAIR", pair)
-    if pair == "1":
-        work, cap = cdiv(tiles, 2), S - S % 2
-        grid = grid_of("half", work, S)
-    else:
-        work, cap = tiles, S
-        grid = grid_of("sm", work, S)
-    tag = f"edgeconv pair={pair} N={N} K={K} B={B}"
+    work, cap = tiles, S
+    grid = grid_of("sm", work, S)
+    tag = f"edgeconv N={N} K={K} B={B}"
     per = check_waves(tag, work, grid)
     g = torch.Generator().manual_seed(20)
     z = bf16r(torch.randn(B, N, 2 * Co, generator=g))
@@ -645,7 +639,7 @@ def test_edgeconv_staged_many_tiles(ops, monkeypatch, pair):
     parts = [run(b0, b1) for b0, b1 in roi_chunks(B, tpr, cap)]
     assert torch.equal(a_big, torch.cat([p[0] for p in parts])) and torch.equal(big, torch.cat([p[1] for p in parts])), \
         "the multi-wave launch differs from one-tile-per-CTA launches"
-    last = sampled_tiles(tiles, 2 * grid if pair == "1" else grid)
+    last = sampled_tiles(tiles, grid)
     bi, ni = roi_rows(last, N)
     nb = plan.idx_p.cpu().long().expand(B, -1, -1)
     a_ref = agg_rows(z, nb, bi, ni, Co, 0.2, True)
