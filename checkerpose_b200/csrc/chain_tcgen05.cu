@@ -44,18 +44,12 @@ constexpr int MAX_WTILES = 48;
 constexpr int SMEM_BYTES = A_CHUNKS * A_CHUNK_BYTES + STAGES * B_STAGE_BYTES + 256;
 static_assert(2 * (SMEM_BYTES + 1024) <= 227 * 1024, "two CTAs per SM");
 
-struct WTile {
-  const uint8_t* ptr;
-  uint32_t bytes;  // rows * 128
-  uint32_t pad;
-};
-
 struct KParams {
   cp_chain_params p;
   int tiles_per_roi;
   int num_node_tiles;
   int T;  // weight tiles per node tile
-  WTile wt[MAX_WTILES];
+  cp::WTile wt[MAX_WTILES];
 };
 
 struct Smem {
@@ -71,23 +65,10 @@ __device__ __forceinline__ uint32_t a_offset(int kc, int row, int chunk) {
   return (uint32_t)(kc * A_CHUNK_BYTES + row * 128 + ((chunk ^ (row & 7)) << 4));
 }
 
-__device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {
-  uint4 r;
-  asm volatile("ld.global.nc.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-  return r;
-}
-
 __device__ __forceinline__ uint32_t bf2_max(uint32_t a, uint32_t b) {
   __nv_bfloat162 x = *reinterpret_cast<__nv_bfloat162*>(&a), y = *reinterpret_cast<__nv_bfloat162*>(&b);
   __nv_bfloat162 m = __hmax2(x, y);
   return *reinterpret_cast<uint32_t*>(&m);
-}
-__device__ __forceinline__ float2 bf2_to_f2(uint32_t a) {
-  return __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&a));
-}
-__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
 }
 
 // ---- prologues: all 256 threads fill A chunks [0, C/64) for the 128 rows of the tile -----------------
@@ -104,7 +85,7 @@ __device__ __forceinline__ void fill_rows(uint8_t* A, const bf16* src, int ld, i
   for (int r = warp * rpi + sub; r < TILE_M; r += NWARPS * rpi) {
     const bool ok = r < rows_valid;
     const void* g = src + (ok ? (row0 + r) * ld + chunk * 8 : 0);
-    asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(a_s + a_offset(chunk >> 3, r, chunk & 7)), "l"(g), "r"(ok ? 16u : 0u) : "memory");
+    cp_async16_zfill(a_s + a_offset(chunk >> 3, r, chunk & 7), g, ok ? 16u : 0u);
   }
   asm volatile("cp.async.commit_group;" ::: "memory");
   asm volatile("cp.async.wait_group 0;" ::: "memory");
@@ -337,7 +318,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) chain_kernel(const __grid_constan
               tc_fence_after_sync();
               for (int nbi = 0; nbi < nblk; ++nbi) {
                 for (int kci = 0; kci < kc_count; ++kci) {
-                  const WTile& wt = kp.wt[widx + nbi * kc_count + kci];
+                  const cp::WTile& wt = kp.wt[widx + nbi * kc_count + kci];
                   const long long it = mc + nbi * kc_count + kci;
                   const int s = (int)(it % STAGES);
                   mbar_wait(&sm.full[s], (uint32_t)((it / STAGES) & 1));
@@ -368,7 +349,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) chain_kernel(const __grid_constan
                 const int s = (int)(pc % STAGES);
                 const long long use = pc / STAGES;
                 if (use > 0) mbar_wait(&sm.empty[s], (uint32_t)((use - 1) & 1));
-                const WTile& wt = kp.wt[(int)(pc % kp.T)];
+                const cp::WTile& wt = kp.wt[(int)(pc % kp.T)];
                 if (elect_one()) {
                   mbar_arrive_expect_tx(&sm.full[s], wt.bytes);
                   bulk_g2s(sm.Bst + s * B_STAGE_BYTES, wt.ptr, wt.bytes, &sm.full[s]);
@@ -465,7 +446,6 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
     const bool two_phase = (p.prologue == CP_PRO_TAPS && l == 0);
     CP_REQUIRE(two_phase || L.kin <= 256, CP_E_UNSUPPORTED, "cp_chain_fwd: layer %d kin=%d > 256", l, L.kin);
     const int npass = (npad + TMEM_COLS - 1) / TMEM_COLS;
-    const uint8_t* wbase = reinterpret_cast<const uint8_t*>(L.w_packed);
     for (int pass = 0; pass < npass; ++pass) {
       const int col0 = pass * TMEM_COLS;
       const int pcols = (npad - col0 < TMEM_COLS) ? (npad - col0) : TMEM_COLS;
@@ -475,15 +455,9 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
         const int kc_begin = (two_phase && ph == 1) ? 4 : 0;
         const int kc_count = two_phase ? (ph == 0 ? 4 : p.Cg / 64) : L.kin / 64;
         for (int nbi = 0; nbi < nblk; ++nbi) {
-          const int nb = col0 / 128 + nbi;
-          const int rows = (npad - nb * 128 < 128) ? (npad - nb * 128) : 128;
           for (int kci = 0; kci < kc_count; ++kci) {
             CP_REQUIRE(T < MAX_WTILES, CP_E_UNSUPPORTED, "cp_chain_fwd: weight tile table overflow");
-            const int kc = kc_begin + kci;
-            kp.wt[T].ptr = wbase + (size_t)nb * 128 * L.kin * 2 + (size_t)kc * rows * 128;
-            kp.wt[T].bytes = (uint32_t)rows * 128;
-            kp.wt[T].pad = 0;
-            ++T;
+            kp.wt[T++] = cp::packed_tile(L.w_packed, col0 / 128 + nbi, kc_begin + kci, L.kin, npad);
           }
         }
       }

@@ -49,6 +49,28 @@ int num_sms();
 
 static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
+// Packed weight layout, written by cp_pack_weight / cp_pack_weight_split and sized by cp_packed_weight_bytes: an (Nout x K)
+// matrix, K a multiple of 64, zero-padded to npad = Nout rounded up to 16 rows, in bf16.  The rows form blocks of 128 (the
+// last block holds the npad - 128 nb rows left), each block is stored as its K chunks of 64 columns one after the other,
+// and a chunk of `rows` rows is a rows x 128-byte tile in the K-major SWIZZLE_128B layout tcgen05.mma reads: row r at
+// r * 128, its 16-byte piece j at ((j ^ (r & 7)) << 4).  One bulk copy moves one tile into shared memory.
+__host__ __device__ __forceinline__ int packed_block_rows(int nb, int npad) { return npad - 128 * nb < 128 ? npad - 128 * nb : 128; }
+// byte offset of the tile of block nb (rows = packed_block_rows(nb, npad)), K chunk kc
+__host__ __device__ __forceinline__ size_t packed_tile_offset(size_t nb, size_t kc, size_t rows, size_t K) {
+  return nb * 128 * K * 2 + kc * rows * 128;
+}
+
+// One packed weight tile in the tile tables of the persistent kernels (pad keeps the entries 16 bytes)
+struct WTile {
+  const uint8_t* ptr;
+  uint32_t bytes;
+  uint32_t pad;
+};
+static inline WTile packed_tile(const void* w_packed, int nb, int kc, int K, int npad) {
+  const int rows = packed_block_rows(nb, npad);
+  return {static_cast<const uint8_t*>(w_packed) + packed_tile_offset(nb, kc, rows, K), (uint32_t)rows * 128u, 0u};
+}
+
 __device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.f ? v : v * slope; }
 
 template <typename T> __device__ __forceinline__ float to_f32(T v);

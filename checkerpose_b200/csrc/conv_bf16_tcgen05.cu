@@ -80,33 +80,6 @@ struct TileIt {
   }
 };
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void cp_async16_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-
 // ------------------------------------------------------------------------------------------------------
 // A loaders
 // ------------------------------------------------------------------------------------------------------
@@ -229,8 +202,8 @@ __device__ void weight_producer(const CvParams& kp, uint8_t* sm, Bars* bars) {
           uint8_t* w_s = sm + s * STAGE_BYTES + A_BYTES;
           const uint32_t half = (uint32_t)(cols / 2) * 128u, rank = blockIdx.x & 1;
           mbar_arrive_expect_tx(&bars->full[s], (uint32_t)cols * 128u);
-          const uint8_t* src = cols == 256 ? wb + (size_t)rank * 128 * p.K * 2 + (size_t)kc * 128 * 128     // packed 128-row block `rank`
-                                           : wb + (size_t)kc * cols * 128 + (size_t)rank * half;               // half of the single block
+          const uint8_t* src = cols == 256 ? wb + cp::packed_tile_offset(rank, kc, 128, p.K)                 // packed 128-row block `rank`
+                                           : wb + cp::packed_tile_offset(0, kc, cols, p.K) + (size_t)rank * half;   // half of the single block
           bulk_g2s_multicast(w_s + rank * half, src, half, &bars->full[s], (uint16_t)3);
         }
         __syncwarp();
@@ -239,9 +212,9 @@ __device__ void weight_producer(const CvParams& kp, uint8_t* sm, Bars* bars) {
       if (elect_one()) {
         uint8_t* w_s = sm + s * STAGE_BYTES + A_BYTES;
         mbar_arrive_expect_tx(&bars->full[s], (uint32_t)cols * 128u);
-        bulk_g2s(w_s, wb + (size_t)(col0 / 128) * 128 * p.K * 2 + (size_t)kc * rows0 * 128, (uint32_t)rows0 * 128u, &bars->full[s]);
+        bulk_g2s(w_s, wb + cp::packed_tile_offset(col0 / 128, kc, rows0, p.K), (uint32_t)rows0 * 128u, &bars->full[s]);
         if (rows1 > 0)
-          bulk_g2s(w_s + 128 * 128, wb + (size_t)(col0 / 128 + 1) * 128 * p.K * 2 + (size_t)kc * rows1 * 128, (uint32_t)rows1 * 128u, &bars->full[s]);
+          bulk_g2s(w_s + 128 * 128, wb + cp::packed_tile_offset(col0 / 128 + 1, kc, rows1, p.K), (uint32_t)rows1 * 128u, &bars->full[s]);
       }
       __syncwarp();
     }
@@ -325,7 +298,7 @@ __device__ void epilogue(const CvParams& kp, const CUtensorMap* out_map, uint8_t
       if (kp.tma_out) {
         const uint32_t tbuf = tbuf0 + (nstore & 1) * EPI_TILE_BYTES;
         ++nstore;
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (lane == 0) bulk_wait_read<1>();
         __syncwarp();
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
@@ -336,9 +309,8 @@ __device__ void epilogue(const CvParams& kp, const CUtensorMap* out_map, uint8_t
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0 && row0 < p.M) {
-          asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                       ::"l"(out_map), "r"(tbuf), "r"(n0), "r"((int)row0), "r"(0) : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          tma_store_3d(out_map, tbuf, n0, (int)row0, 0);
+          bulk_commit();
         }
       } else if (row_ok) {
         bf16* orow = out + row * p.ld_out;
@@ -351,7 +323,7 @@ __device__ void epilogue(const CvParams& kp, const CUtensorMap* out_map, uint8_t
     __syncwarp();
     if (lane == 0) mbar_arrive(&bars->acc_empty[slot]);
   }
-  if (kp.tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+  if (kp.tma_out && lane == 0) bulk_wait_read<0>();
 }
 
 template <bool MC>

@@ -85,30 +85,6 @@ struct Units {
   }
 };
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(uint32_t smem_dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(smem_dst), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
 // ------------------------------------------------------------------------------------------------------
 template <bool PAIR>
 __device__ void slab_producer(const SlabParams& kp, const CUtensorMap* x_map, uint8_t* sm, Bars* bars) {
@@ -156,14 +132,15 @@ __device__ void weight_producer(const SlabParams& kp, uint8_t* sm, Bars* bars) {
             // this CTA's half of the tile's rows (= output columns): a whole 128-row block of the packed matrix when the tile
             // has 256 columns, half of the single block otherwise
             const uint32_t half = (uint32_t)(npad / 2) * 128u;
-            const uint8_t* src = npad == 256 ? wb + (size_t)rank * 128 * p.K * 2 + kc * 128 * 128 : wb + kc * npad * 128 + (size_t)rank * half;
+            const uint8_t* src = npad == 256 ? wb + cp::packed_tile_offset(rank, kc, 128, p.K)
+                                             : wb + cp::packed_tile_offset(0, kc, npad, p.K) + (size_t)rank * half;
             mbar_arrive_expect_tx(&bars->w_full[s], half);
             bulk_g2s(w_s, src, half, &bars->w_full[s]);
           } else {
             const int rows0 = min(128, npad), rows1 = npad - rows0;
             mbar_arrive_expect_tx(&bars->w_full[s], (uint32_t)npad * 128u);
-            bulk_g2s(w_s, wb + kc * rows0 * 128, (uint32_t)rows0 * 128u, &bars->w_full[s]);
-            if (rows1 > 0) bulk_g2s(w_s + 128 * 128, wb + (size_t)128 * p.K * 2 + kc * rows1 * 128, (uint32_t)rows1 * 128u, &bars->w_full[s]);
+            bulk_g2s(w_s, wb + cp::packed_tile_offset(0, kc, rows0, p.K), (uint32_t)rows0 * 128u, &bars->w_full[s]);
+            if (rows1 > 0) bulk_g2s(w_s + 128 * 128, wb + cp::packed_tile_offset(1, kc, rows1, p.K), (uint32_t)rows1 * 128u, &bars->w_full[s]);
           }
         }
         __syncwarp();
@@ -325,16 +302,15 @@ __device__ void epilogue(const SlabParams& kp, const CUtensorMap* out_map, uint8
       if (kp.tma_out) {
         const uint32_t tbuf = tbuf0 + (nstore & 1) * EPI_TILE_BYTES;
         ++nstore;
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");
+        if (lane == 0) bulk_wait_read<1>();
         __syncwarp();
 #pragma unroll
         for (int e = 0; e < 4; ++e) sts128(tbuf + lane * 64 + ((e ^ sw) << 4), make_uint4(w[e * 4], w[e * 4 + 1], w[e * 4 + 2], w[e * 4 + 3]));
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0 && row0 < kp.G) {
-          asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-                       ::"l"(out_map), "r"(tbuf), "r"(n0), "r"((int)row0), "r"(0) : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          tma_store_3d(out_map, tbuf, n0, (int)row0, 0);
+          bulk_commit();
         }
       } else if (p.compact ? valid : g < kp.G) {
         bf16* o = out + orow * p.ld_out + n0;
@@ -364,7 +340,7 @@ __device__ void epilogue(const SlabParams& kp, const CUtensorMap* out_map, uint8
         if (j < p.seg_n) p.seg_out[(((int64_t)b * p.seg_n + j) * Hs + (py - p.vy0)) * Ws + (px - p.vx0)] = seg_acc[j] + __ldg(p.seg_b + j);
     }
   }
-  if (kp.tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");
+  if (kp.tma_out && lane == 0) bulk_wait_read<0>();
 }
 
 template <bool PAIR>

@@ -8,6 +8,9 @@
 // once with cp.async (double-buffered over the slices), and a quarter-warp reduces one node PAIR of the plan's programs
 // (shared rows once) with 128-bit shared-memory loads.
 #include "common.cuh"
+#include "sm100.cuh"
+
+using sm100::cp_async16;
 
 namespace {
 
@@ -22,9 +25,6 @@ __device__ __forceinline__ float4 lds128f(uint32_t addr) {
 }
 __device__ __forceinline__ float4 max4(float4 a, float4 b) {
   return make_float4(fmaxf(a.x, b.x), fmaxf(a.y, b.y), fmaxf(a.z, b.z), fmaxf(a.w, b.w));
-}
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
 }
 
 __global__ void __launch_bounds__(NTHREADS, 2)

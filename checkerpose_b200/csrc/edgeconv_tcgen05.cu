@@ -84,12 +84,6 @@ __host__ __device__ constexpr int prog_bytes(int KCH) { return CP_PLAN_PAIRS * p
 __host__ __device__ constexpr int off_ring(int KCH) { return (OFF_PROG + 2 * prog_bytes(KCH) + 127) & ~127; }
 __host__ __device__ constexpr int ring_rows(int KCH) { return (SMEM_BYTES - 1024 - off_ring(KCH)) / 128; }
 
-struct WTile {
-  const uint8_t* ptr;
-  uint32_t bytes;  // rows * 128
-  uint32_t pad;
-};
-
 struct EcParams {
   cp_edgeconv_params p;
   int KC;            // 64-channel slices of the aggregated feature (= GEMM K chunks) = rounds per tile
@@ -99,7 +93,7 @@ struct EcParams {
   int tiles_per_roi;
   int tpr_shift;     // log2(tiles_per_roi) when it is a power of two (every shipped N), else -1
   int tma_out;       // bf16 output with nout % 32 == 0: the epilogue stores through the tensor map
-  WTile wt[MAX_WTILES];  // order: slice-major, then column block
+  cp::WTile wt[MAX_WTILES];  // order: slice-major, then column block
 };
 
 // Tiles of this CTA: blockIdx.x, then every gridDim.x-th tile.
@@ -136,16 +130,6 @@ __device__ __forceinline__ uint32_t bf2_max3(uint32_t a, uint32_t b, uint32_t c)
 __device__ __forceinline__ uint4 bf8_max3(uint4 a, uint4 b, uint4 c) {
   return make_uint4(bf2_max3(a.x, b.x, c.x), bf2_max3(a.y, b.y, c.y), bf2_max3(a.z, b.z, c.z), bf2_max3(a.w, b.w, c.w));
 }
-__device__ __forceinline__ float2 bf2_to_f2(uint32_t a) { return __bfloat1622float2(*reinterpret_cast<__nv_bfloat162*>(&a)); }
-__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-  uint4 r;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
-  return r;
-}
 __device__ __forceinline__ uint2 lds64(uint32_t addr) {
   uint2 r;
   asm volatile("ld.shared.v2.u32 {%0,%1}, [%2];" : "=r"(r.x), "=r"(r.y) : "r"(addr));
@@ -159,34 +143,7 @@ __device__ __forceinline__ uint32_t lds32(uint32_t addr) {
 __device__ __forceinline__ void sts32(uint32_t addr, uint32_t v) {
   asm volatile("st.shared.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
 }
-__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
-__device__ __forceinline__ uint4 ldg_nc_v4(const void* p) {
-  uint4 r;
-  asm volatile("ld.global.nc.L1::no_allocate.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "l"(p));
-  return r;
-}
 __device__ __forceinline__ void prefetch_l2(const void* p) { asm volatile("prefetch.global.L2 [%0];" ::"l"(p)); }
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-// cp.async (LDGSTS): 16 bytes per lane, no register staging; a warp instruction moves four 128-byte row slices.
-// (Measured on B200, scripts/ubench/membw.cu: per-row cp.async.bulk copies cost ~55 clk each on the issuing thread,
-// 2.3 B/clk/SM at 128 B pieces, so the TMA engine is kept for the 16 KB weight tiles.)
-__device__ __forceinline__ void cp_async16(uint32_t dst, const void* src) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16;" ::"r"(dst), "l"(src) : "memory");
-}
 
 __device__ __forceinline__ uint32_t a_offset(int buf, int row, int chunk) {
   return (uint32_t)(OFF_A + buf * A_BUF_BYTES + row * 128 + ((chunk ^ (row & 7)) << 4));
@@ -213,7 +170,7 @@ __device__ void weight_producer(const EcParams& kp, uint8_t* sm, Bars* bars) {
         const int s = cnt % B_STAGES;
         const uint32_t use = cnt / B_STAGES;
         if (use > 0) mbar_wait(&bars->b_empty[s], (use - 1) & 1);
-        const WTile& w = kp.wt[c * NB + nb];
+        const cp::WTile& w = kp.wt[c * NB + nb];
         if (elect_one()) {
           mbar_arrive_expect_tx(&bars->b_full[s], w.bytes);
           bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, w.ptr, w.bytes, &bars->b_full[s]);
@@ -367,7 +324,7 @@ __device__ void stager(const EcParams& kp, uint8_t* sm, Bars* bars, int pw, int 
         for (int piece = tid; piece < PROG_BYTES / 16; piece += STG_THREADS) cp_async16(pd + piece * 16, prog_src + piece * 16);
       }
       // asynchronous arrival: fires when all of this thread's copies so far have landed; nobody waits here
-      asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(&bars->stg_full[r % NBAR])) : "memory");
+      cp_async_arrive_noinc(&bars->stg_full[r % NBAR]);
     }
   }
 }
@@ -437,8 +394,8 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
       const uint32_t nr4 = (uint32_t)KCH - nc4;     // chunks of each node's own rows            }
       // own Q slices: issued first, their (L2) latency hides behind the row reads
       const bf16* zq = reinterpret_cast<const bf16*>(p.z) + p.Co + c * 64 + sub * 8;
-      const uint4 qa = na != 255 ? ldg_nc_v4(zq + (size_t)(row0 + na) * p.ld_z) : make_uint4(0, 0, 0, 0);
-      const uint4 qb = nb != 255 ? ldg_nc_v4(zq + (size_t)(row0 + nb) * p.ld_z) : make_uint4(0, 0, 0, 0);
+      const uint4 qa = na != 255 ? ldg_nc_na_v4(zq + (size_t)(row0 + na) * p.ld_z) : make_uint4(0, 0, 0, 0);
+      const uint4 qb = nb != 255 ? ldg_nc_na_v4(zq + (size_t)(row0 + nb) * p.ld_z) : make_uint4(0, 0, 0, 0);
 
       uint4 acc = make_uint4(NEG_INF2, NEG_INF2, NEG_INF2, NEG_INF2);
       uint32_t pa = pe;
@@ -479,13 +436,6 @@ __device__ void aggregator(const EcParams& kp, uint8_t* sm, Bars* bars, int aw, 
 // ------------------------------------------------------------------------------------------------------
 // epilogue: warp q drains TMEM lanes [32 q, 32 q + 32), 32 columns at a time
 // ------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t smem_src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(map), "r"(smem_src), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-
 template <bool ACT, bool TMA_OUT>
 __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, uint8_t* sm, Bars* bars, uint32_t tmem_base, int ew, int lane) {
   constexpr int ACC_BLK = 128;      // columns per accumulator block (= per MMA)
@@ -554,7 +504,7 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
       if (TMA_OUT) {
         // 32 rows x 64 B tile in the SWIZZLE_64B layout of the tensor map; the TMA engine writes it to
         // out[b, n0 + 32 q .. +32, c0 .. c0+32) and clips rows beyond N
-        if (lane == 0) bulk_wait_read0();   // the warp's previous store is done reading the tile
+        if (lane == 0) bulk_wait_read<0>();   // the warp's previous store is done reading the tile
         __syncwarp();
 #pragma unroll
         for (int e = 0; e < 4; ++e) {
@@ -590,7 +540,7 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
       }
     }
   }
-  if (TMA_OUT && lane == 0) bulk_wait_read0();   // shared memory must outlive the last stores' reads
+  if (TMA_OUT && lane == 0) bulk_wait_read<0>();   // shared memory must outlive the last stores' reads
 }
 
 template <int KCH>
@@ -724,15 +674,8 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
   else
     CP_REQUIRE(p.out_mode == CP_OUT_F32 && p.n_valid >= 1 && p.n_valid <= p.ld_out && p.n_valid <= kp.npad, CP_E_INVALID,
                "cp_edgeconv_fwd: bad f32 output spec");
-  const uint8_t* wbase = reinterpret_cast<const uint8_t*>(L.w_packed);
   for (int c = 0; c < kp.KC; ++c)
-    for (int nb = 0; nb < kp.NB; ++nb) {
-      const int rows = (kp.npad - nb * 128 < 128) ? (kp.npad - nb * 128) : 128;
-      WTile& w = kp.wt[c * kp.NB + nb];
-      w.ptr = wbase + (size_t)nb * 128 * L.kin * 2 + (size_t)c * rows * 128;
-      w.bytes = (uint32_t)rows * 128;
-      w.pad = 0;
-    }
+    for (int nb = 0; nb < kp.NB; ++nb) kp.wt[c * kp.NB + nb] = cp::packed_tile(L.w_packed, nb, c, L.kin, kp.npad);
   const int num_sms = cp::num_sms();
   const int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;
   // bf16 outputs whose width is a multiple of 32 columns leave through TMA tensor stores: a 3-D map (columns, nodes, RoIs)

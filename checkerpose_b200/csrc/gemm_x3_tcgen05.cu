@@ -64,27 +64,10 @@ struct X3Params {
   int tma_out;       // the epilogue leaves through TMA tensor stores (ld_out % 4 == 0, Nout % 4 == 0, 16-byte aligned base)
 };
 
-__device__ __forceinline__ uint32_t pack_bf2(float a, float b) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(a, b);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
 __device__ __forceinline__ float bf_round(float a) { return __bfloat162float(__float2bfloat16_rn(a)); }
 
 __device__ __forceinline__ void sts64(uint32_t addr, uint32_t a, uint32_t b) {
   asm volatile("st.shared.v2.u32 [%0], {%1,%2};" ::"r"(addr), "r"(a), "r"(b) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
 }
 
 // ------------------------------------------------------------------------------------------------------
@@ -193,8 +176,8 @@ __device__ void a_loader(const X3Params& kp, uint8_t* sm, Bars* bars, int lw, in
         const float4 v = cur[i];
         const float hx = bf_round(v.x), hy = bf_round(v.y), hz = bf_round(v.z), hw = bf_round(v.w);
         const uint32_t off = (uint32_t)(r * 128 + (((c4 >> 1) ^ (r & 7)) << 4) + (c4 & 1) * 8);
-        sts64(a_hi + off, pack_bf2(hx, hy), pack_bf2(hz, hw));
-        sts64(a_lo + off, pack_bf2(v.x - hx, v.y - hy), pack_bf2(v.z - hz, v.w - hw));
+        sts64(a_hi + off, f2_to_bf2(hx, hy), f2_to_bf2(hz, hw));
+        sts64(a_lo + off, f2_to_bf2(v.x - hx, v.y - hy), f2_to_bf2(v.z - hz, v.w - hw));
       }
       fence_proxy_async_smem();
       __syncwarp();
@@ -223,12 +206,11 @@ __device__ void weight_producer(const X3Params& kp, uint8_t* sm, Bars* bars) {
         uint8_t* w_hi = sm + s * STAGE_BYTES + 2 * A_BYTES;
         uint8_t* w_lo = w_hi + W_BYTES;
         mbar_arrive_expect_tx(&bars->full[s], (uint32_t)cols * 128u * 2u);
-        // packed layout (cp_pack_weight): 128-row block b at b * 128 * K * 2 bytes; inside it chunk kc at kc * rows * 128
-        const size_t o0 = (size_t)(col0 / 128) * 128 * p.K * 2 + (size_t)kc * rows0 * 128;
+        const size_t o0 = cp::packed_tile_offset(col0 / 128, kc, rows0, p.K);
         bulk_g2s(w_hi, reinterpret_cast<const uint8_t*>(p.w_hi) + o0, (uint32_t)rows0 * 128u, &bars->full[s]);
         bulk_g2s(w_lo, reinterpret_cast<const uint8_t*>(p.w_lo) + o0, (uint32_t)rows0 * 128u, &bars->full[s]);
         if (rows1 > 0) {
-          const size_t o1 = (size_t)(col0 / 128 + 1) * 128 * p.K * 2 + (size_t)kc * rows1 * 128;
+          const size_t o1 = cp::packed_tile_offset(col0 / 128 + 1, kc, rows1, p.K);
           bulk_g2s(w_hi + 128 * 128, reinterpret_cast<const uint8_t*>(p.w_hi) + o1, (uint32_t)rows1 * 128u, &bars->full[s]);
           bulk_g2s(w_lo + 128 * 128, reinterpret_cast<const uint8_t*>(p.w_lo) + o1, (uint32_t)rows1 * 128u, &bars->full[s]);
         }
@@ -267,10 +249,6 @@ __device__ void mma_issuer(const X3Params& kp, uint8_t* sm, Bars* bars, uint32_t
       __syncwarp();
     }
   }
-}
-
-__device__ __forceinline__ void sts128(uint32_t addr, float a, float b, float c, float d) {
-  asm volatile("st.shared.v4.f32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "f"(a), "f"(b), "f"(c), "f"(d) : "memory");
 }
 
 // warp q drains TMEM lanes [32 q, 32 q + 32): 32 columns at a time -> + bias -> activation -> a 32 x 32 fp32 tile in shared
@@ -321,7 +299,7 @@ __device__ void epilogue(const X3Params& kp, const CUtensorMap* out_map, uint8_t
       if (kp.tma_out) {
         const uint32_t tbuf = tbuf0 + (nstore & 1) * EPI_TILE_BYTES;
         ++nstore;
-        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 1;" ::: "memory");   // the store that last used this tile has read it
+        if (lane == 0) bulk_wait_read<1>();   // the store that last used this tile has read it
         __syncwarp();
 #pragma unroll
         for (int e4 = 0; e4 < 8; ++e4)
@@ -329,9 +307,8 @@ __device__ void epilogue(const X3Params& kp, const CUtensorMap* out_map, uint8_t
         fence_proxy_async_smem();
         __syncwarp();
         if (lane == 0 && row0 < p.M) {
-          asm volatile("cp.async.bulk.tensor.2d.global.shared::cta.bulk_group [%0, {%2, %3}], [%1];"
-                       ::"l"(out_map), "r"(tbuf), "r"(n0), "r"((int)row0) : "memory");
-          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+          tma_store_2d(out_map, tbuf, n0, (int)row0);
+          bulk_commit();
         }
       } else if (row_ok) {
 #pragma unroll
@@ -343,7 +320,7 @@ __device__ void epilogue(const X3Params& kp, const CUtensorMap* out_map, uint8_t
     __syncwarp();
     if (lane == 0) mbar_arrive(&bars->acc_empty[slot]);
   }
-  if (kp.tma_out && lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // shared memory outlives the last stores' reads
+  if (kp.tma_out && lane == 0) bulk_wait_read<0>();   // shared memory outlives the last stores' reads
 }
 
 __global__ void __launch_bounds__(NTHREADS, 1) gemm_x3_kernel(const __grid_constant__ X3Params kp, const __grid_constant__ CUtensorMap out_map) {
@@ -382,10 +359,8 @@ __global__ void pack_weight_split_kernel(const float* __restrict__ w, int Nout, 
   const int64_t total = (int64_t)Npad * K;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int n = (int)(e / K), k = (int)(e - (int64_t)n * K);
-    const int nb = n >> 7, r = n & 127;
-    const int rows_blk = min(128, Npad - nb * 128);
-    const int kc = k >> 6, kk = k & 63;
-    const size_t off = (size_t)nb * 128 * K + (size_t)kc * rows_blk * 64 + (size_t)r * 64 + (size_t)(((kk >> 3) ^ (r & 7)) << 3) + (kk & 7);
+    const int nb = n >> 7, r = n & 127, kk = k & 63;
+    const size_t off = cp::packed_tile_offset(nb, k >> 6, cp::packed_block_rows(nb, Npad), K) / 2 + (size_t)r * 64 + (size_t)(((kk >> 3) ^ (r & 7)) << 3) + (kk & 7);
     const float v = (n < Nout) ? w[(size_t)n * K + k] : 0.f;
     const bf16 h = __float2bfloat16_rn(v);
     hi[off] = h;

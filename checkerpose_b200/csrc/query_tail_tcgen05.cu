@@ -49,24 +49,6 @@ struct QtParams {
   int num_tiles;
 };
 
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(void* smem_dst, const CUtensorMap* map, int c0, int c1, uint64_t* bar) {
-  asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%2, %3}], [%4];"
-               ::"r"(smem_u32(smem_dst)), "l"(map), "r"(c0), "r"(c1), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t (&r)[32]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-      "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-      : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-        "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-        "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-        "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-      : "r"(taddr));
-}
-
 __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_constant__ QtParams kp, const __grid_constant__ CUtensorMap src_map) {
   extern __shared__ uint8_t smem_raw[];
   uint8_t* sm = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -104,7 +86,8 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     // ---- producer ----
     if (elect_one()) {
       mbar_arrive_expect_tx(&bars->w_full, (uint32_t)(NMID * KC * 128));
-      bulk_g2s(sm + OFF_W, p.w1_packed, (uint32_t)(NMID * KC * 128), &bars->w_full);   // packed: chunk c at c * 64 rows * 128 B
+      // the whole packed matrix (cp::packed_tile_offset): one block of 64 rows, chunk c at c * 64 * 128 bytes
+      bulk_g2s(sm + OFF_W, p.w1_packed, (uint32_t)(NMID * KC * 128), &bars->w_full);
     }
     __syncwarp();
     uint32_t it = 0;
@@ -113,7 +96,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
       if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       if (elect_one()) {
         mbar_arrive_expect_tx(&bars->full[s], (uint32_t)(KC * A_CHUNK_BYTES));
-        for (int c = 0; c < KC; ++c) tma_load_2d(sm + s * A_STAGE_BYTES + c * A_CHUNK_BYTES, &src_map, c * 64, tile * TILE_M, &bars->full[s]);
+        for (int c = 0; c < KC; ++c) tma_load_2d(smem_u32(sm + s * A_STAGE_BYTES + c * A_CHUNK_BYTES), &src_map, c * 64, tile * TILE_M, &bars->full[s]);
       }
       __syncwarp();
     }

@@ -190,24 +190,17 @@ __global__ void fold_edgeconv_kernel(const float* __restrict__ w, const float* _
   }
 }
 
-// Tile image for the tcgen05 kernels (see chain_tcgen05.cu): N blocks of up to 128 rows, K chunks of 64
-// bf16 (=128 B rows); within a tile row r, 16-byte chunk c is stored at r*128 + ((c ^ (r & 7)) << 4)
-// (K-major SWIZZLE_128B canonical layout, 8-row groups of 1024 B).
+// Packed weight image for the tcgen05 kernels (layout: cp::packed_tile_offset)
 __global__ void pack_weight_kernel(const float* __restrict__ w, int Nout, int K, int Npad, bf16* __restrict__ out) {
-  const int KC = K / 64;
   const int64_t total = (int64_t)Npad * K;
   for (int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (int64_t)gridDim.x * blockDim.x) {
     const int n = (int)(e / K), k = (int)(e - (int64_t)n * K);
-    const int nb = n >> 7, r = n & 127;
-    const int rows_blk = min(128, Npad - nb * 128);
-    const int kc = k >> 6, kk = k & 63;
+    const int nb = n >> 7, r = n & 127, kk = k & 63;
     const int chunk = kk >> 3, within = kk & 7;
-    const size_t tile_off = (size_t)nb * 128 * K + (size_t)kc * rows_blk * 64;  // in elements
-    const size_t off = tile_off + (size_t)r * 64 + (size_t)((chunk ^ (r & 7)) << 3) + within;
+    const size_t off = cp::packed_tile_offset(nb, k >> 6, cp::packed_block_rows(nb, Npad), K) / 2 + (size_t)r * 64 + (size_t)((chunk ^ (r & 7)) << 3) + within;
     const float v = (n < Nout) ? w[(size_t)n * K + k] : 0.f;
     out[off] = __float2bfloat16_rn(v);
   }
-  (void)KC;
 }
 
 // ------------------------------------------------------------------------------------------------

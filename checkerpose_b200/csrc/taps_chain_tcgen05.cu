@@ -57,11 +57,6 @@ constexpr int OFF_BAR = OFF_BIAS + BIAS_FLOATS * 4;
 constexpr int SMEM_BYTES = OFF_BAR + 512;
 static_assert(SMEM_BYTES + 1024 <= 227 * 1024, "shared memory budget");
 
-struct WT {
-  const uint8_t* ptr;
-  uint32_t bytes, pad;
-};
-
 struct TcParams {
   cp_chain_params p;
   int tiles_per_roi, num_tiles;
@@ -69,7 +64,7 @@ struct TcParams {
   int P2;        // 128-column blocks of layer 2 per half (1: nout2 = 256, one half; 2: nout2 = 512, two halves)
   int halves2;   // 1 or 2 accumulator passes for layer 2
   int T;         // weight tiles per node tile
-  WT wt[MAX_WT]; // in the order the MMA thread consumes them
+  cp::WTile wt[MAX_WT]; // in the order the MMA thread consumes them
 };
 
 struct Bars {
@@ -82,28 +77,6 @@ struct Bars {
 static_assert(sizeof(Bars) <= 512, "barrier block");
 
 __device__ __forceinline__ uint32_t chunk_off(int row, int piece) { return (uint32_t)(row * 128 + ((piece ^ (row & 7)) << 4)); }
-__device__ __forceinline__ uint32_t f2_to_bf2(float lo, float hi) {
-  __nv_bfloat162 v = __floats2bfloat162_rn(lo, hi);
-  return *reinterpret_cast<uint32_t*>(&v);
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-// 16-byte cp.async; src_bytes = 0 writes zeros (no global access)
-__device__ __forceinline__ void cp_async16_zfill(uint32_t dst, const void* src, uint32_t src_bytes) {
-  asm volatile("cp.async.cg.shared.global [%0], [%1], 16, %2;" ::"r"(dst), "l"(src), "r"(src_bytes) : "memory");
-}
-__device__ __forceinline__ void cp_async_arrive_noinc(uint64_t* bar) {
-  asm volatile("cp.async.mbarrier.arrive.noinc.shared::cta.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ uint4 lds128(uint32_t addr) {
-  uint4 r;
-  asm volatile("ld.shared.v4.u32 {%0,%1,%2,%3}, [%4];" : "=r"(r.x), "=r"(r.y), "=r"(r.z), "=r"(r.w) : "r"(addr));
-  return r;
-}
-__device__ __forceinline__ void sts128(uint32_t addr, uint4 v) {
-  asm volatile("st.shared.v4.u32 [%0], {%1,%2,%3,%4};" ::"r"(addr), "r"(v.x), "r"(v.y), "r"(v.z), "r"(v.w) : "memory");
-}
 
 // ------------------------------------------------------------------------------------------------------
 // gather producers
@@ -278,13 +251,6 @@ __device__ void mma_issuer(const TcParams& kp, uint8_t* sm, Bars* bars, uint32_t
 // ------------------------------------------------------------------------------------------------------
 // epilogue: warp (q = w & 3, half = w >> 2) drains TMEM lanes [32 q, 32 q + 32), every second 32-column block
 // ------------------------------------------------------------------------------------------------------
-__device__ __forceinline__ void tma_store_3d(const CUtensorMap* map, uint32_t smem_src, int c0, int c1, int c2) {
-  asm volatile("cp.async.bulk.tensor.3d.global.shared::cta.bulk_group [%0, {%2, %3, %4}], [%1];"
-               ::"l"(map), "r"(smem_src), "r"(c0), "r"(c1), "r"(c2) : "memory");
-}
-__device__ __forceinline__ void bulk_commit() { asm volatile("cp.async.bulk.commit_group;" ::: "memory"); }
-__device__ __forceinline__ void bulk_wait_read0() { asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory"); }
-
 __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, uint8_t* sm, Bars* bars, uint32_t tmem_base, int ew, int lane) {
   const cp_chain_params& p = kp.p;
   const int q = ew & 3, hh = ew >> 2;
@@ -314,14 +280,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
       const uint32_t tbase = tmem_base + slot * ACC_COLS + ((uint32_t)(q * 32) << 16);
       for (int c0 = hh * 32; c0 < ncols; c0 += 32 * (NUM_E_WARPS / 4)) {
         uint32_t r[32];
-        asm volatile(
-            "tcgen05.ld.sync.aligned.32x32b.x32.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15,"
-            "%16,%17,%18,%19,%20,%21,%22,%23,%24,%25,%26,%27,%28,%29,%30,%31}, [%32];"
-            : "=r"(r[0]), "=r"(r[1]), "=r"(r[2]), "=r"(r[3]), "=r"(r[4]), "=r"(r[5]), "=r"(r[6]), "=r"(r[7]), "=r"(r[8]),
-              "=r"(r[9]), "=r"(r[10]), "=r"(r[11]), "=r"(r[12]), "=r"(r[13]), "=r"(r[14]), "=r"(r[15]), "=r"(r[16]),
-              "=r"(r[17]), "=r"(r[18]), "=r"(r[19]), "=r"(r[20]), "=r"(r[21]), "=r"(r[22]), "=r"(r[23]), "=r"(r[24]),
-              "=r"(r[25]), "=r"(r[26]), "=r"(r[27]), "=r"(r[28]), "=r"(r[29]), "=r"(r[30]), "=r"(r[31])
-            : "r"(tbase + (uint32_t)c0));
+        tmem_ld32(tbase + (uint32_t)c0, r);
         float v[32];
         uint4 bb[8];
 #pragma unroll
@@ -351,7 +310,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
           __syncwarp();
           if (lane == 0) mbar_arrive(&bars->h_full[c0 >> 6]);   // this warp's half of chunk c0 / 64 is in place
         } else {
-          if (lane == 0) bulk_wait_read0();   // the warp's previous store is done reading the tile
+          if (lane == 0) bulk_wait_read<0>();   // the warp's previous store is done reading the tile
           __syncwarp();
 #pragma unroll
           for (int e = 0; e < 4; ++e) sts128(tbuf + lane * 64 + ((e ^ sw) << 4), w[e]);
@@ -368,7 +327,7 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
       if (lane == 0) mbar_arrive(&bars->acc_empty[slot]);
     }
   }
-  if (lane == 0) bulk_wait_read0();   // shared memory must outlive the last stores' reads
+  if (lane == 0) bulk_wait_read<0>();   // shared memory must outlive the last stores' reads
 }
 
 __global__ void __launch_bounds__(NTHREADS, 1) taps_chain_kernel(const __grid_constant__ TcParams kp, const __grid_constant__ CUtensorMap out_map) {
@@ -442,16 +401,14 @@ bool taps_chain_try(const cp_chain_params& p, cudaStream_t s, int* rc) {
   kp.halves2 = L2.nout / 256;
   kp.P2 = 2;
   int T = 0;
-  auto tile_ptr = [](const cp_chain_layer& L, int nb, int kc) {   // packed layout of cp_pack_weight (all blocks have 128 rows here)
-    return reinterpret_cast<const uint8_t*>(L.w_packed) + (size_t)nb * 128 * L.kin * 2 + (size_t)kc * 128 * 128;
-  };
+  auto tile = [](const cp_chain_layer& L, int nb, int kc) { return cp::packed_tile(L.w_packed, nb, kc, L.kin, L.nout); };
   for (int c = 0; c < kp.KX; ++c)
-    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = {tile_ptr(L0, nb, c), 128 * 128, 0};
+    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L0, nb, c);
   for (int c = 0; c < NH; ++c)
-    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = {tile_ptr(L1, nb, c), 128 * 128, 0};
+    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L1, nb, c);
   for (int half = 0; half < kp.halves2; ++half)
     for (int c = 0; c < NH; ++c)
-      for (int nb = 0; nb < kp.P2; ++nb) kp.wt[T++] = {tile_ptr(L2, half * 2 + nb, c), 128 * 128, 0};
+      for (int nb = 0; nb < kp.P2; ++nb) kp.wt[T++] = tile(L2, half * 2 + nb, c);
   kp.T = T;
   const int num_sms = cp::num_sms();
   const int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;

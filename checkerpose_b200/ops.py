@@ -19,13 +19,27 @@ OUT_BF16, OUT_F32 = 0, 1
 
 #: number of kernel launches issued through this module (bench.py reports it as ``gpu_launches``)
 launch_count = 0
-#: when set to a list, chain_fwd appends (signature, start_event, end_event) per launch (bench.py roofline)
+#: when set to a list, every launch of the tcgen05 GEMM kernels appends (signature, start_event, end_event) (bench.py roofline)
 chain_event_log = None
 
 
 def _count(n=1):
     global launch_count
     launch_count += n
+
+
+def _timed_launch(fn, name, p, sig):
+    """One launch of ``fn(&p, stream)``; with chain_event_log set, CUDA events on the launching stream around it are
+    logged under ``sig``."""
+    if chain_event_log is None:
+        check(fn(C.byref(p), _stream()), name)
+    else:
+        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+        e0.record()
+        check(fn(C.byref(p), _stream()), name)
+        e1.record()
+        chain_event_log.append((sig, e0, e1))
+    _count()
 
 
 def _stream():
@@ -209,18 +223,6 @@ def pack_weight_split(w: torch.Tensor):
     return hi, lo
 
 
-def _gemm_x3(p: GemmX3Params, sig):
-    if chain_event_log is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_gemm_x3(C.byref(p), _stream()), "cp_gemm_x3")
-        e1.record()
-        chain_event_log.append((sig, e0, e1))
-    else:
-        check(lib.cp_gemm_x3(C.byref(p), _stream()), "cp_gemm_x3")
-    _count()
-
-
 def gemm_x3_linear(a1, w_split, nout, bias=None, act=False, slope=0.0, a2=None, out=None):
     """y = act([a1|a2] @ W.T + bias) in float32 on the tensor cores (cp_gemm_x3, CP_X3_LINEAR); a* (..., K*) fp32 rows."""
     _need_cuda(a1, a2, bias, w_split[0], w_split[1])
@@ -243,7 +245,7 @@ def gemm_x3_linear(a1, w_split, nout, bias=None, act=False, slope=0.0, a2=None, 
     p.w_hi, p.w_lo = _p(w_split[0]), _p(w_split[1])
     p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
     p.out, p.ld_out, p.Nout = _p(out), out.stride(-2) if out.dim() > 1 else nout, int(nout)
-    _gemm_x3(p, ("X3", K1 + K2, (int(nout),), OUT_F32, M, 0))
+    _timed_launch(lib.cp_gemm_x3, "cp_gemm_x3", p, ("X3", K1 + K2, (int(nout),), OUT_F32, M, 0))
     return out
 
 
@@ -263,23 +265,11 @@ def gemm_x3_conv(x_nhwc, w_split, nout, KH, KW, pad, Ho, Wo, bias=None, act=Fals
     p.w_hi, p.w_lo = _p(w_split[0]), _p(w_split[1])
     p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
     p.out, p.ld_out, p.Nout = _p(out), int(nout), int(nout)
-    _gemm_x3(p, ("X3C", KH * KW * Cin, (int(nout),), OUT_F32, B * Ho * Wo, 0))
+    _timed_launch(lib.cp_gemm_x3, "cp_gemm_x3", p, ("X3C", KH * KW * Cin, (int(nout),), OUT_F32, B * Ho * Wo, 0))
     return out
 
 
 # ------------------------------------------------------------------- bf16 implicit-GEMM convolution on tcgen05
-def _conv_bf16(p: ConvBf16Params, sig):
-    if chain_event_log is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_conv_bf16(C.byref(p), _stream()), "cp_conv_bf16")
-        e1.record()
-        chain_event_log.append((sig, e0, e1))
-    else:
-        check(lib.cp_conv_bf16(C.byref(p), _stream()), "cp_conv_bf16")
-    _count()
-
-
 def conv_bf16(x_nhwc, w_packed, nout, KH, KW, pad, Ho, Wo, bias=None, act=False, slope=0.0, transposed=False):
     """Conv2d KH x KW stride 1 / ConvTranspose2d stride 2 over a bf16 NHWC map (B,H,W,Cin) -> (B,Ho,Wo,nout) bf16 as an implicit
     GEMM on the tensor cores (cp_conv_bf16); W rows in (ky, kx, c) order, packed by pack_weight."""
@@ -296,7 +286,7 @@ def conv_bf16(x_nhwc, w_packed, nout, KH, KW, pad, Ho, Wo, bias=None, act=False,
     p.w_packed = _p(w_packed)
     p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
     p.out, p.ld_out, p.Nout = _p(out), int(nout), int(nout)
-    _conv_bf16(p, ("CV", KH * KW * Cin, (int(nout),), OUT_BF16, B * Ho * Wo, 0))
+    _timed_launch(lib.cp_conv_bf16, "cp_conv_bf16", p, ("CV", KH * KW * Cin, (int(nout),), OUT_BF16, B * Ho * Wo, 0))
     return out
 
 
@@ -317,23 +307,11 @@ def linear_bf16(a1, w_packed, nout, bias=None, act=False, slope=0.0, a2=None, ou
     p.w_packed = _p(w_packed)
     p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
     p.out, p.ld_out, p.Nout = _p(out), out.stride(-2) if out.dim() > 1 else nout, int(nout)
-    _conv_bf16(p, ("LB", K1 + K2, (int(nout),), OUT_BF16, M, 0))
+    _timed_launch(lib.cp_conv_bf16, "cp_conv_bf16", p, ("LB", K1 + K2, (int(nout),), OUT_BF16, M, 0))
     return out
 
 
 # ------------------------------------------------------------------- slab convolutions over zero-bordered maps
-def _conv_slab(p: ConvSlabParams, sig):
-    if chain_event_log is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_conv_slab(C.byref(p), _stream()), "cp_conv_slab")
-        e1.record()
-        chain_event_log.append((sig, e0, e1))
-    else:
-        check(lib.cp_conv_slab(C.byref(p), _stream()), "cp_conv_slab")
-    _count()
-
-
 def _slab_common(xp, w_packed, K, nout, bias, act, slope):
     _need_cuda(xp, bias, w_packed)
     assert xp.dtype == torch.bfloat16 and xp.is_contiguous() and xp.dim() == 4
@@ -399,7 +377,7 @@ def conv_slab_same(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0, 
     p.vy0, p.vy1, p.vx0, p.vx1 = 0, Hp - 1, 0, Wp - 1
     p.compact = 0
     # signature: ..., rows of the launch, multiply-accumulates of the convolution proper (without the border rows)
-    _conv_slab(p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * (Hp - 1) * (Wp - 1) * KH * KW * Cin * int(nout)))
+    _timed_launch(lib.cp_conv_slab, "cp_conv_slab", p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * (Hp - 1) * (Wp - 1) * KH * KW * Cin * int(nout)))
     return out if seg is None else (out, seg_out)
 
 
@@ -422,7 +400,7 @@ def conv_slab_full(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0):
             ph.shift[t] = (ky - 1) * Wp + (kx - 1)
     p.vy0, p.vy1, p.vx0, p.vx1 = 0, Hp, 0, Wp
     p.compact = 0
-    _conv_slab(p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * Hp * Wp * KH * KW * Cin * int(nout)))
+    _timed_launch(lib.cp_conv_slab, "cp_conv_slab", p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * Hp * Wp * KH * KW * Cin * int(nout)))
     return out
 
 
@@ -455,7 +433,7 @@ def convT_slab(x_nhwc, w_packed, nout, bias=None, act=False, slope=0.0):
             ph.out_off = dy * OWp + dx
     p.vy0, p.vy1, p.vx0, p.vx1 = 0, H, 0, W
     p.compact, p.out_sb, p.out_sy, p.out_sx = 1, OHp * OWp, 2 * OWp, 2
-    _conv_slab(p, ("CS", 9 * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * H * W * 9 * Cin * int(nout)))
+    _timed_launch(lib.cp_conv_slab, "cp_conv_slab", p, ("CS", 9 * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * H * W * 9 * Cin * int(nout)))
     return out
 
 
@@ -606,17 +584,7 @@ def chain_fwd(*, prologue, B, N, layers, out, out_mode, n_valid=0,
     for i, L in enumerate(layers):
         p.layers[i] = L
     p.out_mode, p.out, p.ld_out, p.n_valid = out_mode, _p(out), out.shape[-1], int(n_valid)
-    if chain_event_log is not None:
-        # bench.py: CUDA events on the launching stream around this one launch
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_chain_fwd(C.byref(p), _stream()), "cp_chain_fwd")
-        e1.record()
-        kin0 = layers[0].kin
-        chain_event_log.append(((prologue, kin0, tuple(L.nout for L in layers), out_mode, B, N), e0, e1))
-    else:
-        check(lib.cp_chain_fwd(C.byref(p), _stream()), "cp_chain_fwd")
-    _count()
+    _timed_launch(lib.cp_chain_fwd, "cp_chain_fwd", p, (prologue, layers[0].kin, tuple(L.nout for L in layers), out_mode, B, N))
     return out
 
 
@@ -693,15 +661,7 @@ def edgeconv_fwd(*, z, plan: GraphPlan, graph_sel, agg_slope, layer, out, out_mo
         p.a_out, p.ld_a_out = _p(a_out), a_out.shape[-1]
     p.layer = layer
     p.out_mode, p.out, p.ld_out, p.n_valid = out_mode, _p(out), out.shape[-1], int(n_valid)
-    if chain_event_log is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_edgeconv_fwd(C.byref(p), _stream()), "cp_edgeconv_fwd")
-        e1.record()
-        chain_event_log.append((("EC", p.Co, (layer.nout,), out_mode, p.B, p.N), e0, e1))
-    else:
-        check(lib.cp_edgeconv_fwd(C.byref(p), _stream()), "cp_edgeconv_fwd")
-    _count()
+    _timed_launch(lib.cp_edgeconv_fwd, "cp_edgeconv_fwd", p, ("EC", p.Co, (layer.nout,), out_mode, p.B, p.N))
     return out
 
 
@@ -751,15 +711,7 @@ def query_decode_fwd(*, src, w1_packed, b1, slope, w2, b2, plane, Ltot, x_bits, 
     p.plane, p.Ltot = int(plane), int(Ltot)
     p.x_bits, p.y_bits, p.x_id, p.y_id, p.x_id_kp, p.y_id_kp = _p(x_bits), _p(y_bits), _p(x_id), _p(y_id), _p(x_id_kp), _p(y_id_kp)
     p.perm, p.graph_sel = _p(perm), _p(graph_sel)
-    if chain_event_log is not None:
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        check(lib.cp_query_decode_fwd(C.byref(p), _stream()), "cp_query_decode_fwd")
-        e1.record()
-        chain_event_log.append((("QT", kin, (64, 2), OUT_F32, B, N), e0, e1))
-    else:
-        check(lib.cp_query_decode_fwd(C.byref(p), _stream()), "cp_query_decode_fwd")
-    _count()
+    _timed_launch(lib.cp_query_decode_fwd, "cp_query_decode_fwd", p, ("QT", kin, (64, 2), OUT_F32, B, N))
 
 
 def permute_rows(x, perm, graph_sel, to_keypoint_order):
