@@ -47,6 +47,9 @@ int make_f32_tensor_map_2d(void* map128, void* out, int64_t ncols, int64_t nrows
 // SM count of the CURRENT device (cached per device index; the persistent kernels size their grids with it)
 int num_sms();
 
+// cp_knn for C > 64 (knn_tcgen05.cu): arguments already checked by cp_knn
+int knn_wide(const float* x, int B, int C, int N, int k, int64_t* idx64, int32_t* idx32, cudaStream_t st);
+
 static inline int ceil_div(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 
 // Packed weight layout, written by cp_pack_weight / cp_pack_weight_split and sized by cp_packed_weight_bytes: an (Nout x K)

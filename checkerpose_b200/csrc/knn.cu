@@ -14,7 +14,8 @@
 // the reference materialises the (N,N) matrix (64 MB per object at N=4096).
 //
 // Block = 8 warps = 8 queries at a time; candidate points are staged through shared memory in
-// coalesced tiles shared by the 8 warps.
+// coalesced tiles shared by the 8 warps.  C <= 64 only: wider inputs (feature-space graphs) go to
+// knn_tcgen05.cu, which returns the same (d, j)-ordered result with tensor-core pruning.
 #include "common.cuh"
 
 namespace {
@@ -117,10 +118,10 @@ extern "C" int cp_knn(const float* x, int B, int C, int N, int k, int64_t* idx64
   CP_REQUIRE(x && idx64, CP_E_INVALID, "cp_knn: null pointer");
   CP_REQUIRE(B > 0 && C > 0 && N > 0, CP_E_INVALID, "cp_knn: bad shape B=%d C=%d N=%d", B, C, N);
   CP_REQUIRE(k >= 1 && k <= 64 && k <= N, CP_E_UNSUPPORTED, "cp_knn: need 1 <= k <= min(64, N), got k=%d N=%d", k, N);
-  CP_REQUIRE(C <= 64, CP_E_UNSUPPORTED, "cp_knn: C=%d > 64 not supported", C);
+  cudaStream_t st = (cudaStream_t)s;
+  if (C > 64) return cp::knn_wide(x, B, C, N, k, idx64, idx32, st);
   dim3 grid(cp::ceil_div(N, KNN_WARPS), B);
   size_t smem = ((size_t)C * KNN_TILE + (size_t)KNN_WARPS * C) * sizeof(float);
-  cudaStream_t st = (cudaStream_t)s;
   if (C == 3) {
     knn_kernel<3><<<grid, KNN_WARPS * 32, smem, st>>>(x, C, N, k, idx64, idx32);
   } else {

@@ -46,7 +46,7 @@ int cp_device_arch(void);
  * knn(x, k)  pipeline.py:18-23 == init.py:27-32 == pipeline_lm.py:18-23 == init_lm.py:27-32.
  * x (B, C, N) f32 -> idx64 (B, N, k) int64, nearest first (self is entry 0); optional int32 copy
  * idx32 (may be NULL).  fp32 direct-difference distances, ties broken towards the lower index.
- * 1 <= k <= 64, k <= N, C <= 64. */
+ * 1 <= k <= 64, k <= N, any C >= 1 (C > 64: tensor-core pruning, the same exact fp32 result). */
 int cp_knn(const float* x, int B, int C, int N, int k, int64_t* idx64, int32_t* idx32, cp_stream_t s);
 
 /* ---- layout conversion at the module boundary ----------------------------------------------
