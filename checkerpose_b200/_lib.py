@@ -65,7 +65,6 @@ class ConvBf16Params(C.Structure):
     _fields_ = [
         ("mode", c_i32),
         ("a1", c_vp), ("ld1", c_i32), ("k1", c_i32),
-        ("a2", c_vp), ("ld2", c_i32), ("k2", c_i32),
         ("H", c_i32), ("W", c_i32), ("Ho", c_i32), ("Wo", c_i32), ("KH", c_i32), ("KW", c_i32), ("pad", c_i32),
         ("M", c_i64), ("K", c_i32),
         ("w_packed", c_vp),

@@ -1,11 +1,10 @@
-// bf16 implicit-GEMM convolution / Linear on tcgen05: the image branch of the bf16 mode without a library call
+// bf16 implicit-GEMM convolution on tcgen05: the image branch of the bf16 mode without a library call
 // (SURVEY.md section 8f rank 1; get_gdrn_upsample_module checkerpose/model/pipeline.py:183-211, Index2Feat_module's
 // patch_generator :144-145, seg_block :349,383, InitNet_GNN.conv1x1 init.py:112).
 //
 // Same skeleton as the split-precision kernel of the float32 mode (gemm_x3_tcgen05.cu, which runs the tensor pipe at 96 % of
 // the sustained bf16 peak), with bf16 operands and ONE tcgen05.mma per K step:
-//   out[m, :Nout] = act(A[m, :K] . W^T + bias),  A[m] = row m of [a1 | a2]                                    (LINEAR)
-//                                                     = the kernel taps of output pixel m of an NHWC map, zero-padded  (CONV / CONVT)
+//   out[m, :Nout] = act(A[m, :K] . W^T + bias),  A[m] = the kernel taps of output pixel m of an NHWC map, zero-padded  (CONV / CONVT)
 // One persistent CTA of 16 warps per SM; tile = 128 rows x <= 256 output columns; K chunks of 64 channels; FOUR operand
 // stages of 48 KB (A 16 KB + W 32 KB) -- an MMA chunk is only 512 clk here, so the ring has to cover the L2 latency:
 //   warps 8-15  A loaders: cp.async (LDGSTS, 16 bytes, zero-fill outside the map) straight into the SWIZZLE_128B operand tile,
@@ -84,8 +83,8 @@ struct TileIt {
 // A loaders
 // ------------------------------------------------------------------------------------------------------
 struct RowInfo {       // per thread: its 4 rows of the current tile
-  int64_t base[RPT];   // LINEAR: row index.  CONV: element offset of input pixel (b, oy - pad, ox - pad) (may be negative: only
-                       // dereferenced for taps inside the map).  CONVT: pixel index b * H * W.  LINEAR / CONVT: -1 = beyond M
+  int64_t base[RPT];   // CONV: element offset of input pixel (b, oy - pad, ox - pad) (may be negative: only dereferenced for
+                       // taps inside the map).  CONVT: pixel index b * H * W, -1 = beyond M
   int oyx[RPT];        // CONV / CONVT: oy | ox << 16 (CONV marks rows beyond M with 0x7fff7fff: every tap fails the bounds check)
 };
 
@@ -98,8 +97,6 @@ __device__ __forceinline__ void rows_of_tile(const CvParams& kp, int m_tile, int
     if (m >= p.M) {
       ri.base[i] = -1;
       ri.oyx[i] = 0x7fff7fff;
-    } else if (p.mode == CP_X3_LINEAR) {
-      ri.base[i] = m;
     } else {
       const int hw = p.Ho * p.Wo;
       const int64_t b = m / hw;
@@ -128,7 +125,6 @@ __device__ void a_loader(const CvParams& kp, uint8_t* sm, Bars* bars, int tl) {
   const int piece = tl & 7;
   const uint32_t sm_base = smem_u32(sm);
   const bf16* a1 = reinterpret_cast<const bf16*>(p.a1);
-  const bf16* a2 = reinterpret_cast<const bf16*>(p.a2);
   RowInfo ri;
   ChunkPos pos;
   uint32_t it = 0;
@@ -141,18 +137,7 @@ __device__ void a_loader(const CvParams& kp, uint8_t* sm, Bars* bars, int tl) {
       const uint32_t s = it % STAGES;
       if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       const uint32_t a_s = sm_base + s * STAGE_BYTES;
-      if (p.mode == CP_X3_LINEAR) {
-        const int k = kc * 64 + piece * 8;
-        const bool first = k < p.k1;
-        const bf16* src = first ? a1 + k : a2 + (k - p.k1);
-        const int64_t ld = first ? p.ld1 : p.ld2;
-#pragma unroll
-        for (int i = 0; i < RPT; ++i) {
-          const int r = (tl >> 3) + 32 * i;
-          const bool ok = ri.base[i] >= 0;
-          cp_async16_zfill(a_s + r * 128 + ((piece ^ (r & 7)) << 4), ok ? src + ri.base[i] * ld : src, ok ? 16u : 0u);
-        }
-      } else if (p.mode == CP_X3_CONV) {
+      if (p.mode == CP_X3_CONV) {
         const int dy = pos.ky - p.pad, dx = pos.kx - p.pad;
         const bf16* src = a1 + ((int64_t)pos.ky * p.W + pos.kx) * p.k1 + pos.cc * 64 + piece * 8;
 #pragma unroll
@@ -371,21 +356,12 @@ extern "C" int cp_conv_bf16(const cp_conv_bf16_params* pp, cp_stream_t s) {
              "cp_conv_bf16: K=%d must be a multiple of 64, weights 16-byte aligned, ld_out >= Nout", p.K);
   CvParams kp;
   kp.p = p;
-  kp.c_chunks = 1;
-  if (p.mode == CP_X3_LINEAR) {
-    CP_REQUIRE(p.k1 > 0 && p.k1 % 64 == 0 && p.k2 >= 0 && p.k2 % 64 == 0 && p.k1 + p.k2 == p.K && (p.k2 == 0 || p.a2), CP_E_UNSUPPORTED,
-               "cp_conv_bf16: k1=%d, k2=%d must be multiples of 64 summing to K=%d", p.k1, p.k2, p.K);
-    CP_REQUIRE(p.ld1 >= p.k1 && (p.ld1 & 7) == 0 && (reinterpret_cast<uintptr_t>(p.a1) & 15) == 0 &&
-               (p.k2 == 0 || (p.ld2 >= p.k2 && (p.ld2 & 7) == 0 && (reinterpret_cast<uintptr_t>(p.a2) & 15) == 0)), CP_E_INVALID,
-               "cp_conv_bf16: operand rows must be 16-byte aligned (ld %% 8 == 0)");
-  } else {
-    CP_REQUIRE(p.mode == CP_X3_CONV || p.mode == CP_X3_CONVT, CP_E_INVALID, "cp_conv_bf16: bad mode %d", p.mode);
-    CP_REQUIRE(p.k1 > 0 && p.k1 % 64 == 0 && p.KH > 0 && p.KW > 0 && p.KH * p.KW * p.k1 == p.K, CP_E_UNSUPPORTED,
-               "cp_conv_bf16: conv needs Cin %% 64 == 0 and K == KH*KW*Cin (Cin=%d KH=%d KW=%d K=%d)", p.k1, p.KH, p.KW, p.K);
-    CP_REQUIRE(p.H > 0 && p.W > 0 && p.Ho > 0 && p.Wo > 0 && p.Ho < 32768 && p.Wo < 32768 && p.pad >= 0 && p.M % ((int64_t)p.Ho * p.Wo) == 0 &&
-               (reinterpret_cast<uintptr_t>(p.a1) & 15) == 0, CP_E_INVALID, "cp_conv_bf16: bad map sizes H=%d W=%d Ho=%d Wo=%d", p.H, p.W, p.Ho, p.Wo);
-    kp.c_chunks = p.k1 / 64;
-  }
+  CP_REQUIRE(p.mode == CP_X3_CONV || p.mode == CP_X3_CONVT, CP_E_INVALID, "cp_conv_bf16: bad mode %d", p.mode);
+  CP_REQUIRE(p.k1 > 0 && p.k1 % 64 == 0 && p.KH > 0 && p.KW > 0 && p.KH * p.KW * p.k1 == p.K, CP_E_UNSUPPORTED,
+             "cp_conv_bf16: conv needs Cin %% 64 == 0 and K == KH*KW*Cin (Cin=%d KH=%d KW=%d K=%d)", p.k1, p.KH, p.KW, p.K);
+  CP_REQUIRE(p.H > 0 && p.W > 0 && p.Ho > 0 && p.Wo > 0 && p.Ho < 32768 && p.Wo < 32768 && p.pad >= 0 && p.M % ((int64_t)p.Ho * p.Wo) == 0 &&
+             (reinterpret_cast<uintptr_t>(p.a1) & 15) == 0, CP_E_INVALID, "cp_conv_bf16: bad map sizes H=%d W=%d Ho=%d Wo=%d", p.H, p.W, p.Ho, p.Wo);
+  kp.c_chunks = p.k1 / 64;
   kp.KC = p.K / 64;
   kp.npad = (p.Nout + 15) / 16 * 16;
   kp.nblk = (kp.npad + BN - 1) / BN;

@@ -322,18 +322,100 @@ def init_head_node_major(init_net, feat_last, obj_ids, dtype):
 
 
 # --------------------------------------------------------------------------------------------------
-# image branch helpers (library convolutions)
+# image branch: one BN-folded description of a conv stack, three executors built from it
 # --------------------------------------------------------------------------------------------------
-def _to_channels_last(x):
-    """NCHW -> channels_last without torch's generic strided copy: the bf16 HRNet maps go through the tiled transpose
-    kernel (cp_transpose_cn_to_nc on (B, C, H*W)); the result is the same channels_last-strided NCHW tensor."""
-    cl = torch.channels_last
-    if x.is_contiguous(memory_format=cl):
-        return x
+def image_layers(module):
+    """The layers of an image-branch module (up_net block, patch_generator, seg_block, conv1x1: an nn.Sequential or one
+    layer), walked once, as tuples ``(kind, w, b, m, relu)``.  A convolution (kind "conv" / "convT") carries its fp32 weight
+    ``w`` in the module's own layout and its fp32 bias ``b`` (or None), with a following BatchNorm2d folded in on the output
+    channels (axis 0 of a Conv2d weight, axis 1 of a ConvTranspose2d weight), the module ``m`` itself (stride, padding, ...)
+    and whether a following ReLU is fused.  "relu", "lrelu" and "up" (UpsamplingBilinear2d(scale_factor=2)) entries carry
+    only ``m``.  Every executor builds from this list, so all of them run bit-identical folded weights."""
+    mods = list(module) if isinstance(module, nn.Sequential) else [module]
+    layers = []
+    i = 0
+    while i < len(mods):
+        m = mods[i]
+        if isinstance(m, (nn.Conv2d, nn.ConvTranspose2d)):
+            tr = isinstance(m, nn.ConvTranspose2d)
+            w = m.weight.detach().float()
+            b = None if m.bias is None else m.bias.detach().float()
+            if i + 1 < len(mods) and isinstance(mods[i + 1], nn.BatchNorm2d):
+                bn = mods[i + 1]
+                sc = bn.weight.detach().float() / torch.sqrt(bn.running_var.detach().float() + bn.eps)
+                sh = bn.bias.detach().float() - sc * bn.running_mean.detach().float()
+                w = w * (sc.view(1, -1, 1, 1) if tr else sc.view(-1, 1, 1, 1))
+                b = sh if b is None else b * sc + sh
+                i += 1
+            relu = i + 1 < len(mods) and isinstance(mods[i + 1], nn.ReLU)
+            if relu:
+                i += 1
+            layers.append(("convT" if tr else "conv", w, b, m, relu))
+        elif isinstance(m, nn.ReLU):
+            layers.append(("relu", None, None, m, False))
+        elif isinstance(m, nn.LeakyReLU):
+            layers.append(("lrelu", None, None, m, False))
+        elif isinstance(m, nn.UpsamplingBilinear2d):
+            if float(m.scale_factor) != 2.0:
+                raise RuntimeError("image branch: only UpsamplingBilinear2d(scale_factor=2) is supported")
+            layers.append(("up", None, None, m, False))
+        else:
+            raise RuntimeError(f"unsupported layer in image branch: {type(m).__name__}")
+        i += 1
+    return layers
+
+
+def _gemm_layers(module, pack, mode):
+    """image_layers(module) for our implicit-GEMM kernels: each convolution as (kind, pack(W rows in (ky, kx, c) order, Cin
+    zero-padded to the kernels' 64-channel K chunks), b, (cout, kh, kw, pad, cin_pad), relu).  They take Conv2d stride 1 and
+    ConvTranspose2d stride 2 / output_padding 1 with square padding, no dilation or groups, and ReLU but not LeakyReLU;
+    ``mode`` names the branch in the error raised for anything else."""
+    layers = []
+    for kind, w, b, m, relu in image_layers(module):
+        if kind in ("relu", "up"):
+            layers.append((kind, None, None, None, False))
+            continue
+        tr = kind == "convT"
+        if kind == "lrelu" or not (m.groups == 1 and tuple(m.dilation) == (1, 1) and m.padding[0] == m.padding[1] and
+                                   tuple(m.stride) == ((2, 2) if tr else (1, 1)) and (not tr or tuple(m.output_padding) == (1, 1))):
+            raise RuntimeError(f"{mode} image branch: unsupported layer {m}")
+        kh, kw = m.kernel_size
+        cin, cout = (w.shape[0], w.shape[1]) if tr else (w.shape[1], w.shape[0])
+        wk = w.permute(1, 2, 3, 0) if tr else w.permute(0, 2, 3, 1)        # (cout, kh, kw, cin)
+        cin_pad = (cin + 63) // 64 * 64
+        if cin_pad != cin:
+            wk = F.pad(wk, (0, cin_pad - cin))
+        layers.append((kind, pack(wk.reshape(cout, kh * kw * cin_pad).contiguous()), None if b is None else b.contiguous(),
+                       (cout, kh, kw, int(m.padding[0]), cin_pad), relu))
+    return layers
+
+
+def _nhwc(x, dtype):
+    """NCHW (any strides) -> contiguous (B,H,W,C) of ``dtype``: a view when x already is one, else one launch of
+    cp_transpose_cn_to_nc (the tiled transpose for the bf16 HRNet maps)."""
+    v = x.permute(0, 2, 3, 1)
+    if v.is_contiguous() and v.dtype == dtype:
+        return v
     B, Cc, H, W = x.shape
-    if x.is_cuda and x.is_contiguous() and x.dtype == torch.bfloat16 and Cc % 64 == 0 and (H * W) % 64 == 0:
-        return ops.to_node_major(x.view(B, Cc, H * W), torch.bfloat16).view(B, H, W, Cc).permute(0, 3, 1, 2)
-    return x.contiguous(memory_format=cl)
+    return ops.to_node_major(x.contiguous().view(B, Cc, H * W), dtype).view(B, H, W, Cc)
+
+
+def _pad_channels(y, cin_pad):
+    """Zero channels of an NHWC map up to the implicit-GEMM kernels' 64-channel granularity."""
+    return y if y.shape[-1] == cin_pad else F.pad(y, (0, cin_pad - y.shape[-1]))
+
+
+def _gather_conv(conv, y, kind, ws, b, geom, relu):
+    """One convolution of a _gemm_layers entry on a gather kernel (ops.gemm_x3_conv / ops.conv_bf16) over the contiguous NHWC
+    map y; stride 1 for "conv", stride 2 with output_padding 1 for "convT"."""
+    cout, kh, kw, pad, cin_pad = geom
+    y = _pad_channels(y, cin_pad)
+    H, W = y.shape[1], y.shape[2]
+    if kind == "conv":
+        Ho, Wo = H + 2 * pad - kh + 1, W + 2 * pad - kw + 1
+    else:
+        Ho, Wo = (H - 1) * 2 - 2 * pad + kh + 1, (W - 1) * 2 - 2 * pad + kw + 1
+    return conv(y, ws, cout, kh, kw, pad, Ho, Wo, b, relu, 0.0, transposed=(kind == "convT"))
 
 
 class _FoldedSeq:
@@ -344,43 +426,14 @@ class _FoldedSeq:
     _fused_relu_ok = None   # torch.cudnn_convolution_relu availability, probed on first use
 
     def __init__(self, module):
-        mods = list(module) if isinstance(module, nn.Sequential) else [module]
         self.ops = []
         self.bias_f32 = {}     # op index -> f32 bias (the bf16 copy in ops is what cuDNN's fused conv+bias+ReLU takes)
-        i = 0
-        while i < len(mods):
-            m = mods[i]
-            if isinstance(m, (nn.Conv2d, nn.ConvTranspose2d)):
-                w = m.weight.detach().float()
-                b = None if m.bias is None else m.bias.detach().float()
-                if i + 1 < len(mods) and isinstance(mods[i + 1], nn.BatchNorm2d):
-                    bn = mods[i + 1]
-                    sc = bn.weight.detach().float() / torch.sqrt(bn.running_var.detach().float() + bn.eps)
-                    sh = bn.bias.detach().float() - sc * bn.running_mean.detach().float()
-                    if isinstance(m, nn.ConvTranspose2d):
-                        w = w * sc.view(1, -1, 1, 1)
-                    else:
-                        w = w * sc.view(-1, 1, 1, 1)
-                    b = sh if b is None else b * sc + sh
-                    i += 1
-                kind = "convT" if isinstance(m, nn.ConvTranspose2d) else "conv"
-                relu = i + 1 < len(mods) and isinstance(mods[i + 1], nn.ReLU)
-                if relu:
-                    i += 1
-                self.ops.append((kind, w.to(torch.bfloat16).contiguous(memory_format=torch.channels_last),
-                                 None if b is None else b.to(torch.bfloat16), m, relu))
-                self.bias_f32[len(self.ops) - 1] = None if b is None else b.contiguous()
-            elif isinstance(m, nn.ReLU):
-                self.ops.append(("relu", None, None, m, False))
-            elif isinstance(m, nn.LeakyReLU):
-                self.ops.append(("lrelu", None, None, m, False))
-            elif isinstance(m, nn.UpsamplingBilinear2d):
-                if float(m.scale_factor) != 2.0:
-                    raise RuntimeError("image branch: only UpsamplingBilinear2d(scale_factor=2) is supported")
-                self.ops.append(("up", None, None, m, False))
-            else:
-                raise RuntimeError(f"unsupported layer in image branch: {type(m).__name__}")
-            i += 1
+        for kind, w, b, m, relu in image_layers(module):
+            if w is not None:
+                self.bias_f32[len(self.ops)] = None if b is None else b.contiguous()
+                w = w.to(torch.bfloat16).contiguous(memory_format=torch.channels_last)
+                b = None if b is None else b.to(torch.bfloat16)
+            self.ops.append((kind, w, b, m, relu))
 
     @classmethod
     def _conv_relu(cls, x, w, b, m):
@@ -407,18 +460,17 @@ class _FoldedSeq:
 
     def __call__(self, x, skip=None, defer_last_bias=False):
         """defer_last_bias: return (y, bias) with the last convolution's bias NOT applied (its consumer fuses it)."""
-        cl = torch.channels_last
         start = 0
         last = len(self.ops) - 1
         if self.ops[0][0] == "up":
-            a = _to_channels_last(x)
-            s = None if skip is None else _to_channels_last(skip)
+            a = _nhwc(x, torch.bfloat16).permute(0, 3, 1, 2)
+            s = None if skip is None else _nhwc(skip, torch.bfloat16).permute(0, 3, 1, 2)
             x = ops.upsample2x_cat(a, s)
             start = 1
         else:
             if skip is not None:
                 x = torch.cat([x, skip], dim=1)
-            x = _to_channels_last(x)
+            x = _nhwc(x, torch.bfloat16).permute(0, 3, 1, 2)
         for oi, (kind, w, b, m, relu) in enumerate(self.ops[start:], start):
             if kind == "conv":
                 if relu and b is not None:
@@ -436,94 +488,32 @@ class _FoldedSeq:
             elif kind == "lrelu":
                 x = F.leaky_relu(x, m.negative_slope)
             else:
-                x = ops.upsample2x_cat(_to_channels_last(x), None)
+                x = ops.upsample2x_cat(_nhwc(x, torch.bfloat16).permute(0, 3, 1, 2), None)
         return (x, None) if defer_last_bias else x
 
 
-class _OwnConvSeq:
-    """An image-branch conv stack (up_net block, patch_generator, seg_block, conv1x1) on our own implicit-GEMM kernels:
-    BatchNorm folded into the weights, every convolution one launch over NHWC maps with bias + ReLU in its epilogue --
-    ``split=True`` (float32 mode): the split-precision tensor-core kernel cp_gemm_x3 on fp32 maps; ``split=False`` (bf16
-    mode, image branch "tcgen05"): cp_conv_bf16 on bf16 maps.  The bilinear x2 upsampling of the concatenated skip
-    connection runs on cp_upsample2x_cat_nhwc.  NCHW in, NCHW (channels_last strides) out."""
+class _X3ConvSeq:
+    """The float32 image branch: every convolution of a conv stack one launch of the split-precision implicit GEMM cp_gemm_x3
+    over fp32 NHWC maps, bias + ReLU in its epilogue; the bilinear x2 upsampling of the concatenated skip connection runs on
+    cp_upsample2x_cat_nhwc.  NCHW in, NCHW (channels_last strides) out."""
 
-    def __init__(self, module, split=True):
-        self.split = split
-        self.dtype = torch.float32 if split else torch.bfloat16
-        pack = ops.pack_weight_split if split else ops.pack_weight
-        mods = list(module) if isinstance(module, nn.Sequential) else [module]
-        self.ops = []
-        i = 0
-        while i < len(mods):
-            m = mods[i]
-            if isinstance(m, (nn.Conv2d, nn.ConvTranspose2d)):
-                tr = isinstance(m, nn.ConvTranspose2d)
-                w = m.weight.detach().float()
-                b = None if m.bias is None else m.bias.detach().float()
-                if i + 1 < len(mods) and isinstance(mods[i + 1], nn.BatchNorm2d):
-                    bn = mods[i + 1]
-                    sc = bn.weight.detach().float() / torch.sqrt(bn.running_var.detach().float() + bn.eps)
-                    sh = bn.bias.detach().float() - sc * bn.running_mean.detach().float()
-                    w = w * (sc.view(1, -1, 1, 1) if tr else sc.view(-1, 1, 1, 1))
-                    b = sh if b is None else b * sc + sh
-                    i += 1
-                relu = i + 1 < len(mods) and isinstance(mods[i + 1], nn.ReLU)
-                if relu:
-                    i += 1
-                kh, kw = m.kernel_size
-                ok = (m.groups == 1 and tuple(m.dilation) == (1, 1) and m.padding[0] == m.padding[1] and
-                      (tuple(m.stride) == ((2, 2) if tr else (1, 1))) and (not tr or tuple(m.output_padding) == (1, 1)))
-                cin, cout = (w.shape[0], w.shape[1]) if tr else (w.shape[1], w.shape[0])
-                if not ok:
-                    raise RuntimeError(f"float32 image branch: unsupported convolution {m}")
-                wk = w.permute(1, 2, 3, 0) if tr else w.permute(0, 2, 3, 1)        # (cout, kh, kw, cin)
-                cin_pad = (cin + 63) // 64 * 64                                      # the kernel's K chunks are 64 channels
-                if cin_pad != cin:
-                    wk = F.pad(wk, (0, cin_pad - cin))
-                wm = wk.reshape(cout, kh * kw * cin_pad).contiguous()
-                self.ops.append(("convT" if tr else "conv", pack(wm), None if b is None else b.contiguous(),
-                                 (cout, kh, kw, int(m.padding[0]), cin_pad), relu))
-            elif isinstance(m, nn.UpsamplingBilinear2d):
-                if float(m.scale_factor) != 2.0:
-                    raise RuntimeError("image branch: only UpsamplingBilinear2d(scale_factor=2) is supported")
-                self.ops.append(("up", None, None, None, False))
-            elif isinstance(m, nn.ReLU):
-                self.ops.append(("relu", None, None, None, False))
-            else:
-                raise RuntimeError(f"unsupported layer in image branch: {type(m).__name__}")
-            i += 1
-
-    def _nhwc(self, x):
-        """NCHW (any strides) -> contiguous (B,H,W,C) of this stack's dtype."""
-        v = x.permute(0, 2, 3, 1)
-        if v.is_contiguous() and v.dtype == self.dtype:
-            return v
-        B, Cc, H, W = x.shape
-        return ops.to_node_major(x.contiguous().view(B, Cc, H * W), self.dtype).view(B, H, W, Cc)
+    def __init__(self, module):
+        self.ops = _gemm_layers(module, ops.pack_weight_split, "float32")
 
     def __call__(self, x, skip=None):
-        conv = ops.gemm_x3_conv if self.split else ops.conv_bf16
         start = 0
         if self.ops[0][0] == "up":
-            a = self._nhwc(x).permute(0, 3, 1, 2)
-            s = None if skip is None else self._nhwc(skip).permute(0, 3, 1, 2)
+            a = _nhwc(x, torch.float32).permute(0, 3, 1, 2)
+            s = None if skip is None else _nhwc(skip, torch.float32).permute(0, 3, 1, 2)
             y = ops.upsample2x_cat(a, s).permute(0, 2, 3, 1)         # (B,2H,2W,Ca+Cb) contiguous
             start = 1
         else:
             if skip is not None:
                 x = torch.cat([x, skip], dim=1)
-            y = self._nhwc(x)
+            y = _nhwc(x, torch.float32)
         for kind, ws, b, geom, relu in self.ops[start:]:
             if kind in ("conv", "convT"):
-                cout, kh, kw, pad, cin_pad = geom
-                if y.shape[-1] != cin_pad:                    # zero channels up to the kernel's 64-channel granularity
-                    y = F.pad(y, (0, cin_pad - y.shape[-1]))
-                H, W = y.shape[1], y.shape[2]
-                if kind == "conv":
-                    Ho, Wo = H + 2 * pad - kh + 1, W + 2 * pad - kw + 1
-                else:
-                    Ho, Wo = (H - 1) * 2 - 2 * pad + kh + 1, (W - 1) * 2 - 2 * pad + kw + 1
-                y = conv(y, ws, cout, kh, kw, pad, Ho, Wo, b, relu, 0.0, transposed=(kind == "convT"))
+                y = _gather_conv(ops.gemm_x3_conv, y, kind, ws, b, geom, relu)
             elif kind == "relu":
                 y = torch.relu_(y)
             else:
@@ -531,7 +521,7 @@ class _OwnConvSeq:
         return y.permute(0, 3, 1, 2)
 
 
-class _SlabConvSeq(_OwnConvSeq):
+class _SlabConvSeq:
     """The bf16 image branch on cp_conv_slab: every map of a block lives in a BORDERED NHWC buffer (B, H+1, W+1, C) -- a zero
     last row and last column per image, which over the flat pixel index are all four borders at once -- so that a kernel tap is
     a row shift of one TMA-loaded activation slab (csrc/conv_slab_tcgen05.cu).  The x2 upsampling of the concatenated skip
@@ -543,7 +533,7 @@ class _SlabConvSeq(_OwnConvSeq):
     back to the gather kernel cp_conv_bf16."""
 
     def __init__(self, module):
-        super().__init__(module, split=False)
+        self.ops = _gemm_layers(module, ops.pack_weight, "bf16")
 
     @staticmethod
     def _view(buf):
@@ -551,15 +541,12 @@ class _SlabConvSeq(_OwnConvSeq):
         y._cp_padded = buf
         return y
 
-    def _cl(self, x):
+    @staticmethod
+    def _cl(x):
         """(B,C,H,W) -> a bf16 view / copy with channel stride 1 (what the upsampling kernel reads)."""
         if x.dtype == torch.bfloat16 and x.stride(1) == 1 and all(st % 8 == 0 for st in (x.stride(0), x.stride(2), x.stride(3))):
             return x
-        return self._nhwc(x).permute(0, 3, 1, 2)
-
-    @staticmethod
-    def _pad_channels(buf, cin_pad):
-        return buf if buf.shape[-1] == cin_pad else F.pad(buf, (0, cin_pad - buf.shape[-1]))
+        return _nhwc(x, torch.bfloat16).permute(0, 3, 1, 2)
 
     def __call__(self, x, skip=None, seg=None):
         """``seg`` = (weight (n, C), bias (n,)) f32 of a 1x1 convolution to fuse into this block's LAST convolution: the
@@ -576,14 +563,14 @@ class _SlabConvSeq(_OwnConvSeq):
             _, ws, b, (cout, kh, kw, pad, cin_pad), relu = kinds[0]
             if skip is not None:
                 x = torch.cat([x, skip], dim=1)
-            buf = ops.convT_slab(self._pad_channels(self._nhwc(x), cin_pad), ws, cout, b, relu, 0.0)
+            buf = ops.convT_slab(_pad_channels(_nhwc(x, torch.bfloat16), cin_pad), ws, cout, b, relu, 0.0)
             start = 1
         else:
             buf = getattr(x, "_cp_padded", None) if skip is None else None
             if buf is None:
                 if skip is not None:
                     x = torch.cat([x, skip], dim=1)
-                y = self._nhwc(x)
+                y = _nhwc(x, torch.bfloat16)
         for oi in range(start, len(kinds)):
             kind, ws, b, geom, relu = kinds[oi]
             if kind == "relu":
@@ -600,7 +587,7 @@ class _SlabConvSeq(_OwnConvSeq):
             if cout <= 256 and (same or full):
                 if buf is None:
                     buf, y = ops.to_bordered(y), None
-                buf = self._pad_channels(buf, cin_pad)
+                buf = _pad_channels(buf, cin_pad)
                 if same:
                     if seg is not None and oi == len(kinds) - 1 and seg[0].shape[1] == cout:
                         buf, seg_out = ops.conv_slab_same(buf, ws, cout, kh, kw, b, relu, 0.0, seg=seg)
@@ -612,13 +599,7 @@ class _SlabConvSeq(_OwnConvSeq):
             # gather kernel on a contiguous map
             if buf is not None:
                 y, buf = buf[:, :-1, :-1, :].contiguous(), None
-            y = self._pad_channels(y, cin_pad)
-            H, W = y.shape[1], y.shape[2]
-            if kind == "conv":
-                Ho, Wo = H + 2 * pad - kh + 1, W + 2 * pad - kw + 1
-            else:
-                Ho, Wo = (H - 1) * 2 - 2 * pad + kh + 1, (W - 1) * 2 - 2 * pad + kw + 1
-            y = ops.conv_bf16(y, ws, cout, kh, kw, pad, Ho, Wo, b, relu, 0.0, transposed=(kind == "convT"))
+            y = _gather_conv(ops.conv_bf16, y, kind, ws, b, geom, relu)
         res = self._view(buf) if buf is not None else y.permute(0, 3, 1, 2)
         res._cp_seg = seg_out
         return res
@@ -626,7 +607,7 @@ class _SlabConvSeq(_OwnConvSeq):
 
 def _x3_module(module):
     _require_eval(module)
-    return _PREP.get(module, ("x3seq",), lambda: _OwnConvSeq(module, split=True))
+    return _PREP.get(module, ("x3seq",), lambda: _X3ConvSeq(module))
 
 
 def _tc_module(module):

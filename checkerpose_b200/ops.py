@@ -249,23 +249,29 @@ def gemm_x3_linear(a1, w_split, nout, bias=None, act=False, slope=0.0, a2=None, 
     return out
 
 
+def _conv_gemm_params(p, x_nhwc, dtype, nout, KH, KW, pad, Ho, Wo, bias, act, slope, transposed):
+    """Fill the fields cp_gemm_x3_params and cp_conv_bf16_params share for Conv2d KH x KW stride 1 / ConvTranspose2d stride 2
+    of the NHWC map x_nhwc (B,H,W,Cin) of ``dtype`` -> the (B,Ho,Wo,nout) output map of ``dtype``."""
+    assert x_nhwc.dtype == dtype and x_nhwc.is_contiguous() and x_nhwc.dim() == 4
+    B, H, W, Cin = x_nhwc.shape
+    out = torch.empty((B, Ho, Wo, nout), dtype=dtype, device=x_nhwc.device)
+    p.mode = X3_CONVT if transposed else X3_CONV
+    p.a1, p.ld1, p.k1 = _p(x_nhwc), Cin, Cin
+    p.H, p.W, p.Ho, p.Wo, p.KH, p.KW, p.pad = H, W, int(Ho), int(Wo), int(KH), int(KW), int(pad)
+    p.M, p.K = B * Ho * Wo, KH * KW * Cin
+    p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
+    p.out, p.ld_out, p.Nout = _p(out), int(nout), int(nout)
+    return out
+
+
 def gemm_x3_conv(x_nhwc, w_split, nout, KH, KW, pad, Ho, Wo, bias=None, act=False, slope=0.0, transposed=False):
     """Conv2d KH x KW stride 1 / ConvTranspose2d stride 2 over an fp32 NHWC map (B,H,W,Cin) -> (B,Ho,Wo,nout) fp32, as an
     implicit GEMM on the tensor cores (cp_gemm_x3, CP_X3_CONV / CP_X3_CONVT); W rows in (ky, kx, c) order."""
     _need_cuda(x_nhwc, bias, w_split[0], w_split[1])
-    assert x_nhwc.dtype == torch.float32 and x_nhwc.is_contiguous() and x_nhwc.dim() == 4
-    B, H, W, Cin = x_nhwc.shape
-    out = torch.empty((B, Ho, Wo, nout), dtype=torch.float32, device=x_nhwc.device)
     p = GemmX3Params()
-    p.mode = X3_CONVT if transposed else X3_CONV
-    p.a1, p.ld1, p.k1 = _p(x_nhwc), Cin, Cin
-    p.a2, p.ld2, p.k2 = None, 0, 0
-    p.H, p.W, p.Ho, p.Wo, p.KH, p.KW, p.pad = H, W, int(Ho), int(Wo), int(KH), int(KW), int(pad)
-    p.M, p.K = B * Ho * Wo, KH * KW * Cin
+    out = _conv_gemm_params(p, x_nhwc, torch.float32, nout, KH, KW, pad, Ho, Wo, bias, act, slope, transposed)
     p.w_hi, p.w_lo = _p(w_split[0]), _p(w_split[1])
-    p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
-    p.out, p.ld_out, p.Nout = _p(out), int(nout), int(nout)
-    _timed_launch(lib.cp_gemm_x3, "cp_gemm_x3", p, ("X3C", KH * KW * Cin, (int(nout),), OUT_F32, B * Ho * Wo, 0))
+    _timed_launch(lib.cp_gemm_x3, "cp_gemm_x3", p, ("X3C", p.K, (int(nout),), OUT_F32, p.M, 0))
     return out
 
 
@@ -274,40 +280,10 @@ def conv_bf16(x_nhwc, w_packed, nout, KH, KW, pad, Ho, Wo, bias=None, act=False,
     """Conv2d KH x KW stride 1 / ConvTranspose2d stride 2 over a bf16 NHWC map (B,H,W,Cin) -> (B,Ho,Wo,nout) bf16 as an implicit
     GEMM on the tensor cores (cp_conv_bf16); W rows in (ky, kx, c) order, packed by pack_weight."""
     _need_cuda(x_nhwc, bias, w_packed)
-    assert x_nhwc.dtype == torch.bfloat16 and x_nhwc.is_contiguous() and x_nhwc.dim() == 4
-    B, H, W, Cin = x_nhwc.shape
-    out = torch.empty((B, Ho, Wo, nout), dtype=torch.bfloat16, device=x_nhwc.device)
     p = ConvBf16Params()
-    p.mode = X3_CONVT if transposed else X3_CONV
-    p.a1, p.ld1, p.k1 = _p(x_nhwc), Cin, Cin
-    p.a2, p.ld2, p.k2 = None, 0, 0
-    p.H, p.W, p.Ho, p.Wo, p.KH, p.KW, p.pad = H, W, int(Ho), int(Wo), int(KH), int(KW), int(pad)
-    p.M, p.K = B * Ho * Wo, KH * KW * Cin
+    out = _conv_gemm_params(p, x_nhwc, torch.bfloat16, nout, KH, KW, pad, Ho, Wo, bias, act, slope, transposed)
     p.w_packed = _p(w_packed)
-    p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
-    p.out, p.ld_out, p.Nout = _p(out), int(nout), int(nout)
-    _timed_launch(lib.cp_conv_bf16, "cp_conv_bf16", p, ("CV", KH * KW * Cin, (int(nout),), OUT_BF16, B * Ho * Wo, 0))
-    return out
-
-
-def linear_bf16(a1, w_packed, nout, bias=None, act=False, slope=0.0, a2=None, out=None):
-    """y = act([a1|a2] @ W.T + bias), bf16 rows in / bf16 out, on cp_conv_bf16's LINEAR mode."""
-    _need_cuda(a1, a2, bias, w_packed)
-    assert a1.dtype == torch.bfloat16 and a1.is_contiguous()
-    K1 = a1.shape[-1]
-    M = a1.numel() // K1
-    K2 = 0 if a2 is None else a2.shape[-1]
-    if out is None:
-        out = torch.empty(a1.shape[:-1] + (nout,), dtype=torch.bfloat16, device=a1.device)
-    p = ConvBf16Params()
-    p.mode = X3_LINEAR
-    p.a1, p.ld1, p.k1 = _p(a1), K1, K1
-    p.a2, p.ld2, p.k2 = _p(a2), K2, K2
-    p.M, p.K = M, K1 + K2
-    p.w_packed = _p(w_packed)
-    p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
-    p.out, p.ld_out, p.Nout = _p(out), out.stride(-2) if out.dim() > 1 else nout, int(nout)
-    _timed_launch(lib.cp_conv_bf16, "cp_conv_bf16", p, ("LB", K1 + K2, (int(nout),), OUT_BF16, M, 0))
+    _timed_launch(lib.cp_conv_bf16, "cp_conv_bf16", p, ("CV", p.K, (int(nout),), OUT_BF16, p.M, 0))
     return out
 
 
@@ -322,6 +298,19 @@ def _slab_common(xp, w_packed, K, nout, bias, act, slope):
     p.bias, p.act, p.slope = _p(bias), int(bool(act)), float(slope)
     p.Nout = int(nout)
     return p
+
+
+def _slab_grid_taps(p, KH, KW, Wp, cy, cx):
+    """One phase of KH x KW taps over the stored grid: tap (ky, kx) reads the row shift (ky - cy) * Wp + (kx - cx)."""
+    p.num_phases = 1
+    ph = p.phase[0]
+    ph.ntaps = KH * KW
+    for ky in range(KH):
+        for kx in range(KW):
+            t = ky * KW + kx
+            ph.wtap[t] = t
+            ph.shift[t] = (ky - cy) * Wp + (kx - cx)
+    p.compact = 0
 
 
 def zero_border(xp):
@@ -366,16 +355,8 @@ def conv_slab_same(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0, 
     seg_out = _slab_seg(p, seg, B, Hp, Wp, nout, xp.device)
     out = torch.empty((B, Hp, Wp, nout), dtype=torch.bfloat16, device=xp.device)
     p.out, p.ld_out = _p(out), int(nout)
-    p.num_phases = 1
-    ph = p.phase[0]
-    ph.ntaps = KH * KW
-    for ky in range(KH):
-        for kx in range(KW):
-            t = ky * KW + kx
-            ph.wtap[t] = t
-            ph.shift[t] = (ky - KH // 2) * Wp + (kx - KW // 2)
+    _slab_grid_taps(p, KH, KW, Wp, KH // 2, KW // 2)
     p.vy0, p.vy1, p.vx0, p.vx1 = 0, Hp - 1, 0, Wp - 1
-    p.compact = 0
     # signature: ..., rows of the launch, multiply-accumulates of the convolution proper (without the border rows)
     _timed_launch(lib.cp_conv_slab, "cp_conv_slab", p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * (Hp - 1) * (Wp - 1) * KH * KW * Cin * int(nout)))
     return out if seg is None else (out, seg_out)
@@ -390,16 +371,8 @@ def conv_slab_full(xp, w_packed, nout, KH, KW, bias=None, act=False, slope=0.0):
     p = _slab_common(xp, w_packed, KH * KW * Cin, nout, bias, act, slope)
     out = torch.empty((B, Hp, Wp, nout), dtype=torch.bfloat16, device=xp.device)
     p.out, p.ld_out = _p(out), int(nout)
-    p.num_phases = 1
-    ph = p.phase[0]
-    ph.ntaps = KH * KW
-    for ky in range(KH):
-        for kx in range(KW):
-            t = ky * KW + kx
-            ph.wtap[t] = t
-            ph.shift[t] = (ky - 1) * Wp + (kx - 1)
+    _slab_grid_taps(p, KH, KW, Wp, 1, 1)
     p.vy0, p.vy1, p.vx0, p.vx1 = 0, Hp, 0, Wp
-    p.compact = 0
     _timed_launch(lib.cp_conv_slab, "cp_conv_slab", p, ("CS", KH * KW * Cin, (int(nout),), OUT_BF16, B * Hp * Wp, B * Hp * Wp * KH * KW * Cin * int(nout)))
     return out
 
@@ -439,18 +412,11 @@ def convT_slab(x_nhwc, w_packed, nout, bias=None, act=False, slope=0.0):
 
 def upsample2x_cat_padded(a, b=None):
     """upsample2x_cat writing the interior of a bordered NHWC map: returns (B, 2H+1, 2W+1, Ca+Cb) contiguous."""
-    _need_cuda(a, b)
-    B, Ca, H, W = a.shape
-    Cb = 0 if b is None else b.shape[1]
-    if b is not None and (b.shape[0] != B or b.shape[2:] != a.shape[2:] or b.dtype != a.dtype):
-        raise RuntimeError("upsample2x_cat: sources disagree in shape or dtype")
-    Ct = Ca + Cb
+    B, Ct, H, W, src = _upsample_sources(a, b)
     out = torch.empty((B, 2 * H + 1, 2 * W + 1, Ct), dtype=a.dtype, device=a.device)
     zero_border(out)
-    sa = _nhwc_strides(a)
-    sb = (0, 0, 0) if b is None else _nhwc_strides(b)
-    check(lib.cp_upsample2x_cat_nhwc_to(_p(a), sa[0], sa[1], sa[2], Ca, _p(b), sb[0], sb[1], sb[2], Cb, _dt(a), _p(out),
-                                        out.stride(0), out.stride(1), out.stride(2), B, H, W, _stream()), "cp_upsample2x_cat_nhwc_to")
+    check(lib.cp_upsample2x_cat_nhwc_to(*src, _p(out), out.stride(0), out.stride(1), out.stride(2), B, H, W, _stream()),
+          "cp_upsample2x_cat_nhwc_to")
     _count()
     return out
 
@@ -526,19 +492,24 @@ def _nhwc_strides(t):
     return t.stride(0), t.stride(2), t.stride(3)
 
 
-def upsample2x_cat(a, b=None):
-    """Bilinear x2 (align_corners=True) of cat([a, b], 1) for channels_last (B,C,H,W) inputs.
-    Returns a channels_last (B, Ca+Cb, 2H, 2W) tensor (a permuted view of NHWC storage)."""
+def _upsample_sources(a, b):
+    """Check the sources of the x2 upsampling -> (B, Ca+Cb, H, W, the source arguments of cp_upsample2x_cat_nhwc[_to])."""
     _need_cuda(a, b)
     B, Ca, H, W = a.shape
     Cb = 0 if b is None else b.shape[1]
     if b is not None and (b.shape[0] != B or b.shape[2:] != a.shape[2:] or b.dtype != a.dtype):
         raise RuntimeError("upsample2x_cat: sources disagree in shape or dtype")
-    out = torch.empty((B, 2 * H, 2 * W, Ca + Cb), dtype=a.dtype, device=a.device)
     sa = _nhwc_strides(a)
     sb = (0, 0, 0) if b is None else _nhwc_strides(b)
-    check(lib.cp_upsample2x_cat_nhwc(_p(a), sa[0], sa[1], sa[2], Ca, _p(b), sb[0], sb[1], sb[2], Cb, _dt(a), _p(out),
-                                     B, H, W, _stream()), "cp_upsample2x_cat_nhwc")
+    return B, Ca + Cb, H, W, (_p(a), *sa, Ca, _p(b), *sb, Cb, _dt(a))
+
+
+def upsample2x_cat(a, b=None):
+    """Bilinear x2 (align_corners=True) of cat([a, b], 1) for channels_last (B,C,H,W) inputs.
+    Returns a channels_last (B, Ca+Cb, 2H, 2W) tensor (a permuted view of NHWC storage)."""
+    B, Ct, H, W, src = _upsample_sources(a, b)
+    out = torch.empty((B, 2 * H, 2 * W, Ct), dtype=a.dtype, device=a.device)
+    check(lib.cp_upsample2x_cat_nhwc(*src, _p(out), B, H, W, _stream()), "cp_upsample2x_cat_nhwc")
     _count()
     return out.permute(0, 3, 1, 2)
 

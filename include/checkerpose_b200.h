@@ -118,8 +118,8 @@ typedef struct {
 int cp_pack_weight_split(const float* w, int Nout, int K, void* packed_hi, void* packed_lo, cp_stream_t s);
 int cp_gemm_x3(const cp_gemm_x3_params* p, cp_stream_t s);
 
-/* ---- bf16 implicit-GEMM convolution / Linear on tcgen05 (conv_bf16_tcgen05.cu): the image branch of the bf16 mode ----
- * Same operand gather as cp_gemm_x3 (CP_X3_LINEAR / CP_X3_CONV / CP_X3_CONVT) with bf16 activations and one MMA per K step:
+/* ---- bf16 implicit-GEMM convolution on tcgen05 (conv_bf16_tcgen05.cu): the image branch of the bf16 mode ----
+ * Same operand gather as cp_gemm_x3 (CP_X3_CONV / CP_X3_CONVT) with bf16 activations and one MMA per K step:
  * out[m, :Nout] = act(A[m, :K] . W^T + bias), bf16 in / bf16 out, fp32 accumulation; W packed by cp_pack_weight with rows in
  * (ky, kx, c) order; BatchNorm folded into W / bias by the caller; act: 0 = none, 1 = LeakyReLU(slope) (slope 0 = ReLU).
  * Replaces the cuDNN calls of get_gdrn_upsample_module (pipeline.py:183-211), patch_generator (:144-145), seg_block (:349,383)
@@ -127,7 +127,6 @@ int cp_gemm_x3(const cp_gemm_x3_params* p, cp_stream_t s);
 typedef struct {
   int mode;
   const void* a1; int ld1; int k1;
-  const void* a2; int ld2; int k2;
   int H, W, Ho, Wo, KH, KW, pad;
   int64_t M; int K;
   const void* w_packed;
