@@ -4,6 +4,7 @@ import sys
 
 import numpy as np
 import torch
+import torch.nn.functional as F
 
 REPO = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 if REPO not in sys.path:
@@ -105,3 +106,25 @@ def rel_err(a, b):
     b = np.asarray(b, dtype=np.float64)
     floor = np.sqrt((b ** 2).mean()) + 1e-30
     return float((np.abs(a - b) / np.maximum(np.abs(b), floor)).max())
+
+
+def rel_max(got, ref):
+    """max |got - ref| / max |ref| (ref float64)."""
+    return float((got.double() - ref).abs().max() / ref.abs().max())
+
+
+def bf16r(t):
+    """t rounded to bf16, as float32."""
+    return t.to(torch.bfloat16).float()
+
+
+def agg_rows(z, nb, bi, ni, Co, slope, round_bf16):
+    """A[b, n] = lrelu(max_k P[b, nb[b, n, k]] + Q[b, n]) for the listed rows: exact max, one fp32 add, fp32 LeakyReLU
+    (the kernels' arithmetic), then one rounding to bf16 when the kernel stores bf16.  z (B,N,2Co) float32 values (bf16
+    promotes exactly); the result is on z's device."""
+    idx = nb[bi, ni]                                                  # (R,K)
+    m = torch.full((len(bi), Co), float("-inf"), device=z.device)
+    for k in range(idx.shape[1]):
+        m = torch.maximum(m, z[bi, idx[:, k], :Co])
+    a = F.leaky_relu(m + z[bi, ni, Co:], slope)
+    return bf16r(a) if round_bf16 else a

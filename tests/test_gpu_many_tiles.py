@@ -22,7 +22,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import syn
+from helpers import agg_rows, bf16r, rel_max, syn
 
 pytestmark = pytest.mark.gpu
 torch.set_grad_enabled(False)
@@ -104,14 +104,6 @@ def image_chunks(B, rows_per_image, cap_tiles):
     step = cap_tiles * TILE // rows_per_image
     assert step >= 1
     return [(b0, min(B, b0 + step)) for b0 in range(0, B, step)]
-
-
-def rel_max(got, ref):
-    return float((got.double() - ref).abs().max() / ref.abs().max())
-
-
-def bf16r(t):
-    return t.to(torch.bfloat16).float()
 
 
 def lrelu64(x, s):
@@ -522,17 +514,6 @@ def test_chain_load_many_tiles(ops, what):
 
 
 # ------------------------------------------------------------------------------------------------ EdgeConv aggregation
-def agg_rows(z, nb, bi, ni, Co, slope, round_bf16):
-    """A[b, n] = lrelu(max_k P[b, nb[b, n, k]] + Q[b, n]) for the listed rows: exact max, one fp32 add, fp32 LeakyReLU
-    (the kernels' arithmetic), then one rounding to bf16 when the kernel stores bf16.  z (B,N,2Co) float32 values."""
-    idx = nb[bi, ni]                                                  # (R,K)
-    m = torch.full((len(bi), Co), float("-inf"))
-    for k in range(idx.shape[1]):
-        m = torch.maximum(m, z[bi, idx[:, k], :Co])
-    a = F.leaky_relu(m + z[bi, ni, Co:], slope)
-    return bf16r(a) if round_bf16 else a
-
-
 def lm_graphs(ops, objs, N, K):
     p3d = torch.cat([syn.p3d_normed_tensor(syn.load_fps_xyz("lm", o, N)) for o in objs], dim=0).cuda()
     _, idx32 = ops.knn(p3d, K, want_i32=True)
@@ -676,7 +657,9 @@ def _run_head(wl, case, feats, bbox, obj_ids):
                                               ("full4096", torch.float32, None, None),
                                               ("lm_sweep", torch.bfloat16, 4096, 20),
                                               ("lm_sweep", torch.bfloat16, 4096, 40),
-                                              ("init64", torch.bfloat16, None, None)])
+                                              ("init64", torch.bfloat16, None, None),
+                                              ("ycbv1024", torch.bfloat16, None, None),
+                                              ("ycbv1024", torch.float32, None, None)])
 def test_head_at_bench_batch_is_batch_independent(ops, monkeypatch, config, dtype, N, K):
     """The benchmark's timed batch (bench.py: same nets, seeds, objects and max_batch_size) is bit-identical, output for
     output, to the same RoIs run in 2-RoI batches -- the regime test_gpu_head.py anchors to the oracle -- and a permuted
