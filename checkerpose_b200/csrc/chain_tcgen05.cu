@@ -1,7 +1,6 @@
 // Fused tcgen05 "chain" kernel: the bf16 tensor-core path of the GNN keypoint head.
 //
-// One persistent CTA (256 threads, two CTAs per SM) walks over tiles of 128 keypoints ("nodes") of
-// one RoI.  Per tile:
+// One persistent CTA (256 threads) walks over tiles of 128 keypoints ("nodes") of one RoI.  Per tile:
 //
 //   PROLOGUE  builds the A operand (128 nodes x K channels, bf16) straight in shared memory, in the
 //             K-major SWIZZLE_128B layout tcgen05.mma reads -- it never exists in HBM:
@@ -13,11 +12,24 @@
 //                      phase) the previous graph feature, i.e. the concat of pipeline.py:283
 //   GEMMs     up to three chained Linear(+bias+LeakyReLU) layers on tcgen05: weights are pre-packed
 //             tile images streamed by one producer thread with cp.async.bulk (TMA engine) into a
-//             2-stage mbarrier ring; one elected thread issues tcgen05.mma (M=128, N<=128, K=16) with
-//             fp32 accumulators in TMEM (256 columns per CTA); tcgen05.commit signals stage release and
-//             accumulator-ready.  Between layers the epilogue converts TMEM -> bf16 and writes the
-//             next A operand back into the same shared-memory tile.
+//             3-stage mbarrier ring; one elected thread issues tcgen05.mma (M=128, N<=128, K=16) with
+//             fp32 accumulators in TMEM; tcgen05.commit signals stage release and accumulator-ready.
+//             Between layers the epilogue converts TMEM -> bf16 and writes the next A operand back into
+//             the same shared-memory tile.
 //   OUTPUT    bf16 [P|Q] table for the next EdgeConv layer, or fp32 logits.
+//
+// Two instantiations of every prologue, chosen per launch by the host from the widths:
+//   narrow  K <= 256 resident (A = 64 KB), weight ring 3 x 16 KB: 113 KB of shared memory, two CTAs per SM, 256 TMEM
+//           columns each.  Every width the shipped head (query_dims 256_256_64) launches here fits it.
+//   wide    K <= 512 resident (A = 128 x 512 bf16 = 128 KB), the same ring: 176.3 KB, one CTA per SM, which then owns
+//           all 512 TMEM columns.  A chained layer accumulates its whole output (nout <= 512) in TMEM before the epilogue
+//           overwrites the A tile with it.  A last layer wider than the TMEM columns of the CTA (the [P|Q] table of an
+//           EdgeConv with C' = 512 has 1024 columns; 512 in the narrow kernel) runs as column passes over the same A
+//           tile: pass j accumulates output columns [j*TMEM_COLS, (j+1)*TMEM_COLS) and its epilogue stores them to global
+//           before the next pass reuses the accumulator.  Layer 0 of TAPS is the exception: its second K phase replaces the
+//           taps in the A tile with the graph feature, so the host runs it in one pass (nout <= 512, wide above 256).
+// Widths are multiples of 64 (E, the patch-embedding width of TAPS, a multiple of 16, so that the four taps fill whole
+// 64-channel K chunks); the head pads other widths with exact zeros (head.py, pad_linear_weight / pad_edgeconv).
 //
 // Roofline: with the factored EdgeConv the layer is bandwidth-bound (DESIGN.md section 5); the tensor
 // work per tile (128 x 512 x 256 MACs) is ~4k cycles against a gather of 128 x K x 512 B from L2.
@@ -34,22 +46,29 @@ constexpr int NTHREADS = 256;
 constexpr int NWARPS = 8;
 constexpr int KCHUNK = 64;                       // bf16 elements per 128-byte swizzle row
 constexpr int A_CHUNK_BYTES = TILE_M * 128;      // 16 KB: 128 rows x 64 bf16
-constexpr int A_CHUNKS = 4;                      // K <= 256 resident at a time
 constexpr int B_STAGE_BYTES = 128 * 128;         // 16 KB: <=128 weight rows x 64 bf16
 constexpr int STAGES = 3;
-constexpr int TMEM_COLS = 256;
-constexpr int MAX_WTILES = 48;
-// two CTAs per SM: 2 x (SMEM_BYTES + 1 KB reserved) must stay within 227 KB, so there is no alignment slack -- the
-// kernel traps if the dynamic shared-memory window is not 1024-byte aligned (it is: windows are 1 KB granular)
-constexpr int SMEM_BYTES = A_CHUNKS * A_CHUNK_BYTES + STAGES * B_STAGE_BYTES + 256;
-static_assert(2 * (SMEM_BYTES + 1024) <= 227 * 1024, "two CTAs per SM");
 
+template <bool WIDE>
+struct Cfg {
+  static constexpr int A_CHUNKS = WIDE ? 8 : 4;          // K resident at a time: 512 / 256
+  static constexpr int TMEM_COLS = WIDE ? 512 : 256;     // the whole TMEM of the SM / half of it
+  static constexpr int CTAS_PER_SM = WIDE ? 1 : 2;
+  static constexpr int MAX_WTILES = WIDE ? 160 : 48;     // wide: TAPS 128+512 -> 512 -> 512 -> [P|Q] 1024 takes 160
+  static constexpr int SMEM_BYTES = A_CHUNKS * A_CHUNK_BYTES + STAGES * B_STAGE_BYTES + 256;
+};
+// narrow: two CTAs per SM, 2 x (SMEM_BYTES + 1 KB reserved) must stay within 227 KB, so there is no alignment slack -- the
+// kernel traps if the dynamic shared-memory window is not 1024-byte aligned (it is: windows are 1 KB granular)
+static_assert(2 * (Cfg<false>::SMEM_BYTES + 1024) <= 227 * 1024, "two narrow CTAs per SM");
+static_assert(Cfg<true>::SMEM_BYTES + 1024 <= 227 * 1024, "one wide CTA per SM");
+
+template <bool WIDE>
 struct KParams {
   cp_chain_params p;
   int tiles_per_roi;
   int num_node_tiles;
   int T;  // weight tiles per node tile
-  cp::WTile wt[MAX_WTILES];
+  cp::WTile wt[Cfg<WIDE>::MAX_WTILES];
 };
 
 struct Smem {
@@ -72,38 +91,44 @@ __device__ __forceinline__ uint32_t bf2_max(uint32_t a, uint32_t b) {
 }
 
 // ---- prologues: all 256 threads fill A chunks [0, C/64) for the 128 rows of the tile -----------------
+// A row of C channels is C/8 16-byte pieces.  For C in {64,128,256} a warp covers whole rows with a fixed piece per lane;
+// any other multiple of 64 (up to 512) walks the 128 x C/8 pieces of the tile in thread order, which for the three
+// powers of two is the same assignment.
 
-// rows of a node-major bf16 tensor; C in {64,128,256}.  cp.async (LDGSTS) straight into the swizzled operand layout,
-// zero-filled beyond rows_valid: all of a thread's 16-byte pieces (up to 16 at C = 256) are in flight at once -- one
+// rows of a node-major bf16 tensor.  cp.async (LDGSTS) straight into the swizzled operand layout,
+// zero-filled beyond rows_valid: all of a thread's 16-byte pieces (up to 32 at C = 512) are in flight at once -- one
 // memory round trip per tile instead of the four of the register-staged version (0.224 -> see DESIGN.md section 8).
 __device__ __forceinline__ void fill_rows(uint8_t* A, const bf16* src, int ld, int C, int64_t row0, int rows_valid) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int cpr = C >> 3;  // 16-byte chunks per row
-  const int rpi = 32 / cpr;
-  const int sub = lane / cpr, chunk = lane - sub * cpr;
   const uint32_t a_s = sm100::smem_u32(A);
-  for (int r = warp * rpi + sub; r < TILE_M; r += NWARPS * rpi) {
+  auto piece = [&](int r, int chunk) {
     const bool ok = r < rows_valid;
     const void* g = src + (ok ? (row0 + r) * ld + chunk * 8 : 0);
     cp_async16_zfill(a_s + a_offset(chunk >> 3, r, chunk & 7), g, ok ? 16u : 0u);
+  };
+  if ((32 % cpr) == 0) {
+    const int rpi = 32 / cpr;
+    const int sub = lane / cpr, chunk = lane - sub * cpr;
+    for (int r = warp * rpi + sub; r < TILE_M; r += NWARPS * rpi) piece(r, chunk);
+  } else {
+    for (int it = threadIdx.x; it < TILE_M * cpr; it += NTHREADS) piece(it / cpr, it % cpr);
   }
   asm volatile("cp.async.commit_group;" ::: "memory");
   asm volatile("cp.async.wait_group 0;" ::: "memory");
 }
 
-// EdgeConv aggregation; Co in {64,128,256}
+// EdgeConv aggregation; Co a multiple of 64, <= 512
 __device__ __forceinline__ void fill_agg(uint8_t* A, const cp_chain_params& p, int b, int n0, int rows_valid) {
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int Co = p.Co, K = p.K;
   const int cpr = Co >> 3;
-  const int rpi = 32 / cpr;
-  const int sub = lane / cpr, chunk = lane - sub * cpr;
   const int g = p.graph_sel ? p.graph_sel[b] : 0;
   const int32_t* idx_g = p.idx + (size_t)g * p.N * K;
   const bf16* zb = reinterpret_cast<const bf16*>(p.z) + (size_t)b * p.N * p.ld_z;
   bf16* aout = p.a_out ? reinterpret_cast<bf16*>(p.a_out) + (size_t)b * p.N * p.ld_a_out : nullptr;
   const float slope = p.agg_slope;
-  for (int r = warp * rpi + sub; r < TILE_M; r += NWARPS * rpi) {
+  auto piece = [&](int r, int chunk) {
     uint4 o = make_uint4(0, 0, 0, 0);
     if (r < rows_valid) {
       const int i = n0 + r;
@@ -139,11 +164,44 @@ __device__ __forceinline__ void fill_agg(uint8_t* A, const cp_chain_params& p, i
       if (aout) *reinterpret_cast<uint4*>(aout + (size_t)i * p.ld_a_out + chunk * 8) = o;
     }
     *reinterpret_cast<uint4*>(A + a_offset(chunk >> 3, r, chunk & 7)) = o;
+  };
+  if ((32 % cpr) == 0) {
+    const int rpi = 32 / cpr;
+    const int sub = lane / cpr, chunk = lane - sub * cpr;
+    for (int r = warp * rpi + sub; r < TILE_M; r += NWARPS * rpi) piece(r, chunk);
+  } else {
+    for (int it = threadIdx.x; it < TILE_M * cpr; it += NTHREADS) piece(it / cpr, it % cpr);
+  }
+}
+
+// Index2Feat taps of any E (a multiple of 16, <= 128), masked: K column tap * E + e, as cp_sample_taps lays them out.
+// A row is 4E/8 pieces of 16 bytes, walked in thread order; piece j is K chunk j/8, 16-byte chunk j%8.
+__device__ __forceinline__ void fill_taps_any(uint8_t* A, const cp_chain_params& p, int b, int n0, int rows_valid) {
+  const int E = p.E;
+  const int ppt = E >> 3, ppr = 4 * ppt;   // pieces per tap / per row
+  const bf16* pb = reinterpret_cast<const bf16*>(p.patches) + (size_t)b * p.Hp * p.Wp * E;
+  for (int it = threadIdx.x; it < TILE_M * ppr; it += NTHREADS) {
+    const int r = it / ppr, j = it - r * ppr;
+    const int tap = j / ppt, c8 = j - tap * ppt;
+    uint4 v = make_uint4(0, 0, 0, 0);
+    if (r < rows_valid) {
+      const size_t e = (size_t)b * p.N + n0 + r;
+      const float mk = p.mask ? __ldg(p.mask + e) : 1.f;
+      const int yy = (int)(2 * __ldg(p.y_id + e)) + ((tap & 1) ? p.tap_step : 0);
+      const int xx = (int)(2 * __ldg(p.x_id + e)) + ((tap & 2) ? p.tap_step : 0);
+      if (yy < 0 || xx < 0 || yy >= p.Hp || xx >= p.Wp) __trap();   // caller error (the reference raises an index assert)
+      if (mk != 0.f) v = ldg_nc_v4(pb + (size_t)(yy * p.Wp + xx) * E + c8 * 8);
+    }
+    *reinterpret_cast<uint4*>(A + a_offset(j >> 3, r, j & 7)) = v;
   }
 }
 
 // Index2Feat taps (E == 64: one tap = one 128-byte K chunk), masked
 __device__ __forceinline__ void fill_taps(uint8_t* A, const cp_chain_params& p, int b, int n0, int rows_valid) {
+  if (p.E != 64) {
+    fill_taps_any(A, p, b, n0, rows_valid);
+    return;
+  }
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tap = lane >> 3, chunk = lane & 7;
   const bf16* pb = reinterpret_cast<const bf16*>(p.patches) + (size_t)b * p.Hp * p.Wp * 64;
@@ -242,8 +300,9 @@ __device__ __forceinline__ void epilogue(uint32_t tmem_base, int pcols, int col0
   }
 }
 
-template <int PRO>
-__global__ void __launch_bounds__(NTHREADS, 2) chain_kernel(const __grid_constant__ KParams kp) {
+template <int PRO, bool WIDE>
+__global__ void __launch_bounds__(NTHREADS, Cfg<WIDE>::CTAS_PER_SM) chain_kernel(const __grid_constant__ KParams<WIDE> kp) {
+  constexpr int A_CHUNKS = Cfg<WIDE>::A_CHUNKS, TMEM_COLS = Cfg<WIDE>::TMEM_COLS;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   const cp_chain_params& p = kp.p;
   uint8_t* base = smem_raw;
@@ -304,7 +363,7 @@ __global__ void __launch_bounds__(NTHREADS, 2) chain_kernel(const __grid_constan
         const int pcols = min(TMEM_COLS, npad - col0);
         const int nblk = (pcols + 127) >> 7;
         for (int ph = 0; ph < nphase; ++ph) {
-          const int kc_count = (nphase == 2) ? (ph == 0 ? 4 : (p.Cg >> 6)) : (L.kin >> 6);
+          const int kc_count = (nphase == 2) ? (ph == 0 ? (p.E >> 4) : (p.Cg >> 6)) : (L.kin >> 6);
           if (ph == 1) {
             // second K phase of the pre-graph GEMM: A <- previous graph feature (all MMAs of phase 0 done)
             fill_rows(sm.A, reinterpret_cast<const bf16*>(p.graph_feat), p.ld_gf, p.Cg, row0, rows_valid);
@@ -384,7 +443,67 @@ __global__ void __launch_bounds__(NTHREADS, 2) chain_kernel(const __grid_constan
   if (warp == 1) tmem_dealloc(tmem_base, TMEM_COLS);
 }
 
-bool pow2_64_256(int c) { return c == 64 || c == 128 || c == 256; }
+// Weight-tile table of one launch; false if it would not fit MAXW entries.  Column passes of TMEM_COLS columns, 128-column
+// blocks inside a pass, K chunks inside a block: the order the MMA thread consumes them.
+bool build_wtiles(const cp_chain_params& p, int tmem_cols, int maxw, cp::WTile* wt, int* T_out) {
+  int T = 0;
+  for (int l = 0; l < p.num_layers; ++l) {
+    const cp_chain_layer& L = p.layers[l];
+    const int npad = (L.nout + 15) & ~15;
+    const bool two_phase = (p.prologue == CP_PRO_TAPS && l == 0);
+    const int npass = (npad + tmem_cols - 1) / tmem_cols;
+    for (int pass = 0; pass < npass; ++pass) {
+      const int col0 = pass * tmem_cols;
+      const int pcols = (npad - col0 < tmem_cols) ? (npad - col0) : tmem_cols;
+      const int nblk = (pcols + 127) / 128;
+      const int nphase = two_phase ? 2 : 1;
+      for (int ph = 0; ph < nphase; ++ph) {
+        const int kc_begin = (two_phase && ph == 1) ? p.E / 16 : 0;
+        const int kc_count = two_phase ? (ph == 0 ? p.E / 16 : p.Cg / 64) : L.kin / 64;
+        for (int nbi = 0; nbi < nblk; ++nbi) {
+          for (int kci = 0; kci < kc_count; ++kci) {
+            if (T >= maxw) return false;
+            wt[T++] = cp::packed_tile(L.w_packed, col0 / 128 + nbi, kc_begin + kci, L.kin, npad);
+          }
+        }
+      }
+    }
+  }
+  *T_out = T;
+  return true;
+}
+
+template <bool WIDE>
+int chain_launch(const cp_chain_params& p, cudaStream_t st) {
+  using C = Cfg<WIDE>;
+  KParams<WIDE> kp;
+  kp.p = p;
+  kp.tiles_per_roi = (p.N + TILE_M - 1) / TILE_M;
+  kp.num_node_tiles = kp.tiles_per_roi * p.B;
+  CP_REQUIRE(build_wtiles(p, C::TMEM_COLS, C::MAX_WTILES, kp.wt, &kp.T), CP_E_UNSUPPORTED, "cp_chain_fwd: weight tile table overflow");
+  const int num_sms = cp::num_sms();
+  const int grid = kp.num_node_tiles < C::CTAS_PER_SM * num_sms ? kp.num_node_tiles : C::CTAS_PER_SM * num_sms;
+  cudaError_t e = cudaSuccess;
+  switch (p.prologue) {
+    case CP_PRO_LOAD:
+      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_LOAD, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+      if (e == cudaSuccess) chain_kernel<CP_PRO_LOAD, WIDE><<<grid, NTHREADS, C::SMEM_BYTES, st>>>(kp);
+      break;
+    case CP_PRO_AGG:
+      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_AGG, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+      if (e == cudaSuccess) chain_kernel<CP_PRO_AGG, WIDE><<<grid, NTHREADS, C::SMEM_BYTES, st>>>(kp);
+      break;
+    default:
+      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_TAPS, WIDE>, cudaFuncAttributeMaxDynamicSharedMemorySize, C::SMEM_BYTES);
+      if (e == cudaSuccess) chain_kernel<CP_PRO_TAPS, WIDE><<<grid, NTHREADS, C::SMEM_BYTES, st>>>(kp);
+      break;
+  }
+  CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "cp_chain_fwd: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
+  CP_CHECK_LAUNCH("cp_chain_fwd");
+  return CP_OK;
+}
+
+bool width_ok(int c) { return c >= 64 && c <= 512 && (c % 64) == 0; }
 
 }  // namespace
 
@@ -398,25 +517,28 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
   CP_REQUIRE(p.B > 0 && p.N > 0, CP_E_INVALID, "cp_chain_fwd: bad B=%d N=%d", p.B, p.N);
   CP_REQUIRE(p.num_layers >= 1 && p.num_layers <= 3, CP_E_INVALID, "cp_chain_fwd: num_layers=%d outside [1,3]", p.num_layers);
   CP_REQUIRE(p.out && p.ld_out > 0, CP_E_INVALID, "cp_chain_fwd: no output buffer");
-  int kin0 = 0;
+  // widest K phase the prologue puts into the A tile; the narrow kernel holds 256 channels, the wide one 512
+  int kin0 = 0, kmax = 0;
   switch (p.prologue) {
     case CP_PRO_LOAD:
-      CP_REQUIRE(p.src && pow2_64_256(p.C) && p.ld_src >= p.C && (p.ld_src % 8) == 0, CP_E_UNSUPPORTED,
-                 "cp_chain_fwd(LOAD): need C in {64,128,256}, ld %% 8 == 0 (C=%d ld=%d)", p.C, p.ld_src);
-      kin0 = p.C;
+      CP_REQUIRE(p.src && width_ok(p.C) && p.ld_src >= p.C && (p.ld_src % 8) == 0, CP_E_UNSUPPORTED,
+                 "cp_chain_fwd(LOAD): need C a multiple of 64 in [64,512], ld %% 8 == 0 (C=%d ld=%d)", p.C, p.ld_src);
+      kin0 = kmax = p.C;
       break;
     case CP_PRO_AGG:
-      CP_REQUIRE(p.z && p.idx && pow2_64_256(p.Co) && p.ld_z >= 2 * p.Co && (p.ld_z % 8) == 0, CP_E_UNSUPPORTED,
-                 "cp_chain_fwd(AGG): need Co in {64,128,256} (Co=%d ld_z=%d)", p.Co, p.ld_z);
+      CP_REQUIRE(p.z && p.idx && width_ok(p.Co) && p.ld_z >= 2 * p.Co && (p.ld_z % 8) == 0, CP_E_UNSUPPORTED,
+                 "cp_chain_fwd(AGG): need Co a multiple of 64 in [64,512] (Co=%d ld_z=%d)", p.Co, p.ld_z);
       CP_REQUIRE(p.K >= 1 && p.K <= 64, CP_E_UNSUPPORTED, "cp_chain_fwd(AGG): K=%d outside [1,64]", p.K);
       CP_REQUIRE(!p.a_out || (p.ld_a_out >= p.Co && (p.ld_a_out % 8) == 0), CP_E_INVALID, "cp_chain_fwd(AGG): bad ld_a_out");
-      kin0 = p.Co;
+      kin0 = kmax = p.Co;
       break;
     case CP_PRO_TAPS:
       CP_REQUIRE(p.patches && p.x_id && p.y_id && p.graph_feat, CP_E_INVALID, "cp_chain_fwd(TAPS): null pointer");
-      CP_REQUIRE(p.E == 64 && pow2_64_256(p.Cg) && p.ld_gf >= p.Cg && (p.ld_gf % 8) == 0 && p.tap_step > 0, CP_E_UNSUPPORTED,
-                 "cp_chain_fwd(TAPS): need E == 64 and Cg in {64,128,256} (E=%d Cg=%d)", p.E, p.Cg);
+      CP_REQUIRE(p.E >= 16 && p.E <= 128 && (p.E % 16) == 0 && width_ok(p.Cg) && p.ld_gf >= p.Cg && (p.ld_gf % 8) == 0 &&
+                 p.tap_step > 0, CP_E_UNSUPPORTED,
+                 "cp_chain_fwd(TAPS): need E a multiple of 16 in [16,128] and Cg a multiple of 64 in [64,512] (E=%d Cg=%d)", p.E, p.Cg);
       kin0 = 4 * p.E + p.Cg;
+      kmax = 4 * p.E > p.Cg ? 4 * p.E : p.Cg;
       break;
     default:
       CP_REQUIRE(false, CP_E_INVALID, "cp_chain_fwd: bad prologue %d", p.prologue);
@@ -427,11 +549,9 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
     int rc = CP_OK;
     if (shapes_ok && (p.ld_out % 8) == 0 && cp::taps_chain_try(p, (cudaStream_t)s, &rc)) return rc;
   }
-  KParams kp;
-  kp.p = p;
-  kp.tiles_per_roi = (p.N + TILE_M - 1) / TILE_M;
-  kp.num_node_tiles = kp.tiles_per_roi * p.B;
-  int T = 0;
+  // narrow unless a width needs the wide kernel: K of a layer > 256, a chained output > 256 columns, or a last output wider
+  // than the narrow kernel takes (512 columns in column passes for bf16, 256 for f32)
+  bool wide = kmax > 256;
   int kin_expected = kin0;
   for (int l = 0; l < p.num_layers; ++l) {
     const cp_chain_layer& L = p.layers[l];
@@ -440,56 +560,26 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
     CP_REQUIRE(L.kin == kin_expected, CP_E_INVALID, "cp_chain_fwd: layer %d kin=%d but its input has %d channels", l, L.kin, kin_expected);
     CP_REQUIRE((reinterpret_cast<uintptr_t>(L.w_packed) & 15) == 0, CP_E_INVALID, "cp_chain_fwd: layer %d weights not 16-byte aligned", l);
     const int npad = (L.nout + 15) & ~15;
-    const int max_n = (last && p.out_mode == CP_OUT_BF16) ? 512 : 256;
+    const int max_n = last ? (p.out_mode == CP_OUT_BF16 ? 1024 : 512) : 512;
     CP_REQUIRE(npad <= max_n, CP_E_UNSUPPORTED, "cp_chain_fwd: layer %d nout=%d too wide", l, L.nout);
     CP_REQUIRE(last || (npad % 64) == 0, CP_E_UNSUPPORTED, "cp_chain_fwd: chained layer %d needs nout %% 64 == 0", l);
     const bool two_phase = (p.prologue == CP_PRO_TAPS && l == 0);
-    CP_REQUIRE(two_phase || L.kin <= 256, CP_E_UNSUPPORTED, "cp_chain_fwd: layer %d kin=%d > 256", l, L.kin);
-    const int npass = (npad + TMEM_COLS - 1) / TMEM_COLS;
-    for (int pass = 0; pass < npass; ++pass) {
-      const int col0 = pass * TMEM_COLS;
-      const int pcols = (npad - col0 < TMEM_COLS) ? (npad - col0) : TMEM_COLS;
-      const int nblk = (pcols + 127) / 128;
-      const int nphase = two_phase ? 2 : 1;
-      for (int ph = 0; ph < nphase; ++ph) {
-        const int kc_begin = (two_phase && ph == 1) ? 4 : 0;
-        const int kc_count = two_phase ? (ph == 0 ? 4 : p.Cg / 64) : L.kin / 64;
-        for (int nbi = 0; nbi < nblk; ++nbi) {
-          for (int kci = 0; kci < kc_count; ++kci) {
-            CP_REQUIRE(T < MAX_WTILES, CP_E_UNSUPPORTED, "cp_chain_fwd: weight tile table overflow");
-            kp.wt[T++] = cp::packed_tile(L.w_packed, col0 / 128 + nbi, kc_begin + kci, L.kin, npad);
-          }
-        }
-      }
-    }
+    CP_REQUIRE(two_phase || L.kin <= 512, CP_E_UNSUPPORTED, "cp_chain_fwd: layer %d kin=%d > 512", l, L.kin);
+    // the second K phase of TAPS layer 0 overwrites the taps in the A tile, so that layer must run in one column pass
+    CP_REQUIRE(!two_phase || npad <= 512, CP_E_UNSUPPORTED, "cp_chain_fwd(TAPS): layer 0 nout=%d > 512 (one column pass)", L.nout);
+    if (!two_phase && L.kin > 256) wide = true;
+    if (npad > (last && !two_phase ? (p.out_mode == CP_OUT_BF16 ? 512 : 256) : 256)) wide = true;
     kin_expected = npad;
     if (!last) CP_REQUIRE(npad == L.nout, CP_E_UNSUPPORTED, "cp_chain_fwd: chained layer %d nout must be a multiple of 16", l);
   }
-  kp.T = T;
   if (p.out_mode == CP_OUT_BF16)
     CP_REQUIRE((p.ld_out % 8) == 0, CP_E_INVALID, "cp_chain_fwd: bf16 output needs ld_out %% 8 == 0");
   else
     CP_REQUIRE(p.out_mode == CP_OUT_F32 && p.n_valid >= 1 && p.n_valid <= p.ld_out, CP_E_INVALID, "cp_chain_fwd: bad f32 output spec");
-
-  const int num_sms = cp::num_sms();
-  int grid = kp.num_node_tiles < 2 * num_sms ? kp.num_node_tiles : 2 * num_sms;
-  cudaStream_t st = (cudaStream_t)s;
-  cudaError_t e = cudaSuccess;
-  switch (p.prologue) {
-    case CP_PRO_LOAD:
-      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_LOAD>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-      if (e == cudaSuccess) chain_kernel<CP_PRO_LOAD><<<grid, NTHREADS, SMEM_BYTES, st>>>(kp);
-      break;
-    case CP_PRO_AGG:
-      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_AGG>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-      if (e == cudaSuccess) chain_kernel<CP_PRO_AGG><<<grid, NTHREADS, SMEM_BYTES, st>>>(kp);
-      break;
-    default:
-      e = cudaFuncSetAttribute(chain_kernel<CP_PRO_TAPS>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
-      if (e == cudaSuccess) chain_kernel<CP_PRO_TAPS><<<grid, NTHREADS, SMEM_BYTES, st>>>(kp);
-      break;
+  if (!wide) {
+    cp::WTile probe[Cfg<false>::MAX_WTILES];
+    int T = 0;
+    wide = !build_wtiles(p, Cfg<false>::TMEM_COLS, Cfg<false>::MAX_WTILES, probe, &T);
   }
-  CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "cp_chain_fwd: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
-  CP_CHECK_LAUNCH("cp_chain_fwd");
-  return CP_OK;
+  return wide ? chain_launch<true>(p, (cudaStream_t)s) : chain_launch<false>(p, (cudaStream_t)s);
 }

@@ -42,12 +42,78 @@ def get_compute_dtype():
 
 
 # --------------------------------------------------------------------------------------------------
+# bf16 widths.  The chain kernel takes widths that are multiples of 64 up to 512 (the patch-embedding width E of a refine
+# stage a multiple of 16 up to 128).  Any other width runs padded: each node-major feature is stored with its channels
+# rounded up to that granularity, the extra channels being exact zeros, and every weight gets zero rows for padded outputs,
+# zero columns for padded inputs and zero bias.  A padded channel of a Linear is then 0 + 0 = 0, LeakyReLU(0) = 0, and it
+# meets only zero weights downstream, so it adds exactly 0 to every real channel's sum.  An EdgeConv pads its convolution
+# and BatchNorm before the fold, BatchNorm with gamma = beta = mean = 0 and var = 1: the folded scale and shift of a padded
+# channel are 0, its [P|Q] columns are 0, and the aggregation lrelu(max_k P + Q) of zeros is 0.  Results handed back to
+# the caller are sliced to the true width.
+# --------------------------------------------------------------------------------------------------
+MAX_BF16_WIDTH = 512
+MAX_BF16_EMBED = 128
+
+
+def pad64(c: int) -> int:
+    return (c + 63) // 64 * 64
+
+
+def pad16(c: int) -> int:
+    return (c + 15) // 16 * 16
+
+
+def _pad_segments(t, dim, segs, value=0.0):
+    """Zero-pad ``t`` along ``dim`` segment by segment: ``segs`` = ((true, padded), ...) laid end to end."""
+    if all(a == b for a, b in segs):
+        return t
+    parts, o = [], 0
+    for a, b in segs:
+        x = t.narrow(dim, o, a)
+        if b > a:
+            shape = list(x.shape)
+            shape[dim] = b - a
+            x = torch.cat([x, torch.full(shape, value, dtype=t.dtype, device=t.device)], dim)
+        parts.append(x)
+        o += a
+    return torch.cat(parts, dim)
+
+
+def pad_linear_weight(weight, bias, rows, cols):
+    """(nout, kin) weight and (nout) bias zero-padded: ``rows`` / ``cols`` = ((true, padded), ...) segments."""
+    w = weight.detach().reshape(weight.shape[0], -1).float()
+    w = _pad_segments(_pad_segments(w, 0, rows), 1, cols)
+    b = None if bias is None else _pad_segments(bias.detach().float(), 0, rows)
+    return w, b
+
+
+def pad_edgeconv(w, gamma, beta, mean, var):
+    """EdgeConv convolution (C', 2C[, 1, 1]) and BatchNorm parameters padded before the fold: C -> pad64(C) on both halves of
+    the [x_j - x_i | x_i] input, C' -> pad64(C') with gamma = beta = mean = 0 and var = 1 (folded scale and shift 0)."""
+    co, c = w.shape[0], w.shape[1] // 2
+    rows, half = ((co, pad64(co)),), (c, pad64(c))
+    w = _pad_segments(_pad_segments(w.reshape(co, 2 * c).float(), 0, rows), 1, (half, half))
+    gamma, beta, mean = (_pad_segments(t.float(), 0, rows) for t in (gamma, beta, mean))
+    return w, gamma, beta, mean, _pad_segments(var.float(), 0, rows, 1.0)
+
+
+def _pad_to(x, width):
+    """Node-major x (B,N,c) with its channels zero-padded to ``width`` (no copy when it already has them)."""
+    return x if x.shape[-1] == width else F.pad(x, (0, width - x.shape[-1]))
+
+
+def check_bf16_width(what: str, c: int, limit: int = MAX_BF16_WIDTH) -> None:
+    if c > limit:
+        raise RuntimeError(f"bf16 mode runs {what} up to {limit} channels (got {c}); use float32 mode for wider heads")
+
+
+# --------------------------------------------------------------------------------------------------
 # prepared weights (derived from the module parameters; never stored in the state_dict)
 # --------------------------------------------------------------------------------------------------
 class PreparedLinear:
     """bf16 mode: ``packed`` = bf16 tile image for the chain / EdgeConv kernels.  float32 mode: ``split`` = the
     (hi, lo) bf16 tile images of the split-precision tensor-core GEMM (cp_gemm_x3); layers whose K is not a multiple
-    of 64 (none of the shipped shapes) keep the SIMT GEMM."""
+    of 64 keep the SIMT GEMM.  ``nout`` / ``kin`` are the widths of the (possibly padded) weight."""
 
     def __init__(self, weight, bias, want_packed):
         self.w = weight.detach().reshape(weight.shape[0], -1).contiguous().float()
@@ -68,10 +134,13 @@ def linear32(x, prep: "PreparedLinear", act=False, slope=0.0, a2=None):
 class PreparedEdgeConv(PreparedLinear):
     """StaticGraph_module weights folded to the factored form [P|Q] (see cp_fold_edgeconv)."""
 
-    def __init__(self, sg_module, want_packed):
+    def __init__(self, sg_module, want_packed, pad=False):
         conv, bn, act = sg_module.conv[0], sg_module.conv[1], sg_module.conv[2]
-        wf, bf = ops.fold_edgeconv(conv.weight.detach(), bn.weight.detach(), bn.bias.detach(),
-                                   bn.running_mean.detach(), bn.running_var.detach(), bn.eps)
+        w, gamma, beta = conv.weight.detach(), bn.weight.detach(), bn.bias.detach()
+        mean, var = bn.running_mean.detach(), bn.running_var.detach()
+        if pad:
+            w, gamma, beta, mean, var = pad_edgeconv(w, gamma, beta, mean, var)
+        wf, bf = ops.fold_edgeconv(w, gamma, beta, mean, var, bn.eps)
         super().__init__(wf, bf, want_packed)
         self.C, self.Co = wf.shape[1], wf.shape[0] // 2
         self.slope = float(act.negative_slope)
@@ -116,13 +185,29 @@ _PREP = PrepCache()
 
 
 def prepared_edgeconv(sg_module, dtype) -> PreparedEdgeConv:
+    """bf16 mode: input and output widths padded to multiples of 64 (unchanged when they are)."""
     want = dtype == torch.bfloat16
-    return _PREP.get(sg_module, ("ec", want), lambda: PreparedEdgeConv(sg_module, want))
+    co, c2 = sg_module.conv[0].weight.shape[:2]
+    pad = want and (co % 64 != 0 or (c2 // 2) % 64 != 0)
+    return _PREP.get(sg_module, ("ec", want, pad), lambda: PreparedEdgeConv(sg_module, want, pad))
 
 
-def prepared_linear(lin: nn.Module, dtype) -> PreparedLinear:
+def prepared_linear(lin: nn.Module, dtype, rows=None, cols=None) -> PreparedLinear:
+    """``rows`` / ``cols``: ((true, padded), ...) segments the bf16 weight is zero-padded to (see pad_linear_weight)."""
     want = dtype == torch.bfloat16
-    return _PREP.get(lin, ("lin", want), lambda: PreparedLinear(lin.weight, lin.bias, want))
+    rows = ((lin.weight.shape[0],) * 2,) if rows is None else tuple(rows)
+    cols = ((lin.weight.shape[1],) * 2,) if cols is None else tuple(cols)
+    if all(a == b for a, b in rows + cols):
+        return _PREP.get(lin, ("lin", want), lambda: PreparedLinear(lin.weight, lin.bias, want))
+    return _PREP.get(lin, ("lin", want, rows, cols), lambda: PreparedLinear(*pad_linear_weight(lin.weight, lin.bias, rows, cols), want))
+
+
+def _padded_linear(lin: nn.Module, kin_stored: int, last: bool = False) -> PreparedLinear:
+    """bf16 Linear reading a stored input of ``kin_stored`` (>= in_features) channels; its output padded to a multiple of
+    64 unless it is the ``last`` layer (an f32 result with n_valid columns)."""
+    nout, kin = lin.weight.shape
+    check_bf16_width("a Linear layer", max(kin, nout))
+    return prepared_linear(lin, torch.bfloat16, rows=((nout, nout if last else pad64(nout)),), cols=((kin, kin_stored),))
 
 
 class GraphTable:
@@ -222,17 +307,14 @@ def _require_eval(module):
                            "call .eval() (training-mode BN over B*N*K is out of scope)")
 
 
-def _chain_ok(C):
-    return C in (64, 128, 256)
-
-
 # --------------------------------------------------------------------------------------------------
 # EdgeConv (K2).  Every node-major tensor below is in PLAN order (GraphCtx.to_plan / to_keypoints convert).
 # --------------------------------------------------------------------------------------------------
 def _agg_gemm(z, ctx: GraphCtx, agg_slope, layer, out, out_mode, n_valid=0, a_out=None):
     """A = EdgeConv aggregation of the [P|Q] table z; out = layer(A).  Staged warp-specialised kernel when the
-    graph plan fits it, else the unstaged chain kernel with direct global gathers."""
-    if ctx.plan.staged:
+    graph plan and the widths fit it (C' in {64,128,256}, out <= 512 columns), else the unstaged chain kernel with direct
+    global gathers."""
+    if ctx.plan.staged and z.shape[-1] // 2 in (64, 128, 256) and layer.nout <= 512:
         return ops.edgeconv_fwd(z=z, plan=ctx.plan, graph_sel=ctx.sel, agg_slope=agg_slope, layer=layer, out=out,
                                 out_mode=out_mode, n_valid=n_valid, a_out=a_out)
     return ops.chain_fwd(prologue=ops.PRO_AGG, B=z.shape[0], N=z.shape[1], z=z, idx32=ctx.plan.idx_p, graph_sel=ctx.sel,
@@ -242,18 +324,20 @@ def _agg_gemm(z, ctx: GraphCtx, agg_slope, layer, out, out_mode, n_valid=0, a_ou
 def edgeconv_node_major(sg_module, x_nm, ctx: GraphCtx, dtype):
     """x_nm (B,N,C) of ``dtype`` -> (B,N,Co).  StaticGraph_module.forward (pipeline.py:55-59), one layer on its own."""
     _require_eval(sg_module)
+    if dtype == torch.bfloat16:
+        co, c2 = sg_module.conv[0].weight.shape[:2]
+        check_bf16_width("an EdgeConv", max(co, c2 // 2))
     prep = prepared_edgeconv(sg_module, dtype)
-    B, N, C = x_nm.shape
+    B, N, _ = x_nm.shape
     if dtype == torch.float32:
         z = linear32(x_nm, prep)
         if ctx.plan.struct is not None and ctx.plan.max_unique <= ops.PLAN_UMAX and prep.Co % 32 == 0:
             return ops.edge_aggregate_staged(z, ctx.plan, ctx.sel, prep.slope)     # rows staged in shared memory per tile
         return ops.edge_aggregate(z, ctx.plan.idx_p, ctx.sel, prep.slope)
-    if not (_chain_ok(C) and _chain_ok(prep.Co)):
-        raise RuntimeError(f"bf16 EdgeConv supports C, C' in {{64,128,256}} (got {C}->{prep.Co}); use float32 mode")
+    # bf16: widths padded to multiples of 64; the result keeps the padded channels (zeros)
     z = torch.empty((B, N, 2 * prep.Co), dtype=torch.bfloat16, device=x_nm.device)
-    ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x_nm,
-                  layers=[ops.chain_layer(prep.packed, prep.b, C, 2 * prep.Co, False, 0.0)], out=z, out_mode=ops.OUT_BF16)
+    ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=_pad_to(x_nm, prep.C),
+                  layers=[ops.chain_layer(prep.packed, prep.b, prep.C, 2 * prep.Co, False, 0.0)], out=z, out_mode=ops.OUT_BF16)
     return ops.edge_aggregate(z, ctx.plan.idx_p, ctx.sel, prep.slope)
 
 
@@ -691,10 +775,24 @@ def patches_nhwc(patch_generator, img_feat, dtype):
 # --------------------------------------------------------------------------------------------------
 # refine stage (Refine_moduleGNN.forward, pipeline.py:262-298)
 # --------------------------------------------------------------------------------------------------
+def check_bf16_refine_widths(ref):
+    """Raise for a refine stage whose widths the bf16 kernels cannot run, even padded (before any launch)."""
+    d0 = ref.pre_graph_module[0].weight.shape[0]
+    E = ref.local_feat_ext_block.patch_generator.out_channels
+    if d0 % 4 != 0 or 4 * E != d0:
+        raise RuntimeError(f"bf16 mode needs query_dims[0] divisible by 4 (the patch embedding is query_dims[0] // 4); got "
+                           f"query_dims[0] = {d0}; use float32 mode")
+    check_bf16_width("query_dims[0]", d0)
+    check_bf16_width("the incoming graph feature", ref.pre_graph_module[0].weight.shape[1] - 4 * E)
+    for i in (0, 2, 4):
+        check_bf16_width("the query MLP", max(ref.query_block.mlps[i].weight.shape))
+
+
 def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype, decode=None):
     """One refine stage on plan-order node tensors: gfeat_nm (B,N,Cg) of ``dtype``, roi_mask (B,N) f32 {0,1}, ids (B,N)
     int64, ctx = graph_ctx of the stage's graph (None when it has no graph modules).
-    -> logits (B,N,>=2) f32 [x_new, y_new], graph feature (B,N,C) of ``dtype``.
+    -> logits (B,N,>=2) f32 [x_new, y_new], graph feature (B,N,C) of ``dtype`` (bf16: C = pad64(query_dims[0]), the padded
+    channels zero; gfeat_nm may come padded or at its true width).
     ``decode`` = dict(plane, Ltot, x_bits, y_bits, perm, sel[, x_id_kp, y_id_kp]): in bf16 mode the stage's tail (query layers 2
     and 3 + the decode of pipeline.py:375-381, ids updated IN PLACE) runs as one launch (cp_query_decode_fwd) and the returned
     logits are None."""
@@ -702,16 +800,19 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
     B, N, Cg = gfeat_nm.shape
     dev = gfeat_nm.device
     k = ref.local_feat_ext_block.kernel_size
+    if dtype == torch.bfloat16:
+        check_bf16_refine_widths(ref)
     patches = patches_nhwc(ref.local_feat_ext_block.patch_generator, img_feat, dtype)
-    pg0 = prepared_linear(ref.pre_graph_module[0], dtype)
-    pg1 = prepared_linear(ref.pre_graph_module[2], dtype)
     slope = float(ref.pre_graph_module[1].negative_slope)
     blocks = list(ref.pre_query_block)
-    q = [prepared_linear(ref.query_block.mlps[i], dtype) for i in (0, 2, 4)]
+    qmods = [ref.query_block.mlps[i] for i in (0, 2, 4)]
     qslope = float(ref.query_block.mlps[1].negative_slope)
     x_id = x_id.contiguous()
     y_id = y_id.contiguous()
     if dtype == torch.float32:
+        pg0 = prepared_linear(ref.pre_graph_module[0], dtype)
+        pg1 = prepared_linear(ref.pre_graph_module[2], dtype)
+        q = [prepared_linear(m, dtype) for m in qmods]
         taps = ops.sample_taps(patches, x_id, y_id, roi_mask, k)
         h = linear32(taps, pg0, True, slope, a2=gfeat_nm)
         h = linear32(h, pg1, True, slope)
@@ -721,14 +822,22 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
         t = linear32(t, q[1], True, qslope)
         logits = linear32(t, q[2])
         return logits, h
-    # ---- bf16 fused kernels ----
+    # ---- bf16 fused kernels, widths padded (see the width notes at the top) ----
     E = patches.shape[-1]
-    if not (E == 64 and _chain_ok(Cg) and pg0.nout == 256 and pg1.nout == 256 and q[0].kin == 256):
-        raise RuntimeError("bf16 refine stage supports the shipped dims (num_filters=256, query_dims=(256,256,64)); "
-                           "use float32 mode for other shapes")
+    d0 = ref.pre_graph_module[0].weight.shape[0]
+    cg = ref.pre_graph_module[0].weight.shape[1] - 4 * E          # true width of the incoming graph feature
+    Ep, cgp = pad16(E), pad64(cg)
+    if Ep != E:
+        patches = F.pad(patches, (0, Ep - E))
+    gfeat_nm = _pad_to(gfeat_nm, cgp)
+    pg0 = prepared_linear(ref.pre_graph_module[0], dtype, rows=((d0, pad64(d0)),), cols=((E, Ep),) * 4 + ((cg, cgp),))
+    pg1 = _padded_linear(ref.pre_graph_module[2], pad64(d0))
     preps = [prepared_edgeconv(b, dtype) for b in blocks]
     for b in blocks:
         _require_eval(b)
+    q0 = _padded_linear(qmods[0], pad64(d0))
+    q1 = _padded_linear(qmods[1], q0.nout)
+    q = [q0, q1, _padded_linear(qmods[2], q1.nout, last=True)]
     pg_layers = [ops.chain_layer(pg0.packed, pg0.b, pg0.kin, pg0.nout, True, slope),
                  ops.chain_layer(pg1.packed, pg1.b, pg1.kin, pg1.nout, True, slope)]
     q_layers = [ops.chain_layer(q[0].packed, q[0].b, q[0].kin, q[0].nout, True, qslope),
@@ -739,7 +848,7 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
     taps_args = dict(prologue=ops.PRO_TAPS, patches=patches, tap_step=k, x_id=x_id, y_id=y_id, mask=roi_mask,
                      graph_feat=gfeat_nm)
     if not blocks:
-        feat = torch.empty((B, N, 256), dtype=torch.bfloat16, device=dev)
+        feat = torch.empty((B, N, pg1.nout), dtype=torch.bfloat16, device=dev)
         ops.chain_fwd(**common, **taps_args, layers=pg_layers, out=feat, out_mode=ops.OUT_BF16)
         ops.chain_fwd(**common, prologue=ops.PRO_LOAD, src=feat, layers=q_layers, out=logits, out_mode=ops.OUT_F32,
                       n_valid=q[2].nout)
@@ -751,7 +860,7 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
                   out=z, out_mode=ops.OUT_BF16)
     # EdgeConv j aggregation fused with EdgeConv j+1's [P|Q] GEMM
     for j in range(1, len(blocks)):
-        z2 = torch.empty_like(z)
+        z2 = torch.empty((B, N, 2 * preps[j].Co), dtype=torch.bfloat16, device=dev)
         _agg_gemm(z, ctx, preps[j - 1].slope,
                   ops.chain_layer(preps[j].packed, preps[j].b, preps[j].C, 2 * preps[j].Co, False, 0.0), z2, ops.OUT_BF16)
         z = z2
@@ -774,7 +883,8 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
 # --------------------------------------------------------------------------------------------------
 def mlp_node_major(mods, x_nm, dtype, out_f32=False):
     """nn.Sequential of Linear / LeakyReLU (get_MLP_leakyReLU_layers) on node-major x (B,N,C) of ``dtype``.
-    bf16: chain kernel, up to three layers per launch; ``out_f32`` -> (B,N,>=nout padded to 16) f32 logits."""
+    bf16: chain kernel, up to three layers per launch; ``out_f32`` -> (B,N,>=nout padded to 16) f32 logits, else a bf16
+    result whose width is padded to a multiple of 64 (zeros beyond nout); x_nm may come padded the same way."""
     mods = list(mods)
     layers = []
     i = 0
@@ -789,14 +899,15 @@ def mlp_node_major(mods, x_nm, dtype, out_f32=False):
             pl = prepared_linear(lin, dtype)
             x = linear32(x, pl, act, slope)
         return x
-    x = x_nm
+    x = _pad_to(x_nm, pad64(layers[0][0].weight.shape[1]))
     for j0 in range(0, len(layers), 3):
         grp = layers[j0:j0 + 3]
-        pls = [prepared_linear(lin, dtype) for lin, _, _ in grp]
-        if not all(_chain_ok(pl.kin) for pl in pls):
-            raise RuntimeError("bf16 MLP supports layer inputs in {64,128,256}; use float32 mode for other shapes")
-        cl = [ops.chain_layer(pl.packed, pl.b, pl.kin, pl.nout, act, slope) for pl, (_, act, slope) in zip(pls, grp)]
         last = j0 + 3 >= len(layers)
+        pls, kin = [], x.shape[-1]
+        for jj, (lin, _, _) in enumerate(grp):
+            pls.append(_padded_linear(lin, kin, last=last and out_f32 and jj == len(grp) - 1))
+            kin = pls[-1].nout
+        cl = [ops.chain_layer(pl.packed, pl.b, pl.kin, pl.nout, act, slope) for pl, (_, act, slope) in zip(pls, grp)]
         if last and out_f32:
             out = torch.empty((B, N, (pls[-1].nout + 15) // 16 * 16), dtype=torch.float32, device=x.device)
             ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x, layers=cl, out=out, out_mode=ops.OUT_F32, n_valid=pls[-1].nout)

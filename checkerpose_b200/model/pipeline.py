@@ -89,6 +89,7 @@ class StaticGraph_module(head.DeviceScopedModule):
         dtype = head.get_compute_dtype()
         ctx = head.graph_ctx(self._knn, obj_ids, x.shape[0], x.device)
         y = head.edgeconv_node_major(self, ctx.to_plan(ops.to_node_major(x, dtype)), ctx, dtype)
+        y = y[:, :, :self.conv[0].weight.shape[0]]     # bf16 mode keeps the width padded to a multiple of 64
         return _to_io(ctx.to_keypoints(y), x.dtype)
 
     def forward(self, x, batch_indices=None):
@@ -234,6 +235,7 @@ class Refine_moduleGNN(head.DeviceScopedModule):
         logits, feat = head.refine_node_major(self, img_feat, gfeat, mask.view(B, N), x_id.view(B, N), y_id.view(B, N),
                                               ctx, dtype)
         logits = logits[:, :, :2].contiguous()
+        feat = feat[:, :, :self.query_dims[0]]          # bf16 mode keeps the width padded to a multiple of 64
         if ctx is not None:
             logits, feat = ctx.to_keypoints(logits), ctx.to_keypoints(feat)
         return logits.permute(0, 2, 1), _to_io(feat, graph_feat.dtype)

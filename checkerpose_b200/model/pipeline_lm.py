@@ -63,7 +63,7 @@ class Refine_moduleGNN_ABwoProg(head.DeviceScopedModule):
         gfeat = ops.to_node_major(graph_feat, dtype)
         if ctx is not None:
             gfeat = ctx.to_plan(gfeat)
-        feat = head.abwoprog_refine_node_major(self, gfeat, ctx, dtype)
+        feat = head.abwoprog_refine_node_major(self, gfeat, ctx, dtype)[:, :, :self.query_dims[0]]   # bf16: width padded
         if ctx is not None:
             feat = ctx.to_keypoints(feat)
         return _to_io(feat, graph_feat.dtype)

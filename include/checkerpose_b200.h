@@ -194,6 +194,8 @@ int cp_edge_aggregate(const void* z, int dtype, const int32_t* idx, const int32_
  *                          pipeline.py:147-164, 278-283)
  *   output   CP_OUT_BF16 : out (B*N, ld_out) bf16, all Nout columns (EdgeConv [P|Q] table)
  *            CP_OUT_F32  : out (B*N, ld_out) f32, first n_valid columns (logits)
+ * C / Co are multiples of 64 up to 512.  Shapes whose K and chained outputs fit 256 channels run two CTAs per SM; wider
+ * ones one CTA per SM with a 128 KB operand tile and all 512 TMEM columns (chain_tcgen05.cu).
  * See DESIGN.md for the tile/pipeline description. */
 enum { CP_PRO_LOAD = 0, CP_PRO_AGG = 1, CP_PRO_TAPS = 2 };
 enum { CP_OUT_BF16 = 0, CP_OUT_F32 = 1 };
@@ -201,8 +203,9 @@ enum { CP_OUT_BF16 = 0, CP_OUT_F32 = 1 };
 typedef struct {
   const void* w_packed; /* cp_pack_weight image of the (nout, kin) weight */
   const float* bias;    /* (nout) or NULL */
-  int kin;              /* multiple of 64, <= 512 for layer 0 of TAPS, else <= 256 */
-  int nout;             /* <= 512 for the last layer with CP_OUT_BF16, else <= 256 */
+  int kin;              /* multiple of 64, <= 512 (layer 0 of TAPS: 4E + Cg, each part <= 512) */
+  int nout;             /* chained: multiple of 64, <= 512; last: <= 1024 with CP_OUT_BF16, else <= 512;
+                         * layer 0 of TAPS (two K phases, one column pass): <= 512 */
   int act;              /* 0 none, 1 LeakyReLU */
   float slope;
 } cp_chain_layer;
@@ -214,7 +217,8 @@ typedef struct {
   const void* src; int ld_src; int C;
   /* AGG */
   const void* z; int ld_z; int Co; const int32_t* idx; const int32_t* graph_sel; int K; float agg_slope;
-  /* TAPS: patches (B, Hp, Wp, E) bf16 NHWC, ids (B,N) int64, mask (B,N) f32 {0,1}, graph_feat (B,N,Cg) bf16 */
+  /* TAPS: patches (B, Hp, Wp, E) bf16 NHWC (E a multiple of 16, <= 128), ids (B,N) int64, mask (B,N) f32 {0,1},
+   * graph_feat (B,N,Cg) bf16 (Cg a multiple of 64, <= 512); A = [tap0 | tap1 | tap2 | tap3 | graph_feat], tap t at t*E */
   const void* patches; int Hp, Wp, E, tap_step; const int64_t* x_id; const int64_t* y_id; const float* mask;
   const void* graph_feat; int ld_gf; int Cg;
   /* optional copy of the prologue's A tile (first C / Co channels) to global, bf16 (B*N, ld_a_out) */
