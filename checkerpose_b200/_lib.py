@@ -14,7 +14,8 @@ c_i32, c_i64, c_f32, c_vp, c_sz = C.c_int, C.c_int64, C.c_float, C.c_void_p, C.c
 
 
 class ChainLayer(C.Structure):
-    _fields_ = [("w_packed", c_vp), ("bias", c_vp), ("kin", c_i32), ("nout", c_i32), ("act", c_i32), ("slope", c_f32)]
+    _fields_ = [("w_packed", c_vp), ("bias", c_vp), ("kin", c_i32), ("nout", c_i32), ("act", c_i32), ("slope", c_f32),
+                ("w_stride", c_i64), ("b_stride", c_i32)]
 
 
 class ChainParams(C.Structure):
@@ -103,6 +104,7 @@ class QueryDecodeParams(C.Structure):
         ("plane", c_i32), ("Ltot", c_i32),
         ("x_bits", c_vp), ("y_bits", c_vp), ("x_id", c_vp), ("y_id", c_vp), ("x_id_kp", c_vp), ("y_id_kp", c_vp),
         ("perm", c_vp), ("graph_sel", c_vp),
+        ("w1_stride", c_i64), ("b1_stride", c_i32), ("w2_stride", c_i32), ("b2_stride", c_i32),
     ]
 
 

@@ -68,6 +68,7 @@ struct KParams {
   int tiles_per_roi;
   int num_node_tiles;
   int T;  // weight tiles per node tile
+  int wsel;  // a layer has object-indexed weights (non-zero strides): p.graph_sel selects them per RoI
   cp::WTile wt[Cfg<WIDE>::MAX_WTILES];
 };
 
@@ -343,6 +344,7 @@ __global__ void __launch_bounds__(NTHREADS, Cfg<WIDE>::CTAS_PER_SM) chain_kernel
     const int n0 = (tile - b * kp.tiles_per_roi) * TILE_M;
     const int rows_valid = min(TILE_M, p.N - n0);
     const int64_t row0 = (int64_t)b * p.N + n0;
+    const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, b);
 
     // ---------------- prologue -> A ----------------
     if (PRO == CP_PRO_LOAD) fill_rows(sm.A, reinterpret_cast<const bf16*>(p.src), p.ld_src, p.C, row0, rows_valid);
@@ -409,9 +411,14 @@ __global__ void __launch_bounds__(NTHREADS, Cfg<WIDE>::CTAS_PER_SM) chain_kernel
                 const long long use = pc / STAGES;
                 if (use > 0) mbar_wait(&sm.empty[s], (uint32_t)((use - 1) & 1));
                 const cp::WTile& wt = kp.wt[(int)(pc % kp.T)];
+                const uint8_t* wsrc = wt.ptr;
+                if (kp.wsel) {   // the producer runs ahead into the next node tiles: the object of the tile this weight tile serves
+                  const int wtile = (int)blockIdx.x + (int)(pc / kp.T) * (int)gridDim.x;
+                  wsrc += (int64_t)cp::weight_obj(p.graph_sel, true, wtile / kp.tiles_per_roi) * p.layers[wt.layer].w_stride;
+                }
                 if (elect_one()) {
                   mbar_arrive_expect_tx(&sm.full[s], wt.bytes);
-                  bulk_g2s(sm.Bst + s * B_STAGE_BYTES, wt.ptr, wt.bytes, &sm.full[s]);
+                  bulk_g2s(sm.Bst + s * B_STAGE_BYTES, wsrc, wt.bytes, &sm.full[s]);
                 }
                 __syncwarp();
                 ++pc;
@@ -430,7 +437,8 @@ __global__ void __launch_bounds__(NTHREADS, Cfg<WIDE>::CTAS_PER_SM) chain_kernel
         int mode;
         if (!last) mode = EPI_SMEM;
         else mode = (p.out_mode == CP_OUT_BF16) ? EPI_BF16 : EPI_F32;
-        epilogue(tmem_base, pcols, col0, L.bias, L.nout, L.act, L.slope, mode, sm.A, p.out, p.ld_out, p.n_valid, row0, rows_valid);
+        const float* bias = L.bias ? L.bias + (int64_t)obj * L.b_stride : nullptr;
+        epilogue(tmem_base, pcols, col0, bias, L.nout, L.act, L.slope, mode, sm.A, p.out, p.ld_out, p.n_valid, row0, rows_valid);
         tc_fence_before_sync();
         if (mode == EPI_SMEM) fence_proxy_async_smem();
         __syncthreads();
@@ -463,7 +471,7 @@ bool build_wtiles(const cp_chain_params& p, int tmem_cols, int maxw, cp::WTile* 
         for (int nbi = 0; nbi < nblk; ++nbi) {
           for (int kci = 0; kci < kc_count; ++kci) {
             if (T >= maxw) return false;
-            wt[T++] = cp::packed_tile(L.w_packed, col0 / 128 + nbi, kc_begin + kci, L.kin, npad);
+            wt[T++] = cp::packed_tile(L.w_packed, col0 / 128 + nbi, kc_begin + kci, L.kin, npad, l);
           }
         }
       }
@@ -480,6 +488,8 @@ int chain_launch(const cp_chain_params& p, cudaStream_t st) {
   kp.p = p;
   kp.tiles_per_roi = (p.N + TILE_M - 1) / TILE_M;
   kp.num_node_tiles = kp.tiles_per_roi * p.B;
+  kp.wsel = 0;
+  for (int l = 0; l < p.num_layers; ++l) kp.wsel |= (p.layers[l].w_stride != 0 || p.layers[l].b_stride != 0);
   CP_REQUIRE(build_wtiles(p, C::TMEM_COLS, C::MAX_WTILES, kp.wt, &kp.T), CP_E_UNSUPPORTED, "cp_chain_fwd: weight tile table overflow");
   const int num_sms = cp::num_sms();
   const int grid = kp.num_node_tiles < C::CTAS_PER_SM * num_sms ? kp.num_node_tiles : C::CTAS_PER_SM * num_sms;
@@ -543,6 +553,9 @@ extern "C" int cp_chain_fwd(const cp_chain_params* pp, cp_stream_t s) {
     default:
       CP_REQUIRE(false, CP_E_INVALID, "cp_chain_fwd: bad prologue %d", p.prologue);
   }
+  for (int l = 0; l < p.num_layers; ++l)
+    CP_REQUIRE(p.layers[l].w_stride >= 0 && (p.layers[l].w_stride % 16) == 0 && p.layers[l].b_stride >= 0, CP_E_INVALID,
+               "cp_chain_fwd: layer %d needs w_stride >= 0 a multiple of 16 and b_stride >= 0", l);
   if (p.prologue == CP_PRO_TAPS) {   // the shipped refine-stage shapes run on the warp-specialised kernel
     bool shapes_ok = true;
     for (int l = 0; l < p.num_layers; ++l) shapes_ok = shapes_ok && p.layers[l].w_packed && (reinterpret_cast<uintptr_t>(p.layers[l].w_packed) & 15) == 0;

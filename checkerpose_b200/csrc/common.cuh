@@ -63,16 +63,21 @@ __host__ __device__ __forceinline__ size_t packed_tile_offset(size_t nb, size_t 
   return nb * 128 * K * 2 + kc * rows * 128;
 }
 
-// One packed weight tile in the tile tables of the persistent kernels (pad keeps the entries 16 bytes)
+// One packed weight tile in the tile tables of the persistent kernels: the tile of object 0, and the index of the layer
+// whose w_stride moves it to another object's weights (cp_chain_layer)
 struct WTile {
   const uint8_t* ptr;
   uint32_t bytes;
-  uint32_t pad;
+  uint32_t layer;
 };
-static inline WTile packed_tile(const void* w_packed, int nb, int kc, int K, int npad) {
+static inline WTile packed_tile(const void* w_packed, int nb, int kc, int K, int npad, int layer = 0) {
   const int rows = packed_block_rows(nb, npad);
-  return {static_cast<const uint8_t*>(w_packed) + packed_tile_offset(nb, kc, rows, K), (uint32_t)rows * 128u, 0u};
+  return {static_cast<const uint8_t*>(w_packed) + packed_tile_offset(nb, kc, rows, K), (uint32_t)rows * 128u, (uint32_t)layer};
 }
+// Object of RoI b for the weights of a launch: graph_sel[b] when the launch has object-indexed weights, else 0
+__device__ __forceinline__ int weight_obj(const int32_t* sel, bool wsel, int b) { return (wsel && sel) ? __ldg(sel + b) : 0; }
+// Named barrier over `nthreads` threads (whole warps) of the CTA; id 0 is __syncthreads
+__device__ __forceinline__ void named_bar_sync(int id, int nthreads) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory"); }
 
 __device__ __forceinline__ float lrelu(float v, float slope) { return v > 0.f ? v : v * slope; }
 

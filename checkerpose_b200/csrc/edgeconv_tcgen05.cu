@@ -93,6 +93,7 @@ struct EcParams {
   int tiles_per_roi;
   int tpr_shift;     // log2(tiles_per_roi) when it is a power of two (every shipped N), else -1
   int tma_out;       // bf16 output with nout % 32 == 0: the epilogue stores through the tensor map
+  int wsel;          // object-indexed weights: p.graph_sel selects every tile's weights and bias
   cp::WTile wt[MAX_WTILES];  // order: slice-major, then column block
 };
 
@@ -165,6 +166,8 @@ __device__ void weight_producer(const EcParams& kp, uint8_t* sm, Bars* bars) {
   const TileIt tiles(kp);
   uint32_t cnt = 0;
   for (int ti = 0; ti < tiles.count; ++ti) {
+    const uint8_t* wbase = kp.wt[0].ptr;   // plus the tile's object offset
+    if (kp.wsel) wbase += (int64_t)cp::weight_obj(kp.p.graph_sel, true, tile_roi(kp, tiles.tile(ti))) * kp.p.layer.w_stride;
     for (int c = 0; c < kp.KC; ++c)
       for (int nb = 0; nb < NB; ++nb, ++cnt) {
         const int s = cnt % B_STAGES;
@@ -173,7 +176,7 @@ __device__ void weight_producer(const EcParams& kp, uint8_t* sm, Bars* bars) {
         const cp::WTile& w = kp.wt[c * NB + nb];
         if (elect_one()) {
           mbar_arrive_expect_tx(&bars->b_full[s], w.bytes);
-          bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, w.ptr, w.bytes, &bars->b_full[s]);
+          bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, wbase + (w.ptr - kp.wt[0].ptr), w.bytes, &bars->b_full[s]);
         }
         __syncwarp();
       }
@@ -450,11 +453,24 @@ __device__ void epilogue_warps(const EcParams& kp, const CUtensorMap* out_map, u
   const uint32_t tbuf = sm_base + OFF_TBUF + ew * TBUF_BYTES;
   const uint32_t bias_s = sm_base + OFF_BIAS;
   const float slope = L.slope;
-  const uint32_t bias_blocks = bars->bias_blocks;
+  uint32_t bias_blocks = bars->bias_blocks;
   const int sw = (lane >> 1) & 3;   // SWIZZLE_64B: 16-byte chunk index ^= bits 1-2 of the row
+  int cur_obj = 0;                  // object whose bias row is in shared memory (the kernel loads object 0's)
   for (int ti = 0; ti < tiles.count; ++ti) {
     const int tile = tiles.tile(ti);
     const int b = tile_roi(kp, tile), t = tile - b * kp.tiles_per_roi;
+    const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, b);
+    if (obj != cur_obj) {   // every epilogue warp is past the previous tile's bias reads, then all see the new row
+      cp::named_bar_sync(1, NUM_EPI_WARPS * 32);
+      for (int i = ew * 32 + lane; i < BIAS_BYTES / 4; i += NUM_EPI_WARPS * 32)
+        reinterpret_cast<float*>(sm + OFF_BIAS)[i] = (L.bias && i < L.nout) ? L.bias[(int64_t)obj * L.b_stride + i] : 0.f;
+      cp::named_bar_sync(1, NUM_EPI_WARPS * 32);
+      bool nz = false;
+      if (lane < 16)
+        for (int e = 0; e < 32; ++e) nz |= reinterpret_cast<const float*>(sm + OFF_BIAS)[lane * 32 + e] != 0.f;
+      bias_blocks = __ballot_sync(0xffffffffu, nz);
+      cur_obj = obj;
+    }
     const int n0 = t * TILE_M;
     const int rows_valid = min(TILE_M, p.N - n0);
     const bool row_ok = row < rows_valid;
@@ -658,6 +674,8 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
              "cp_edgeconv_fwd: bad a_out / ld_a_out");
   CP_REQUIRE(L.w_packed && L.kin == p.Co && L.nout >= 1, CP_E_INVALID, "cp_edgeconv_fwd: layer kin=%d must equal Co=%d", L.kin, p.Co);
   CP_REQUIRE((reinterpret_cast<uintptr_t>(L.w_packed) & 15) == 0, CP_E_INVALID, "cp_edgeconv_fwd: weights not 16-byte aligned");
+  CP_REQUIRE(L.w_stride >= 0 && (L.w_stride % 16) == 0 && L.b_stride >= 0, CP_E_INVALID,
+             "cp_edgeconv_fwd: need w_stride >= 0 a multiple of 16 and b_stride >= 0");
   EcParams kp;
   kp.p = p;
   kp.KC = p.Co / 64;
@@ -676,6 +694,7 @@ extern "C" int cp_edgeconv_fwd(const cp_edgeconv_params* pp, cp_stream_t s) {
                "cp_edgeconv_fwd: bad f32 output spec");
   for (int c = 0; c < kp.KC; ++c)
     for (int nb = 0; nb < kp.NB; ++nb) kp.wt[c * kp.NB + nb] = cp::packed_tile(L.w_packed, nb, c, L.kin, kp.npad);
+  kp.wsel = (L.w_stride != 0 || L.b_stride != 0) ? 1 : 0;
   const int num_sms = cp::num_sms();
   const int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;
   // bf16 outputs whose width is a multiple of 32 columns leave through TMA tensor stores: a 3-D map (columns, nodes, RoIs)

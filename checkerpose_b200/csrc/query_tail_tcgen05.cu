@@ -47,7 +47,34 @@ struct QtParams {
   int KC;            // K chunks of 64
   int64_t M;         // B * N
   int num_tiles;
+  int wsel;          // object-indexed weights: p.graph_sel selects them; every tile then holds rows of one RoI
+  int tiles_per_roi; // with wsel
 };
+
+// First row of a tile and its valid rows (the RoI's rows with wsel, else the flat rows of B * N); RoI of the tile with wsel
+__device__ __forceinline__ void tile_rows(const QtParams& kp, int tile, int64_t& row0, int& rows_valid, int& b) {
+  if (kp.wsel) {
+    b = tile / kp.tiles_per_roi;
+    const int n0 = (tile - b * kp.tiles_per_roi) * TILE_M;
+    row0 = (int64_t)b * kp.p.N + n0;
+    rows_valid = min(TILE_M, kp.p.N - n0);
+  } else {
+    b = 0;
+    row0 = (int64_t)tile * TILE_M;
+    rows_valid = (int)min((int64_t)TILE_M, kp.M - row0);
+  }
+}
+
+// b1[64], w2[2][64], b2[2] of object obj -> cst
+__device__ __forceinline__ void load_consts(const cp_query_decode_params& p, float* cst, int64_t obj, int tid, int nthreads) {
+  for (int i = tid; i < 64 + 128 + 2; i += nthreads) {
+    float v;
+    if (i < 64) v = p.b1 ? p.b1[obj * p.b1_stride + i] : 0.f;
+    else if (i < 192) v = p.w2[obj * p.w2_stride + i - 64];          // (2, 64) row-major
+    else v = p.b2 ? p.b2[obj * p.b2_stride + i - 192] : 0.f;
+    cst[i] = v;
+  }
+}
 
 __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_constant__ QtParams kp, const __grid_constant__ CUtensorMap src_map) {
   extern __shared__ uint8_t smem_raw[];
@@ -69,13 +96,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     fence_mbar_init();
   }
   if (warp == 2) tmem_alloc(&bars->tmem_slot, TMEM_COLS);
-  for (int i = threadIdx.x; i < 64 + 128 + 2; i += NTHREADS) {
-    float v;
-    if (i < 64) v = p.b1 ? p.b1[i] : 0.f;
-    else if (i < 192) v = p.w2[i - 64];          // (2, 64) row-major
-    else v = p.b2 ? p.b2[i - 192] : 0.f;
-    cst[i] = v;
-  }
+  load_consts(p, cst, 0, threadIdx.x, NTHREADS);
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -84,19 +105,30 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
 
   if (warp == 0) {
     // ---- producer ----
-    if (elect_one()) {
-      mbar_arrive_expect_tx(&bars->w_full, (uint32_t)(NMID * KC * 128));
-      // the whole packed matrix (cp::packed_tile_offset): one block of 64 rows, chunk c at c * 64 * 128 bytes
-      bulk_g2s(sm + OFF_W, p.w1_packed, (uint32_t)(NMID * KC * 128), &bars->w_full);
-    }
-    __syncwarp();
     uint32_t it = 0;
+    int wobj = -1;   // object whose W1 is resident
     for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x, ++it) {
+      int64_t row0;
+      int rows_valid, b;
+      tile_rows(kp, tile, row0, rows_valid, b);
+      const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, b);
+      if (obj != wobj) {
+        // the previous tile's MMAs read the resident W1: wait until they are done before overwriting it
+        if (it > 0) mbar_wait(&bars->empty[(it - 1) % STAGES], ((it - 1) / STAGES) & 1);
+        if (elect_one()) {
+          mbar_arrive_expect_tx(&bars->w_full, (uint32_t)(NMID * KC * 128));
+          // the whole packed matrix (cp::packed_tile_offset): one block of 64 rows, chunk c at c * 64 * 128 bytes
+          bulk_g2s(sm + OFF_W, reinterpret_cast<const uint8_t*>(p.w1_packed) + (int64_t)obj * p.w1_stride, (uint32_t)(NMID * KC * 128),
+                   &bars->w_full);
+        }
+        __syncwarp();
+        wobj = obj;
+      }
       const uint32_t s = it % STAGES;
       if (it >= STAGES) mbar_wait(&bars->empty[s], ((it / STAGES) - 1) & 1);
       if (elect_one()) {
         mbar_arrive_expect_tx(&bars->full[s], (uint32_t)(KC * A_CHUNK_BYTES));
-        for (int c = 0; c < KC; ++c) tma_load_2d(smem_u32(sm + s * A_STAGE_BYTES + c * A_CHUNK_BYTES), &src_map, c * 64, tile * TILE_M, &bars->full[s]);
+        for (int c = 0; c < KC; ++c) tma_load_2d(smem_u32(sm + s * A_STAGE_BYTES + c * A_CHUNK_BYTES), &src_map, c * 64, (int)row0, &bars->full[s]);
       }
       __syncwarp();
     }
@@ -104,10 +136,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     // ---- MMA issuer ----
     const uint32_t idesc = make_idesc_bf16_m128(NMID);
     const uint32_t w_lo0 = smem_desc_lo(smem_u32(sm + OFF_W));
-    mbar_wait(&bars->w_full, 0);
-    uint32_t it = 0;
+    uint32_t it = 0, wn = 0;
+    int wobj = -1;
     for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x, ++it) {
       const uint32_t s = it % STAGES, slot = it & 1;
+      int64_t row0;
+      int rows_valid, b;
+      tile_rows(kp, tile, row0, rows_valid, b);
+      const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, b);
+      if (obj != wobj) {   // the producer loaded this object's W1
+        mbar_wait(&bars->w_full, wn & 1);
+        ++wn;
+        wobj = obj;
+      }
       if (it >= 2) mbar_wait(&bars->acc_empty[slot], ((it >> 1) - 1) & 1);
       mbar_wait(&bars->full[s], (it / STAGES) & 1);
       tc_fence_after_sync();
@@ -129,8 +170,19 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
     const int q = warp - 4;
     const float slope = p.slope;
     uint32_t it = 0;
+    int cur_obj = 0;   // object whose b1 / W2 / b2 are in cst (the kernel loads object 0's)
     for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x, ++it) {
       const uint32_t slot = it & 1;
+      int64_t row0;
+      int rows_valid, tb_roi;
+      tile_rows(kp, tile, row0, rows_valid, tb_roi);
+      const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, tb_roi);
+      if (obj != cur_obj) {   // every epilogue warp is past the previous tile's reads, then all see the new constants
+        cp::named_bar_sync(1, 128);
+        load_consts(p, cst, obj, q * 32 + lane, 128);
+        cp::named_bar_sync(1, 128);
+        cur_obj = obj;
+      }
       mbar_wait(&bars->acc_full[slot], (it >> 1) & 1);
       tc_fence_after_sync();
       const uint32_t tb = tmem_base + ((uint32_t)(q * 32) << 16) + slot * NMID;
@@ -151,9 +203,9 @@ __global__ void __launch_bounds__(NTHREADS, 1) query_tail_kernel(const __grid_co
       tc_fence_before_sync();
       __syncwarp();
       if (lane == 0) mbar_arrive(&bars->acc_empty[slot]);     // the accumulator is in registers: the next tile's MMAs may run
-      const int64_t e = (int64_t)tile * TILE_M + q * 32 + lane;
-      if (e < kp.M) {
-        const int b = (int)(e / p.N), n = (int)(e - (int64_t)b * p.N);
+      const int64_t e = row0 + q * 32 + lane;
+      if (q * 32 + lane < rows_valid) {
+        const int b = kp.wsel ? tb_roi : (int)(e / p.N), n = (int)(e - (int64_t)b * p.N);
         int kpt = n;
         if (p.perm) kpt = p.perm[(size_t)(p.graph_sel ? p.graph_sel[b] : 0) * p.N + n];
         if (p.logits) {
@@ -195,7 +247,11 @@ extern "C" int cp_query_decode_fwd(const cp_query_decode_params* pp, cp_stream_t
   kp.KC = p.kin / 64;
   kp.M = (int64_t)p.B * p.N;
   CP_REQUIRE(kp.M < (1ll << 31), CP_E_UNSUPPORTED, "cp_query_decode_fwd: B * N must be < 2^31");
-  kp.num_tiles = (int)((kp.M + TILE_M - 1) / TILE_M);
+  CP_REQUIRE(p.w1_stride >= 0 && (p.w1_stride % 16) == 0 && p.b1_stride >= 0 && p.w2_stride >= 0 && p.b2_stride >= 0, CP_E_INVALID,
+             "cp_query_decode_fwd: strides must be >= 0, w1_stride a multiple of 16");
+  kp.wsel = (p.w1_stride != 0 || p.b1_stride != 0 || p.w2_stride != 0 || p.b2_stride != 0) ? 1 : 0;
+  kp.tiles_per_roi = (p.N + TILE_M - 1) / TILE_M;
+  kp.num_tiles = kp.wsel ? kp.tiles_per_roi * p.B : (int)((kp.M + TILE_M - 1) / TILE_M);
   CUtensorMap map;
   memset(&map, 0, sizeof(map));
   const int rc = cp::make_bf16_operand_map(&map, p.src, p.kin, kp.M, p.ld_src, "cp_query_decode_fwd");

@@ -64,6 +64,7 @@ struct TcParams {
   int P2;        // 128-column blocks of layer 2 per half (1: nout2 = 256, one half; 2: nout2 = 512, two halves)
   int halves2;   // 1 or 2 accumulator passes for layer 2
   int T;         // weight tiles per node tile
+  int wsel;      // object-indexed weights: p.graph_sel selects every tile's weights and biases
   cp::WTile wt[MAX_WT]; // in the order the MMA thread consumes them
 };
 
@@ -147,13 +148,15 @@ __device__ void gather_warps(const TcParams& kp, uint8_t* sm, Bars* bars, int gw
 __device__ void weight_producer(const TcParams& kp, uint8_t* sm, Bars* bars) {
   uint32_t cnt = 0;
   for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x) {
+    const int64_t obj = cp::weight_obj(kp.p.graph_sel, kp.wsel != 0, tile / kp.tiles_per_roi);
     for (int w = 0; w < kp.T; ++w, ++cnt) {
       const int s = cnt % B_STAGES;
       const uint32_t use = cnt / B_STAGES;
       if (use > 0) mbar_wait(&bars->b_empty[s], (use - 1) & 1);
       if (elect_one()) {
         mbar_arrive_expect_tx(&bars->b_full[s], kp.wt[w].bytes);
-        bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, kp.wt[w].ptr, kp.wt[w].bytes, &bars->b_full[s]);
+        bulk_g2s(sm + OFF_B + s * B_STAGE_BYTES, kp.wt[w].ptr + obj * kp.p.layers[kp.wt[w].layer].w_stride, kp.wt[w].bytes,
+                 &bars->b_full[s]);
       }
       __syncwarp();
     }
@@ -248,6 +251,16 @@ __device__ void mma_issuer(const TcParams& kp, uint8_t* sm, Bars* bars, uint32_t
   }
 }
 
+// biases of object obj: layer 0 at [0,256), layer 1 at [256,512), layer 2 at [512, 1024); zero where a layer has none
+__device__ void load_biases(const TcParams& kp, uint8_t* sm, int64_t obj, int tid, int nthreads) {
+  for (int i = tid; i < BIAS_FLOATS; i += nthreads) {
+    const int layer = i < 256 ? 0 : i < 512 ? 1 : 2;
+    const int c = i - (layer == 2 ? 512 : layer * 256);
+    const cp_chain_layer& L = kp.p.layers[layer];
+    reinterpret_cast<float*>(sm + OFF_BIAS)[i] = (L.bias && c < L.nout) ? L.bias[obj * L.b_stride + c] : 0.f;
+  }
+}
+
 // ------------------------------------------------------------------------------------------------------
 // epilogue: warp (q = w & 3, half = w >> 2) drains TMEM lanes [32 q, 32 q + 32), every second 32-column block
 // ------------------------------------------------------------------------------------------------------
@@ -260,10 +273,18 @@ __device__ void epilogue_warps(const TcParams& kp, const CUtensorMap* out_map, u
   const uint32_t tbuf = sm_base + OFF_TBUF + ew * TBUF_BYTES;
   const int sw = (lane >> 1) & 3;   // SWIZZLE_64B: 16-byte chunk index ^= bits 1-2 of the row
   uint32_t st = 0, hfree = 0;
+  int cur_obj = 0;   // object whose biases are in shared memory (the kernel loads object 0's)
   for (int tile = blockIdx.x; tile < kp.num_tiles; tile += gridDim.x) {
     const int b = tile / kp.tiles_per_roi, n0 = (tile - b * kp.tiles_per_roi) * TILE_M;
     const int rows_valid = min(TILE_M, p.N - n0);
     const int nstages = 2 + kp.halves2;
+    const int obj = cp::weight_obj(p.graph_sel, kp.wsel != 0, b);
+    if (obj != cur_obj) {   // every epilogue warp is past the previous tile's bias reads, then all see the new row
+      cp::named_bar_sync(1, NUM_E_WARPS * 32);
+      load_biases(kp, sm, obj, ew * 32 + lane, NUM_E_WARPS * 32);
+      cp::named_bar_sync(1, NUM_E_WARPS * 32);
+      cur_obj = obj;
+    }
     for (int k = 0; k < nstages; ++k, ++st) {
       const uint32_t slot = st & 1;
       const int layer = k < 2 ? k : 2;
@@ -353,13 +374,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) taps_chain_kernel(const __grid_co
     fence_mbar_init();
   }
   if (warp == W_WARP) tmem_alloc(&bars->tmem_slot, 2 * ACC_COLS);
-  // biases: layer 0 at [0,256), layer 1 at [256,512), layer 2 at [512, 1024); zero where a layer has none
-  for (int i = threadIdx.x; i < BIAS_FLOATS; i += NTHREADS) {
-    const int layer = i < 256 ? 0 : i < 512 ? 1 : 2;
-    const int c = i - (layer == 2 ? 512 : layer * 256);
-    const cp_chain_layer& L = kp.p.layers[layer];
-    reinterpret_cast<float*>(sm + OFF_BIAS)[i] = (L.bias && c < L.nout) ? L.bias[c] : 0.f;
-  }
+  load_biases(kp, sm, 0, threadIdx.x, NTHREADS);
   tc_fence_before_sync();
   __syncthreads();
   tc_fence_after_sync();
@@ -401,14 +416,16 @@ bool taps_chain_try(const cp_chain_params& p, cudaStream_t s, int* rc) {
   kp.halves2 = L2.nout / 256;
   kp.P2 = 2;
   int T = 0;
-  auto tile = [](const cp_chain_layer& L, int nb, int kc) { return cp::packed_tile(L.w_packed, nb, kc, L.kin, L.nout); };
+  auto tile = [](const cp_chain_layer& L, int nb, int kc, int l) { return cp::packed_tile(L.w_packed, nb, kc, L.kin, L.nout, l); };
   for (int c = 0; c < kp.KX; ++c)
-    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L0, nb, c);
+    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L0, nb, c, 0);
   for (int c = 0; c < NH; ++c)
-    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L1, nb, c);
+    for (int nb = 0; nb < 2; ++nb) kp.wt[T++] = tile(L1, nb, c, 1);
   for (int half = 0; half < kp.halves2; ++half)
     for (int c = 0; c < NH; ++c)
-      for (int nb = 0; nb < kp.P2; ++nb) kp.wt[T++] = tile(L2, half * 2 + nb, c);
+      for (int nb = 0; nb < kp.P2; ++nb) kp.wt[T++] = tile(L2, half * 2 + nb, c, 2);
+  kp.wsel = 0;
+  for (int l = 0; l < 3; ++l) kp.wsel |= (p.layers[l].w_stride != 0 || p.layers[l].b_stride != 0);
   kp.T = T;
   const int num_sms = cp::num_sms();
   const int grid = kp.num_tiles < num_sms ? kp.num_tiles : num_sms;

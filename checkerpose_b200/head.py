@@ -113,7 +113,10 @@ def check_bf16_width(what: str, c: int, limit: int = MAX_BF16_WIDTH) -> None:
 class PreparedLinear:
     """bf16 mode: ``packed`` = bf16 tile image for the chain / EdgeConv kernels.  float32 mode: ``split`` = the
     (hi, lo) bf16 tile images of the split-precision tensor-core GEMM (cp_gemm_x3); layers whose K is not a multiple
-    of 64 keep the SIMT GEMM.  ``nout`` / ``kin`` are the widths of the (possibly padded) weight."""
+    of 64 keep the SIMT GEMM.  ``nout`` / ``kin`` are the widths of the (possibly padded) weight.  ``w_stride`` / ``b_stride`` /
+    ``w_elems`` are the distances between consecutive objects' ``packed`` / ``b`` / ``w`` (0: one object; StackedPrep)."""
+
+    w_stride = b_stride = w_elems = 0
 
     def __init__(self, weight, bias, want_packed):
         self.w = weight.detach().reshape(weight.shape[0], -1).contiguous().float()
@@ -185,7 +188,14 @@ _PREP = PrepCache()
 
 
 def prepared_edgeconv(sg_module, dtype) -> PreparedEdgeConv:
-    """bf16 mode: input and output widths padded to multiples of 64 (unchanged when they are)."""
+    """bf16 mode: input and output widths padded to multiples of 64 (unchanged when they are).  Inside an object-bank forward:
+    the StackedPrep of the layer over every member net."""
+    if _BANK is not None:
+        return _BANK.stacked(sg_module, ("ec",), lambda m: _prepared_edgeconv(m, dtype))
+    return _prepared_edgeconv(sg_module, dtype)
+
+
+def _prepared_edgeconv(sg_module, dtype) -> PreparedEdgeConv:
     want = dtype == torch.bfloat16
     co, c2 = sg_module.conv[0].weight.shape[:2]
     pad = want and (co % 64 != 0 or (c2 // 2) % 64 != 0)
@@ -193,7 +203,15 @@ def prepared_edgeconv(sg_module, dtype) -> PreparedEdgeConv:
 
 
 def prepared_linear(lin: nn.Module, dtype, rows=None, cols=None) -> PreparedLinear:
-    """``rows`` / ``cols``: ((true, padded), ...) segments the bf16 weight is zero-padded to (see pad_linear_weight)."""
+    """``rows`` / ``cols``: ((true, padded), ...) segments the bf16 weight is zero-padded to (see pad_linear_weight).  Inside an
+    object-bank forward: the StackedPrep of the layer over every member net."""
+    if _BANK is not None:
+        key = ("lin", None if rows is None else tuple(rows), None if cols is None else tuple(cols))
+        return _BANK.stacked(lin, key, lambda m: _prepared_linear(m, dtype, rows, cols))
+    return _prepared_linear(lin, dtype, rows, cols)
+
+
+def _prepared_linear(lin: nn.Module, dtype, rows=None, cols=None) -> PreparedLinear:
     want = dtype == torch.bfloat16
     rows = ((lin.weight.shape[0],) * 2,) if rows is None else tuple(rows)
     cols = ((lin.weight.shape[1],) * 2,) if cols is None else tuple(cols)
@@ -208,6 +226,11 @@ def _padded_linear(lin: nn.Module, kin_stored: int, last: bool = False) -> Prepa
     nout, kin = lin.weight.shape
     check_bf16_width("a Linear layer", max(kin, nout))
     return prepared_linear(lin, torch.bfloat16, rows=((nout, nout if last else pad64(nout)),), cols=((kin, kin_stored),))
+
+
+def _chain(prep, kin, nout, act, slope):
+    """Chain-kernel layer of a prepared weight (object-indexed when ``prep`` is a StackedPrep)."""
+    return ops.chain_layer(prep.packed, prep.b, kin, nout, act, slope, prep.w_stride, prep.b_stride)
 
 
 class GraphTable:
@@ -266,7 +289,10 @@ class GraphCtx:
 
 
 def graph_ctx(knn_src, obj_ids, batch: int, device) -> GraphCtx:
-    """Plan of a module's graph (built once, cached on the graph object) + selector for this batch."""
+    """Plan of a module's graph (built once, cached on the graph object) + selector for this batch.  Inside an object-bank
+    forward the graph is the members' graphs stacked (graph g = net g's) and obj_ids are the 1-based bank indices."""
+    if _BANK is not None:
+        knn_src = _BANK.graph(knn_src)
     device = torch.device(device)
     t = _graph_tensor(knn_src, device)
     hit = getattr(t, "_cp_plan", None)
@@ -337,7 +363,7 @@ def edgeconv_node_major(sg_module, x_nm, ctx: GraphCtx, dtype):
     # bf16: widths padded to multiples of 64; the result keeps the padded channels (zeros)
     z = torch.empty((B, N, 2 * prep.Co), dtype=torch.bfloat16, device=x_nm.device)
     ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=_pad_to(x_nm, prep.C),
-                  layers=[ops.chain_layer(prep.packed, prep.b, prep.C, 2 * prep.Co, False, 0.0)], out=z, out_mode=ops.OUT_BF16)
+                  layers=[_chain(prep, prep.C, 2 * prep.Co, False, 0.0)], out=z, out_mode=ops.OUT_BF16)
     return ops.edge_aggregate(z, ctx.plan.idx_p, ctx.sel, prep.slope)
 
 
@@ -356,7 +382,7 @@ def init_head_node_major(init_net, feat_last, obj_ids, dtype):
         conv = _bf16_module(init_net.conv1x1)
         x0, bias0 = conv(feat_last.to(torch.bfloat16), defer_last_bias=True)   # bias applied by the layout change below
     else:
-        x0 = image_block(init_net.conv1x1, feat_last, dtype)                   # 1x1 conv = split-precision GEMM, NHWC result
+        x0 = GroupMaps.cat(image_block(init_net.conv1x1, feat_last, dtype))    # 1x1 conv = split-precision GEMM, NHWC result
     blocks = list(init_net.pre_query_block)
     mlp = prepared_linear(init_net.mlp, dtype)
     nbits = mlp.nout
@@ -384,7 +410,7 @@ def init_head_node_major(init_net, feat_last, obj_ids, dtype):
         return logits, x, ctx
     # bf16: LOAD->[W_0] ; AGG->[W_j] ... ; AGG(+store feature)->[mlp]
     logits = torch.empty((B, N, 16), dtype=torch.float32, device=dev)
-    mlp_layer = ops.chain_layer(mlp.packed, mlp.b, 64, nbits, False, 0.0)
+    mlp_layer = _chain(mlp, 64, nbits, False, 0.0)
     if not blocks:
         ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x, layers=[mlp_layer], out=logits, out_mode=ops.OUT_F32, n_valid=nbits)
         return logits, x, ctx
@@ -392,13 +418,11 @@ def init_head_node_major(init_net, feat_last, obj_ids, dtype):
     for b in blocks:
         _require_eval(b)
     z = torch.empty((B, N, 2 * preps[0].Co), dtype=torch.bfloat16, device=dev)
-    ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x,
-                  layers=[ops.chain_layer(preps[0].packed, preps[0].b, preps[0].C, 2 * preps[0].Co, False, 0.0)],
-                  out=z, out_mode=ops.OUT_BF16)
+    ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x, graph_sel=ctx.sel,
+                  layers=[_chain(preps[0], preps[0].C, 2 * preps[0].Co, False, 0.0)], out=z, out_mode=ops.OUT_BF16)
     for j in range(1, len(blocks)):
         z2 = torch.empty((B, N, 2 * preps[j].Co), dtype=torch.bfloat16, device=dev)
-        _agg_gemm(z, ctx, preps[j - 1].slope, ops.chain_layer(preps[j].packed, preps[j].b, preps[j].C, 2 * preps[j].Co, False, 0.0),
-                  z2, ops.OUT_BF16)
+        _agg_gemm(z, ctx, preps[j - 1].slope, _chain(preps[j], preps[j].C, 2 * preps[j].Co, False, 0.0), z2, ops.OUT_BF16)
         z = z2
     gfeat = torch.empty((B, N, preps[-1].Co), dtype=torch.bfloat16, device=dev)
     _agg_gemm(z, ctx, preps[-1].slope, mlp_layer, logits, ops.OUT_F32, n_valid=nbits, a_out=gfeat)
@@ -753,6 +777,8 @@ def image_block(module, x, dtype, skip=None, seg_module=None):
     """Run an image-branch block (up_net[i], patch_generator, seg_block) in ``dtype``; ``skip`` is concatenated
     to ``x`` along the channels first (pipeline.py:372).  ``seg_module``: the 1x1 seg_block that will be applied to this
     block's result -- the slab image branch computes it in the block's last epilogue (result attribute ``_cp_seg``)."""
+    if isinstance(x, GroupMaps):
+        return _BANK.image_block(module, x, dtype, skip, seg_module)
     if _IMG_REUSE is not None and id(module) in _IMG_REUSE:
         return _IMG_REUSE[id(module)]
     if dtype == torch.bfloat16 and _IMAGE_BRANCH == "cudnn":
@@ -769,6 +795,8 @@ def image_block(module, x, dtype, skip=None, seg_module=None):
 
 def patches_nhwc(patch_generator, img_feat, dtype):
     p = image_block(patch_generator, img_feat, dtype)  # (B,E,Hp,Wp)
+    if isinstance(p, GroupMaps):
+        return torch.cat([m.permute(0, 2, 3, 1) for m in p.maps])
     return p.permute(0, 2, 3, 1).contiguous()
 
 
@@ -838,13 +866,11 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
     q0 = _padded_linear(qmods[0], pad64(d0))
     q1 = _padded_linear(qmods[1], q0.nout)
     q = [q0, q1, _padded_linear(qmods[2], q1.nout, last=True)]
-    pg_layers = [ops.chain_layer(pg0.packed, pg0.b, pg0.kin, pg0.nout, True, slope),
-                 ops.chain_layer(pg1.packed, pg1.b, pg1.kin, pg1.nout, True, slope)]
-    q_layers = [ops.chain_layer(q[0].packed, q[0].b, q[0].kin, q[0].nout, True, qslope),
-                ops.chain_layer(q[1].packed, q[1].b, q[1].kin, q[1].nout, True, qslope),
-                ops.chain_layer(q[2].packed, q[2].b, q[2].kin, q[2].nout, False, 0.0)]
+    pg_layers = [_chain(pg0, pg0.kin, pg0.nout, True, slope), _chain(pg1, pg1.kin, pg1.nout, True, slope)]
+    q_layers = [_chain(q[0], q[0].kin, q[0].nout, True, qslope), _chain(q[1], q[1].kin, q[1].nout, True, qslope),
+                _chain(q[2], q[2].kin, q[2].nout, False, 0.0)]
     logits = torch.empty((B, N, 16), dtype=torch.float32, device=dev)
-    common = dict(B=B, N=N)
+    common = dict(B=B, N=N, graph_sel=None if ctx is None else ctx.sel)
     taps_args = dict(prologue=ops.PRO_TAPS, patches=patches, tap_step=k, x_id=x_id, y_id=y_id, mask=roi_mask,
                      graph_feat=gfeat_nm)
     if not blocks:
@@ -856,13 +882,13 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
     # K3 + pre-graph MLP + first [P|Q] GEMM in one launch
     z = torch.empty((B, N, 2 * preps[0].Co), dtype=torch.bfloat16, device=dev)
     ops.chain_fwd(**common, **taps_args,
-                  layers=pg_layers + [ops.chain_layer(preps[0].packed, preps[0].b, preps[0].C, 2 * preps[0].Co, False, 0.0)],
+                  layers=pg_layers + [_chain(preps[0], preps[0].C, 2 * preps[0].Co, False, 0.0)],
                   out=z, out_mode=ops.OUT_BF16)
     # EdgeConv j aggregation fused with EdgeConv j+1's [P|Q] GEMM
     for j in range(1, len(blocks)):
         z2 = torch.empty((B, N, 2 * preps[j].Co), dtype=torch.bfloat16, device=dev)
         _agg_gemm(z, ctx, preps[j - 1].slope,
-                  ops.chain_layer(preps[j].packed, preps[j].b, preps[j].C, 2 * preps[j].Co, False, 0.0), z2, ops.OUT_BF16)
+                  _chain(preps[j], preps[j].C, 2 * preps[j].Co, False, 0.0), z2, ops.OUT_BF16)
         z = z2
     # last aggregation (stored: it is the next stage's graph feature) fused with the first query layer, then the rest
     feat = torch.empty((B, N, preps[-1].Co), dtype=torch.bfloat16, device=dev)
@@ -871,7 +897,8 @@ def refine_node_major(ref, img_feat, gfeat_nm, roi_mask, x_id, y_id, ctx, dtype,
     if decode is not None and q[1].nout == 64 and q[2].nout == 2 and q[1].kin in (64, 128, 256):
         ops.query_decode_fwd(src=hq, w1_packed=q[1].packed, b1=q[1].b, slope=qslope, w2=q[2].w, b2=q[2].b, plane=decode["plane"],
                              Ltot=decode["Ltot"], x_bits=decode["x_bits"], y_bits=decode["y_bits"], x_id=x_id, y_id=y_id,
-                             perm=decode["perm"], graph_sel=decode["sel"], x_id_kp=decode.get("x_id_kp"), y_id_kp=decode.get("y_id_kp"))
+                             perm=decode["perm"], graph_sel=decode["sel"], x_id_kp=decode.get("x_id_kp"), y_id_kp=decode.get("y_id_kp"),
+                             w_stride=(q[1].w_stride, q[2].w_elems), b_stride=(q[1].b_stride, q[2].b_stride))
         return None, feat
     ops.chain_fwd(**common, prologue=ops.PRO_LOAD, src=hq, layers=q_layers[1:], out=logits, out_mode=ops.OUT_F32,
                   n_valid=q[2].nout)
@@ -907,7 +934,7 @@ def mlp_node_major(mods, x_nm, dtype, out_f32=False):
         for jj, (lin, _, _) in enumerate(grp):
             pls.append(_padded_linear(lin, kin, last=last and out_f32 and jj == len(grp) - 1))
             kin = pls[-1].nout
-        cl = [ops.chain_layer(pl.packed, pl.b, pl.kin, pl.nout, act, slope) for pl, (_, act, slope) in zip(pls, grp)]
+        cl = [_chain(pl, pl.kin, pl.nout, act, slope) for pl, (_, act, slope) in zip(pls, grp)]
         if last and out_f32:
             out = torch.empty((B, N, (pls[-1].nout + 15) // 16 * 16), dtype=torch.float32, device=x.device)
             ops.chain_fwd(prologue=ops.PRO_LOAD, B=B, N=N, src=x, layers=cl, out=out, out_mode=ops.OUT_F32, n_valid=pls[-1].nout)
@@ -1024,8 +1051,135 @@ def pose_head_forward(net, img_feats, obj_ids=None, stage=None, dtype=None, bbox
         y_id = ops.permute_rows(y_id.view(B, N, 1), perm, sel, True).view(B, N)
     seg = getattr(img_feat, "_cp_seg", None)         # fused into the last up_net convolution's epilogue (slab image branch)
     if seg is None:
-        seg = image_block(net.seg_block, img_feat, dtype).float().contiguous()
+        seg = GroupMaps.cat(image_block(net.seg_block, img_feat, dtype)).float().contiguous()
     corr = None
     if bbox is not None:
         corr = (ops.correspondences_packed if packed else ops.correspondences)(roi_bit, seg, bbox, x_id, y_id)
     return (roi_bit, x_bits, y_bits, seg, x_id, y_id), corr
+
+
+# --------------------------------------------------------------------------------------------------
+# object banks: one forward over RoIs of many single-object nets (model/object_bank.py)
+# --------------------------------------------------------------------------------------------------
+# The bf16 GNN kernels take object-indexed weights (cp_chain_layer.w_stride / b_stride, cp_query_decode_params strides): a
+# tile of RoI b uses object graph_sel[b].  A bank forward walks the head of its first net with the hooks below active:
+# prepared_edgeconv / prepared_linear return the layer's weights of every member stacked object by object, graph_ctx the
+# members' kNN graphs stacked into one G-graph plan, and image_block runs the image branch (whose kernels carry one set of
+# weights per launch) per object group on the group's contiguous rows of the object-sorted batch.
+_BANK = None
+
+
+class GroupMaps:
+    """Image-branch maps of an object-sorted batch, one tensor per object group (``maps[i]`` = rows of ``groups[i]``)."""
+
+    def __init__(self, maps, groups):
+        self.maps, self.groups = list(maps), groups
+        self._cp_seg = None
+
+    @property
+    def shape(self):
+        return (sum(m.shape[0] for m in self.maps),) + tuple(self.maps[0].shape[1:])
+
+    @property
+    def device(self):
+        return self.maps[0].device
+
+    @staticmethod
+    def cat(x):
+        """The whole batch as one NCHW tensor with NHWC storage (x unchanged when it is not a GroupMaps)."""
+        if not isinstance(x, GroupMaps):
+            return x
+        return torch.cat([m.permute(0, 2, 3, 1) for m in x.maps]).permute(0, 3, 1, 2)
+
+
+class StackedPrep:
+    """bf16 prepared weights of one layer of every member net, concatenated object by object (``packed`` (G, bytes), ``b``
+    (G, nout), ``w`` (G, nout, kin)): slice g is byte for byte what member g alone runs with.  ``members`` keeps the members'
+    own prepared weights: they are rebuilt when a member's parameters change, and so is the stack (BankEngine.stacked)."""
+
+    def __init__(self, members):
+        m0 = members[0]
+        self.members = members
+        self.nout, self.kin = m0.nout, m0.kin
+        for a in ("C", "Co", "slope"):
+            if hasattr(m0, a):
+                setattr(self, a, getattr(m0, a))
+        self.packed = torch.stack([m.packed for m in members])
+        self.w = torch.stack([m.w for m in members])
+        self.b = None if m0.b is None else torch.stack([m.b for m in members])
+        self.w_stride, self.w_elems = self.packed.stride(0), self.w.stride(0)
+        self.b_stride = 0 if self.b is None else self.b.stride(0)
+
+
+class _StackedGraph:
+    """The members' kNN graphs of one layer stacked into a (G,N,K) table (graph g = member g's), with their keypoints."""
+
+    def __init__(self, srcs):
+        self.srcs = srcs
+        self._hit = None
+        xyz = [getattr(s, "p3d_normed", None) for s in srcs]
+        self.p3d_normed = None if any(x is None for x in xyz) else torch.cat([x.detach().float().cpu() for x in xyz])
+
+    def get(self, device):
+        ts = [_graph_tensor(s, device) for s in self.srcs]
+        key = tuple((id(t), _ver(t)) for t in ts)
+        if self._hit is None or self._hit[0] != key or self._hit[1].device != torch.device(device):
+            self._hit = (key, torch.cat([t.to(device) for t in ts]), ts)
+        return self._hit[1]
+
+
+class BankEngine:
+    """Per-member lookup tables of an object bank: for every submodule (and kNN graph) of the first net, the same one of
+    every member; the stacked weights and graphs built from them."""
+
+    def __init__(self, nets):
+        self.nets = nets
+        self._members, self._graphs, self._stack = {}, {}, {}
+        subs = [dict(n.named_modules()) for n in nets]
+        for name, m in subs[0].items():
+            self._members[id(m)] = [s[name] for s in subs]
+            knn = m.__dict__.get("_knn")
+            if knn is not None and id(knn) not in self._graphs:
+                self._graphs[id(knn)] = _StackedGraph([s[name].__dict__["_knn"] for s in subs])
+        self.groups = None
+
+    def stacked(self, module, key, build_one):
+        members = [build_one(m) for m in self._members[id(module)]]
+        hit = self._stack.get((id(module), key))
+        if hit is None or any(a is not b for a, b in zip(hit.members, members)):
+            hit = StackedPrep(members)
+            self._stack[(id(module), key)] = hit
+        return hit
+
+    def graph(self, knn_src):
+        return self._graphs[id(knn_src)]
+
+    def image_block(self, module, x, dtype, skip, seg_module):
+        """Run image_block per object group with each group's own member modules; -> GroupMaps (``_cp_seg`` = the fused seg
+        outputs of all groups, concatenated, when every group has one)."""
+        mods = self._members[id(module)]
+        segs = None if seg_module is None else self._members[id(seg_module)]
+        global _BANK
+        bank, _BANK = _BANK, None       # members' own preparations inside a group
+        try:
+            ys = [image_block(mods[g], x.maps[i], dtype, skip=None if skip is None else skip.maps[i],
+                              seg_module=None if segs is None else segs[g]) for i, (g, _, _) in enumerate(x.groups)]
+        finally:
+            _BANK = bank
+        out = GroupMaps(ys, x.groups)
+        seg = [getattr(y, "_cp_seg", None) for y in ys]
+        out._cp_seg = None if any(t is None for t in seg) else torch.cat(seg)
+        return out
+
+
+@contextlib.contextmanager
+def object_bank(engine: BankEngine):
+    """Activate the bank hooks for one bf16 head forward walked on ``engine.nets[0]``."""
+    global _BANK
+    if _BANK is not None:
+        raise RuntimeError("object bank forwards do not nest")
+    _BANK = engine
+    try:
+        yield
+    finally:
+        _BANK = None

@@ -519,8 +519,11 @@ class _Layer(ChainLayer):
     """ChainLayer that keeps its tensors alive until the launch has been issued."""
 
 
-def chain_layer(w_packed, bias, kin, nout, act, slope) -> ChainLayer:
-    L = _Layer(C.c_void_p(w_packed.data_ptr()), _p(bias), int(kin), int(nout), int(bool(act)), float(slope))
+def chain_layer(w_packed, bias, kin, nout, act, slope, w_stride=0, b_stride=0) -> ChainLayer:
+    """``w_stride`` (bytes) / ``b_stride`` (floats): distance between consecutive objects' packed weights / biases; RoI b of
+    a launch then uses object graph_sel[b] (see cp_chain_layer)."""
+    L = _Layer(C.c_void_p(w_packed.data_ptr()), _p(bias), int(kin), int(nout), int(bool(act)), float(slope), int(w_stride),
+               int(b_stride))
     L._keepalive = (w_packed, bias)
     return L
 
@@ -533,13 +536,14 @@ def chain_fwd(*, prologue, B, N, layers, out, out_mode, n_valid=0,
     _need_cuda(out, src, z, idx32, graph_sel, a_out, patches, x_id, y_id, mask, graph_feat)
     p = ChainParams()
     p.prologue, p.B, p.N = prologue, B, N
+    p.graph_sel = _p(graph_sel)      # AGG: the RoI's graph; every prologue: its weights when a layer has strides
     if prologue == PRO_LOAD:
         assert src.dtype == torch.bfloat16 and src.stride(-1) == 1
         p.src, p.ld_src, p.C = _p(src), src.stride(-2), src.shape[-1]
     elif prologue == PRO_AGG:
         assert z.dtype == torch.bfloat16 and z.is_contiguous() and idx32.dtype == torch.int32 and idx32.is_contiguous()
         p.z, p.ld_z, p.Co = _p(z), z.shape[-1], z.shape[-1] // 2
-        p.idx, p.graph_sel, p.K, p.agg_slope = _p(idx32), _p(graph_sel), idx32.shape[-1], float(agg_slope)
+        p.idx, p.K, p.agg_slope = _p(idx32), idx32.shape[-1], float(agg_slope)
         if a_out is not None:
             assert a_out.dtype == torch.bfloat16 and a_out.is_contiguous()
             p.a_out, p.ld_a_out = _p(a_out), a_out.shape[-1]
@@ -667,11 +671,13 @@ def decode_refine(logits, plane, Ltot, x_bits, y_bits, x_id, y_id, perm=None, gr
 
 
 def query_decode_fwd(*, src, w1_packed, b1, slope, w2, b2, plane, Ltot, x_bits, y_bits, x_id, y_id, perm=None, graph_sel=None,
-                     x_id_kp=None, y_id_kp=None, logits=None):
+                     x_id_kp=None, y_id_kp=None, logits=None, w_stride=0, b_stride=0):
     """Fused tail of a refine stage (cp_query_decode_fwd): src (B,N,kin) bf16 -> lrelu(Linear kin->64) -> Linear 64->2 -> the
-    decode of decode_refine (bit planes, id = 2 id + bit in place, keypoint-order ids).  One launch, TMA tensor loads."""
+    decode of decode_refine (bit planes, id = 2 id + bit in place, keypoint-order ids).  One launch, TMA tensor loads.
+    Object-indexed weights (RoI b uses object graph_sel[b]): ``w_stride`` = (w1_packed bytes, w2 floats), ``b_stride`` = (b1, b2)
+    floats between consecutive objects; w2 is then (G, 2, 64)."""
     _need_cuda(src, w1_packed, b1, w2, b2, x_bits, y_bits, x_id, y_id, perm, graph_sel, x_id_kp, y_id_kp, logits)
-    assert src.dtype == torch.bfloat16 and src.stride(-1) == 1 and w2.dtype == torch.float32 and w2.is_contiguous() and tuple(w2.shape) == (2, 64)
+    assert src.dtype == torch.bfloat16 and src.stride(-1) == 1 and w2.dtype == torch.float32 and w2.is_contiguous() and tuple(w2.shape[-2:]) == (2, 64)
     B, N, kin = src.shape
     p = QueryDecodeParams()
     p.B, p.N = B, N
@@ -682,6 +688,8 @@ def query_decode_fwd(*, src, w1_packed, b1, slope, w2, b2, plane, Ltot, x_bits, 
     p.plane, p.Ltot = int(plane), int(Ltot)
     p.x_bits, p.y_bits, p.x_id, p.y_id, p.x_id_kp, p.y_id_kp = _p(x_bits), _p(y_bits), _p(x_id), _p(y_id), _p(x_id_kp), _p(y_id_kp)
     p.perm, p.graph_sel = _p(perm), _p(graph_sel)
+    p.w1_stride, p.w2_stride = (0, 0) if w_stride == 0 else (int(w_stride[0]), int(w_stride[1]))
+    p.b1_stride, p.b2_stride = (0, 0) if b_stride == 0 else (int(b_stride[0]), int(b_stride[1]))
     _timed_launch(lib.cp_query_decode_fwd, "cp_query_decode_fwd", p, ("QT", kin, (64, 2), OUT_F32, B, N))
 
 

@@ -186,7 +186,7 @@ int cp_edge_aggregate(const void* z, int dtype, const int32_t* idx, const int32_
                       void* y, int B, int N, int K, int Co, cp_stream_t s);
 
 /* Fused tcgen05 chain (bf16 operands, fp32 accumulation in TMEM).  One launch does, per tile of 128
- * nodes:  PROLOGUE -> A tile in shared memory -> up to 3 chained GEMM(+bias+LeakyReLU) layers whose
+ * nodes of one RoI:  PROLOGUE -> A tile in shared memory -> up to 3 chained GEMM(+bias+LeakyReLU) layers whose
  * weights are streamed with bulk-async copies -> OUTPUT.
  *   prologue CP_PRO_LOAD : A = src[b, n, :C]                                   (bf16 node-major)
  *            CP_PRO_AGG  : A = lrelu(max_k z[b, idx[n,k], :Co] + z[b, n, Co:])  (EdgeConv aggregation)
@@ -208,6 +208,10 @@ typedef struct {
                          * layer 0 of TAPS (two K phases, one column pass): <= 512 */
   int act;              /* 0 none, 1 LeakyReLU */
   float slope;
+  /* object-indexed weights: a tile of RoI b reads w_packed + sel[b] * w_stride (bytes, a multiple of 16) and
+   * bias + sel[b] * b_stride (floats), sel = the launch's graph_sel (NULL => object 0).  0 / 0 = one set of weights. */
+  int64_t w_stride;
+  int b_stride;
 } cp_chain_layer;
 
 typedef struct {
@@ -215,7 +219,7 @@ typedef struct {
   int B, N;
   /* LOAD */
   const void* src; int ld_src; int C;
-  /* AGG */
+  /* AGG (graph_sel: per-RoI graph of AGG and, with non-zero layer strides, per-RoI weights of every prologue) */
   const void* z; int ld_z; int Co; const int32_t* idx; const int32_t* graph_sel; int K; float agg_slope;
   /* TAPS: patches (B, Hp, Wp, E) bf16 NHWC (E a multiple of 16, <= 128), ids (B,N) int64, mask (B,N) f32 {0,1},
    * graph_feat (B,N,Cg) bf16 (Cg a multiple of 64, <= 512); A = [tap0 | tap1 | tap2 | tap3 | graph_feat], tap t at t*E */
@@ -285,7 +289,8 @@ int cp_edge_aggregate_staged_f32(const float* z, const cp_graph_plan* plan, cons
  * quarter-warp per node pair of plan.prog -- take the max in registers with 128-bit shared-memory loads and write
  * the bf16 A operand; one thread issues the MMAs against weights streamed through the TMA engine by another, and
  * eight epilogue warps drain TMEM into TMA tensor stores -- all overlapped through mbarriers.
- * All node-major tensors are in PLAN order.  Co in {64,128,256}; layer.kin == Co; layer.nout <= 512;
+ * All node-major tensors are in PLAN order.  graph_sel selects a RoI's graph and, with non-zero layer strides, its weights.
+ * Co in {64,128,256}; layer.kin == Co; layer.nout <= 512;
  * K <= 40; every tile's distinct-row count <= min(umax, cp_edgeconv_ring_rows(KP)) (else use
  * cp_chain_fwd(CP_PRO_AGG)). */
 typedef struct {
@@ -345,7 +350,10 @@ int cp_decode_refine(const float* logits, int ld, int plane, int Ltot, float* x_
  *   hid   = lrelu(src . W1^T + b1)      kin -> 64      tcgen05, A tiles by TMA tensor loads      (MLP_QueryNet, pipeline.py:174-180)
  *   [x,y] = hid . W2^T + b2             64 -> 2        fp32 register dot products
  * then exactly cp_decode_refine on [x, y] (pipeline.py:375-381).  logits (B*N, ld_logits) f32 may be NULL.
- * kin in {64, 128, 256}; nmid == 64; nout == 2; w1_packed from cp_pack_weight; w2 (2, 64) f32 row-major. */
+ * kin in {64, 128, 256}; nmid == 64; nout == 2; w1_packed from cp_pack_weight; w2 (2, 64) f32 row-major.
+ * Object-indexed weights: RoI b uses w1_packed + sel[b] * w1_stride (bytes, a multiple of 16), b1 + sel[b] * b1_stride,
+ * w2 + sel[b] * w2_stride and b2 + sel[b] * b2_stride (floats), sel = graph_sel (NULL => object 0); all 0 = one set.  With a
+ * non-zero stride every tile holds nodes of one RoI (tiles of ceil(N / 128) per RoI). */
 typedef struct {
   int B, N;
   const void* src; int ld_src; int kin;
@@ -355,6 +363,7 @@ typedef struct {
   int plane, Ltot;
   float* x_bits; float* y_bits; int64_t* x_id; int64_t* y_id; int64_t* x_id_kp; int64_t* y_id_kp;
   const int32_t* perm; const int32_t* graph_sel;
+  int64_t w1_stride; int b1_stride, w2_stride, b2_stride;
 } cp_query_decode_params;
 int cp_query_decode_fwd(const cp_query_decode_params* p, cp_stream_t s);
 /* Plan order <-> keypoint order for node-major rows of row_bytes bytes (multiple of 4), out of place:
