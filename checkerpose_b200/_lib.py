@@ -117,6 +117,8 @@ SIGNATURES = {
     "cp_gemm_x3": (c_i32, [C.POINTER(GemmX3Params), c_vp]),
     "cp_edge_aggregate_staged_f32": (c_i32, [c_vp, C.POINTER(GraphPlanStruct), c_vp, c_f32, c_vp, c_i32, c_i32, c_i32, c_vp]),
     "cp_pnp_ransac": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, c_f32, c_i32, C.c_uint64, c_vp, c_vp, c_vp, c_i32, c_i32, c_i32, c_vp]),
+    "cp_pnp_ransac_sets": (c_i32, [c_vp, c_vp, c_vp, c_vp, c_vp, c_i32, c_i32, C.POINTER(C.c_int32), c_vp, c_f32, c_i32, C.c_uint64, c_vp, c_vp,
+                                   c_vp, c_i32, c_i32, c_i32, c_vp]),
     "cp_query_decode_fwd": (c_i32, [C.POINTER(QueryDecodeParams), c_vp]),
     "cp_conv_bf16": (c_i32, [C.POINTER(ConvBf16Params), c_vp]),
     "cp_conv_slab": (c_i32, [C.POINTER(ConvSlabParams), c_vp]),

@@ -300,10 +300,16 @@ __device__ bool gn_step(Pose& P, const float* Xs, const float* xs, const uint8_t
   return ok;
 }
 
+struct FlagSets {
+  uint32_t mask[3];
+};
+
+// grid (B, V): CTA (b, v) solves RoI b on the correspondences of validity set flag_masks.mask[v] and writes row v * B + b of
+// the outputs; its hypotheses are keyed on rng_index[b] (b when NULL), so every (b, v) is what a launch of one set computes.
 __global__ void __launch_bounds__(NT, 1)
 pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __restrict__ rec12, const float* __restrict__ p3d, const int32_t* __restrict__ graph_sel,
-                  const float* __restrict__ cam_K, int k_stride, uint32_t flag_mask, float thresh, int rounds, uint64_t seed,
-                  float* __restrict__ pose_out, int32_t* __restrict__ ninl_out, uint8_t* __restrict__ inl_mask_out, int N, int S) {
+                  const float* __restrict__ cam_K, int k_stride, FlagSets flag_masks, const int32_t* __restrict__ rng_index, float thresh, int rounds,
+                  uint64_t seed, float* __restrict__ pose_out, int32_t* __restrict__ ninl_out, uint8_t* __restrict__ inl_mask_out, int B, int N, int S) {
   extern __shared__ __align__(16) uint8_t smem[];
   float* Xs = reinterpret_cast<float*>(smem);                 // (N, 3) compacted 3-D points
   float* xs = Xs + (size_t)N * 3;                             // (N, 2) normalised image points
@@ -313,6 +319,9 @@ pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __re
   __shared__ int warp_cnt[NT / 32], s_best_cnt, s_best_h;
   __shared__ Pose s_pose;
   const int b = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+  const uint32_t flag_mask = blockIdx.y == 0 ? flag_masks.mask[0] : blockIdx.y == 1 ? flag_masks.mask[1] : flag_masks.mask[2];
+  const size_t o = (size_t)blockIdx.y * B + b;                // output row
+  const int rb = rng_index ? rng_index[b] : b;                // hypothesis stream
   // records: packed rows (bbox + u16 per keypoint) or the 12-byte {u, v, flags} records of cp_correspondences
   const size_t row_bytes = 16 + 2 * (size_t)N;
   const uint8_t* row = packed ? packed + (size_t)b * row_bytes : nullptr;
@@ -372,7 +381,7 @@ pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __re
   }
   const int M = base;
   if (inl_mask_out)
-    for (int n = tid; n < N; n += NT) inl_mask_out[(size_t)b * N + n] = 0;
+    for (int n = tid; n < N; n += NT) inl_mask_out[o * N + n] = 0;
   Pose P;
   for (int i = 0; i < 9; ++i) P.R[i] = (i % 4 == 0) ? 1.f : 0.f;
   P.t[0] = P.t[1] = P.t[2] = 0.f;
@@ -386,7 +395,7 @@ pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __re
     int my_cnt = -1, my_h = 0x7fffffff;
     for (int r = 0; r < rounds; ++r) {
       const int h = r * NT + tid;
-      uint64_t st = seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(b + 1)) ^ (0x8CB92BA72F3D8DD7ull * (uint64_t)(h + 1));
+      uint64_t st = seed ^ (0xD1B54A32D192ED03ull * (uint64_t)(rb + 1)) ^ (0x8CB92BA72F3D8DD7ull * (uint64_t)(h + 1));
       int idx[4];
       bool ok = true;
       for (int i = 0; i < 4 && ok; ++i) {
@@ -427,7 +436,7 @@ pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __re
       for (int k = tid; k < M; k += NT) {
         const bool in = is_inlier(P, Xs + k * 3, xs + k * 2, fx, fy, thr2);
         c += in ? 1.f : 0.f;
-        if (in && inl_mask_out) inl_mask_out[(size_t)b * N + src[k]] = 1;
+        if (in && inl_mask_out) inl_mask_out[o * N + src[k]] = 1;
       }
       block_sum<1>(&c, red, tid);
       ninl = (int)(red[0] + 0.5);
@@ -436,28 +445,55 @@ pnp_ransac_kernel(const uint8_t* __restrict__ packed, const cp_corr_record* __re
     }
   }
   if (tid == 0) {
-    for (int i = 0; i < 9; ++i) pose_out[(size_t)b * 12 + i] = P.R[i];
-    for (int i = 0; i < 3; ++i) pose_out[(size_t)b * 12 + 9 + i] = P.t[i];
-    ninl_out[b] = ninl;
+    for (int i = 0; i < 9; ++i) pose_out[o * 12 + i] = P.R[i];
+    for (int i = 0; i < 3; ++i) pose_out[o * 12 + 9 + i] = P.t[i];
+    ninl_out[o] = ninl;
   }
 }
 
 }  // namespace
 
-extern "C" int cp_pnp_ransac(const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel, const float* cam_K, int k_batched,
-                             int flag_mask, float reproj_thresh, int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out,
-                             uint8_t* inlier_mask_out, int B, int N, int S, cp_stream_t s) {
+// shared by the two entry points; `name` prefixes the error messages
+static int pnp_launch(const char* name, const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel,
+                      const float* cam_K, int k_batched, const int32_t* flag_masks, int num_sets, const int32_t* rng_index, float reproj_thresh,
+                      int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out, uint8_t* inlier_mask_out, int B, int N, int S,
+                      cp_stream_t s) {
   CP_REQUIRE((packed != nullptr) != (records != nullptr) && p3d && cam_K && pose_out && ninl_out && B > 0 && N >= 4, CP_E_INVALID,
-             "cp_pnp_ransac: bad arguments (exactly one of packed / records)");
-  CP_REQUIRE(S > 0 && S <= 64 && N % 2 == 0 && N <= 8192, CP_E_UNSUPPORTED, "cp_pnp_ransac: needs S <= 64 and an even N <= 8192 (S=%d N=%d)", S, N);
-  CP_REQUIRE(flag_mask >= 1 && flag_mask <= 7 && reproj_thresh > 0.f && iterations >= 1, CP_E_INVALID,
-             "cp_pnp_ransac: flag_mask in [1,7], reproj_thresh > 0, iterations >= 1");
+             "%s: bad arguments (exactly one of packed / records)", name);
+  CP_REQUIRE(S > 0 && S <= 64 && N % 2 == 0 && N <= 8192, CP_E_UNSUPPORTED, "%s: needs S <= 64 and an even N <= 8192 (S=%d N=%d)", name, S, N);
+  FlagSets sets = {{0u, 0u, 0u}};
+  bool masks_ok = true;
+  for (int v = 0; v < num_sets; ++v) {
+    masks_ok &= flag_masks[v] >= 1 && flag_masks[v] <= 7;
+    sets.mask[v] = (uint32_t)flag_masks[v];
+  }
+  CP_REQUIRE(masks_ok && reproj_thresh > 0.f && iterations >= 1, CP_E_INVALID, "%s: flag_mask in [1,7], reproj_thresh > 0, iterations >= 1", name);
   const int rounds = (iterations + NT - 1) / NT;
   const size_t smem = (size_t)N * (3 * 4 + 2 * 4 + 2 + 1);
   cudaError_t e = cudaFuncSetAttribute(pnp_ransac_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-  CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "cp_pnp_ransac: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
-  pnp_ransac_kernel<<<B, NT, smem, (cudaStream_t)s>>>(packed, records, p3d, graph_sel, cam_K, k_batched ? 9 : 0, (uint32_t)flag_mask, reproj_thresh,
-                                                    rounds, seed, pose_out, ninl_out, inlier_mask_out, N, S);
-  CP_CHECK_LAUNCH("cp_pnp_ransac");
+  CP_REQUIRE(e == cudaSuccess, CP_E_CUDA, "%s: cudaFuncSetAttribute failed: %s", name, cudaGetErrorString(e));
+  pnp_ransac_kernel<<<dim3(B, num_sets), NT, smem, (cudaStream_t)s>>>(packed, records, p3d, graph_sel, cam_K, k_batched ? 9 : 0, sets, rng_index,
+                                                                     reproj_thresh, rounds, seed, pose_out, ninl_out, inlier_mask_out, B, N, S);
+  CP_CHECK_LAUNCH(name);
   return CP_OK;
+}
+
+extern "C" int cp_pnp_ransac(const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel, const float* cam_K, int k_batched,
+                             int flag_mask, float reproj_thresh, int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out,
+                             uint8_t* inlier_mask_out, int B, int N, int S, cp_stream_t s) {
+  const int32_t mask = flag_mask;
+  return pnp_launch("cp_pnp_ransac", packed, records, p3d, graph_sel, cam_K, k_batched, &mask, 1, nullptr, reproj_thresh, iterations, seed,
+                    pose_out, ninl_out, inlier_mask_out, B, N, S, s);
+}
+
+extern "C" int cp_pnp_ransac_sets(const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel,
+                                  const float* cam_K, int k_batched, int num_sets, const int32_t* flag_masks, const int32_t* rng_index,
+                                  float reproj_thresh, int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out,
+                                  uint8_t* inlier_mask_out, int B, int N, int S, cp_stream_t s) {
+  CP_REQUIRE(flag_masks && num_sets >= 1 && num_sets <= 3, CP_E_INVALID, "cp_pnp_ransac_sets: needs 1 to 3 flag masks (got %d)", num_sets);
+  for (int v = 0; v < num_sets; ++v)
+    for (int u = 0; u < v; ++u)
+      CP_REQUIRE(flag_masks[u] != flag_masks[v], CP_E_INVALID, "cp_pnp_ransac_sets: flag masks %d and %d are both %d", u, v, flag_masks[v]);
+  return pnp_launch("cp_pnp_ransac_sets", packed, records, p3d, graph_sel, cam_K, k_batched, flag_masks, num_sets, rng_index, reproj_thresh,
+                    iterations, seed, pose_out, ninl_out, inlier_mask_out, B, N, S, s);
 }

@@ -145,23 +145,21 @@ class ObjectBank(head.DeviceScopedModule):
     def forward_with_pose(self, img, bbox, p3d_xyz, cam_K, obj_ids, stage=None, flag=ops.FLAG_ALL, reproj_thresh=2.0,
                           iterations=150, seed=0):
         """PoseNet_GNNskip.forward_with_pose for a mixed batch: p3d_xyz (G,N,3) keypoints in mm of the bank's objects in key
-        order, cam_K (3,3) or (B,3,3).  -> (6-tuple, packed records, R (B,3,3), t (B,3), inlier counts (B)).  PnP runs once per
-        object group, so that every RoI draws the hypotheses it draws in its own net's batch."""
+        order, cam_K (3,3) or (B,3,3).  -> (6-tuple, packed records, R (B,3,3), t (B,3), inlier counts (B)); for a tuple
+        ``flag`` (e.g. ``(ops.FLAG_ALL, ops.FLAG_FULL, ops.FLAG_VISIB)``, what test.py reports) R, t and the counts gain a
+        leading set axis.  One PnP launch over the whole batch: every RoI solves against its object's keypoints and draws
+        the hypotheses it draws in its own net's batch (keyed on its index among the RoIs of its object)."""
         out, packed, g = self._head(img, obj_ids, stage, bbox, True)
         dev = packed.device
-        B, N = packed.shape[0], self.nets[0].npoint
+        N = self.nets[0].npoint
         p3d = p3d_xyz.reshape(-1, N, 3)
         if p3d.shape[0] != len(self.obj_keys):
             raise ValueError(f"p3d_xyz holds {p3d.shape[0]} objects, the bank {len(self.obj_keys)}")
-        K = cam_K.reshape(-1, 3, 3)
-        R = torch.empty((B, 3, 3), dtype=torch.float32, device=dev)
-        t = torch.empty((B, 3), dtype=torch.float32, device=dev)
-        ninl = torch.empty((B,), dtype=torch.int32, device=dev)
+        rank = np.empty(len(g), dtype=np.int32)          # index of every RoI among the RoIs of its object, in caller order
+        for gi in np.unique(g):
+            rank[g == gi] = np.arange(int((g == gi).sum()))
         with torch.cuda.device(dev):
-            for gi in np.unique(g):
-                rows = torch.from_numpy(np.flatnonzero(g == gi)).to(dev)
-                Kg = cam_K if K.shape[0] == 1 else K.index_select(0, rows)
-                Rg, tg, ng = ops.pnp_ransac(packed.index_select(0, rows), p3d[gi:gi + 1], Kg, flag=flag, reproj_thresh=reproj_thresh,
-                                            iterations=iterations, seed=seed)
-                R[rows], t[rows], ninl[rows] = Rg, tg, ng
+            sel = torch.from_numpy(g.astype(np.int32)).to(dev)
+            R, t, ninl = ops.pnp_ransac(packed, p3d, cam_K, graph_sel=sel, flag=flag, reproj_thresh=reproj_thresh, iterations=iterations,
+                                        seed=seed, rng_index=torch.from_numpy(rank).to(dev))
         return out, packed, R, t, ninl

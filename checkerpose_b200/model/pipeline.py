@@ -298,7 +298,10 @@ class PoseNet_GNNskip(head.DeviceScopedModule):
                           reproj_thresh=2.0, iterations=150, seed=0):
         """Extension: head + PnP front-end in one call (from_id_to_pose of test_network_with_test_data.py:32-119 for the whole
         batch on the device).  p3d_xyz (G,N,3) object keypoints in mm (G = 1 or one cloud per graph, selected like the kNN
-        graphs), cam_K (3,3) or (B,3,3).  -> (the reference's 6-tuple, packed records, R (B,3,3), t (B,3), inlier counts (B))."""
+        graphs), cam_K (3,3) or (B,3,3).  -> (the reference's 6-tuple, packed records, R (B,3,3), t (B,3), inlier counts (B)).
+        ``flag``: one validity set (ops.FLAG_*) or a tuple of up to 3, solved in one launch; for a tuple R, t and the counts
+        gain a leading set axis (V,B,...), entry v equal to the call with flag[v].  ``flag=(ops.FLAG_ALL, ops.FLAG_FULL,
+        ops.FLAG_VISIB)`` gives the three poses test.py:335-368 reports (all / full mask / visible mask)."""
         out, packed = self.forward_with_correspondences(img, p3d_normed, bbox, stage=stage, obj_ids=obj_ids, packed=True)
         with torch.cuda.device(packed.device):
             sel = None if obj_ids is None else ops.graph_sel(obj_ids.to(packed.device), p3d_xyz.reshape(-1, self.npoint, 3).shape[0])

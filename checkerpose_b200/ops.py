@@ -772,29 +772,62 @@ def unpack_correspondences_host(packed, S: int = 64):
 FLAG_ALL, FLAG_FULL, FLAG_VISIB = 1, 2, 4
 
 
+def _pnp_flag_sets(flag, rng_index, B):
+    """Host checks of a tuple ``flag`` / of ``rng_index`` -> the flag masks as a ctypes int32 array."""
+    masks = tuple(flag) if isinstance(flag, tuple) else (flag,)
+    if not masks:
+        raise RuntimeError("pnp_ransac: the flag tuple is empty")
+    if len(masks) > 3:
+        raise RuntimeError(f"pnp_ransac: at most 3 flag masks, got {len(masks)}")
+    if any(not 1 <= int(f) <= 7 for f in masks):
+        raise RuntimeError(f"pnp_ransac: flag masks must be in [1, 7], got {masks}")
+    if len(set(int(f) for f in masks)) != len(masks):
+        raise RuntimeError(f"pnp_ransac: duplicate flag masks in {masks}")
+    if rng_index is not None:
+        if rng_index.dtype != torch.int32:
+            raise RuntimeError(f"pnp_ransac: rng_index must be int32, got {rng_index.dtype}")
+        if tuple(rng_index.shape) != (B,):
+            raise RuntimeError(f"pnp_ransac: rng_index must have shape ({B},), got {tuple(rng_index.shape)}")
+    return (C.c_int32 * len(masks))(*(int(f) for f in masks))
+
+
 def pnp_ransac(packed, p3d_xyz, cam_K, graph_sel=None, flag=FLAG_ALL, reproj_thresh=2.0, iterations=150, seed=0,
-               return_inlier_mask=False, S=64):
+               return_inlier_mask=False, S=64, rng_index=None):
     """Batched RANSAC PnP over correspondence records (cp_pnp_ransac): ``packed`` is either the (B, 16 + 2N) uint8 rows of
     ``correspondences_packed`` or the (B,N,3) int32 records of ``correspondences``; p3d_xyz (G,N,3) f32 object keypoints in mm,
-    cam_K (3,3) or (B,3,3) -> (R (B,3,3) f32, t (B,3) f32, inlier count (B) int32[, mask (B,N) u8])."""
-    _need_cuda(packed, p3d_xyz, cam_K, graph_sel)
-    assert packed.is_contiguous()
+    cam_K (3,3) or (B,3,3) -> (R (B,3,3) f32, t (B,3) f32, inlier count (B) int32[, mask (B,N) u8]).
+
+    ``flag`` as a tuple of up to 3 distinct masks solves every set in one launch (cp_pnp_ransac_sets) and gives every output a
+    leading set axis: R (V,B,3,3), t (V,B,3), count (V,B)[, mask (V,B,N)]; entry v equals the call with ``flag=flag[v]`` bit for
+    bit.  ``(FLAG_ALL, FLAG_FULL, FLAG_VISIB)`` are the three poses test.py:335-368 reports.  ``rng_index`` (B) int32: RoI b
+    draws the RANSAC hypotheses RoI rng_index[b] draws in a launch without it (e.g. its index within its object's batch)."""
     B = packed.shape[0]
+    sets = _pnp_flag_sets(flag, rng_index, B) if isinstance(flag, tuple) or rng_index is not None else None
+    _need_cuda(packed, p3d_xyz, cam_K, graph_sel, rng_index)
+    assert packed.is_contiguous()
     is_packed = packed.dtype == torch.uint8
     N = (packed.shape[1] - 16) // 2 if is_packed else packed.shape[1]
     p3d = p3d_xyz.reshape(-1, N, 3).contiguous().float()
     Kc = cam_K.reshape(-1, 9).contiguous().float()
     if Kc.shape[0] not in (1, B):
         raise RuntimeError("pnp_ransac: cam_K must be (3,3) or (B,3,3)")
-    pose = torch.empty((B, 12), dtype=torch.float32, device=packed.device)
-    ninl = torch.empty((B,), dtype=torch.int32, device=packed.device)
-    mask = torch.empty((B, N), dtype=torch.uint8, device=packed.device) if return_inlier_mask else None
-    check(lib.cp_pnp_ransac(_p(packed if is_packed else None), _p(None if is_packed else packed), _p(p3d), _p(graph_sel), _p(Kc), int(Kc.shape[0] == B and B > 1), int(flag), float(reproj_thresh),
-                            int(iterations), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(pose), _p(ninl), _p(mask), B, N, int(S), _stream()),
-          "cp_pnp_ransac")
+    V = 1 if sets is None else len(sets)
+    pose = torch.empty((V, B, 12), dtype=torch.float32, device=packed.device)
+    ninl = torch.empty((V, B), dtype=torch.int32, device=packed.device)
+    mask = torch.empty((V, B, N), dtype=torch.uint8, device=packed.device) if return_inlier_mask else None
+    inputs = (_p(packed if is_packed else None), _p(None if is_packed else packed), _p(p3d), _p(graph_sel), _p(Kc), int(Kc.shape[0] == B and B > 1))
+    rest = (float(reproj_thresh), int(iterations), int(seed) & 0xFFFFFFFFFFFFFFFF, _p(pose), _p(ninl), _p(mask), B, N, int(S), _stream())
+    if sets is None:
+        check(lib.cp_pnp_ransac(*inputs, int(flag), *rest), "cp_pnp_ransac")
+    else:
+        rng = None if rng_index is None else rng_index.contiguous()
+        check(lib.cp_pnp_ransac_sets(*inputs, V, sets, _p(rng), *rest), "cp_pnp_ransac_sets")
     _count()
-    R, t = pose[:, :9].reshape(B, 3, 3), pose[:, 9:]
-    return (R, t, ninl, mask) if return_inlier_mask else (R, t, ninl)
+    R, t = pose[..., :9].reshape(V, B, 3, 3), pose[..., 9:]
+    res = (R, t, ninl, mask)
+    if not isinstance(flag, tuple):
+        res = tuple(None if x is None else x[0] for x in res)
+    return res if return_inlier_mask else res[:3]
 
 
 def split_correspondences(rec: torch.Tensor):

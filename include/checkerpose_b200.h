@@ -400,6 +400,16 @@ int cp_correspondences_unpack(const uint8_t* packed, cp_corr_record* out, int B,
 int cp_pnp_ransac(const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel, const float* cam_K, int k_batched,
                   int flag_mask, float reproj_thresh, int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out,
                   uint8_t* inlier_mask_out, int B, int N, int S, cp_stream_t s);
+/* Several validity sets of every RoI in one launch (test.py:335-368 reports the poses of all three: flag masks 1, 2, 4).
+ * flag_masks: num_sets (1-3) distinct masks in [1,7], a HOST array.  rng_index (B) int32 on the device or NULL: RoI b draws
+ * the hypotheses that RoI rng_index[b] draws in a cp_pnp_ransac launch (NULL: b), e.g. its index within its object's batch.
+ * Outputs are set-major: pose_out (num_sets, B, 12), ninl_out (num_sets, B), inlier_mask_out (num_sets, B, N) or NULL.
+ * Slab v equals, bit for bit, cp_pnp_ransac with flag_mask = flag_masks[v] and the same other arguments; one CTA per
+ * (RoI, set). */
+int cp_pnp_ransac_sets(const uint8_t* packed, const cp_corr_record* records, const float* p3d, const int32_t* graph_sel,
+                       const float* cam_K, int k_batched, int num_sets, const int32_t* flag_masks, const int32_t* rng_index,
+                       float reproj_thresh, int iterations, uint64_t seed, float* pose_out, int32_t* ninl_out,
+                       uint8_t* inlier_mask_out, int B, int N, int S, cp_stream_t s);
 
 /* Elementwise helpers behind common_ops.py:5-27 and pipeline.py:84-127.
  * out = sigmoid(x) > thr ? 1 : 0 as f32 (out_dtype 0) or int64 (out_dtype 1). */
